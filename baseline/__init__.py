@@ -1,5 +1,4 @@
-"""The UNMODIFIED reference (vrettasm/VGPA) as it travels to the GPU box: `baseline/_ref/` is a plain
-copy of the reference tree made by `__graft_entry__.build()` in the authoring container (git-ignored,
-not gpurun-ignored).  Nothing of the product (`vgpa_b200/`) imports this package: it serves the
-drop-in tests (the reference's own objects and optimiser driving the CUDA path), the golden-fixture
-scripts and `bench.py`'s reference figures."""
+"""The UNMODIFIED reference (vrettasm/VGPA), which is not part of this repository: a checkout named by
+the environment variable VGPA_REFERENCE, or a copy in `baseline/_ref/` (git-ignored).  Nothing of the
+product (`vgpa_b200/`) imports this package: it serves the drop-in tests (the reference's own objects
+and optimiser driving the CUDA path), the golden-fixture scripts and `bench.py`'s reference figures."""

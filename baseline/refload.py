@@ -1,32 +1,21 @@
-"""Import the unmodified reference from baseline/_ref (or from /root/reference in the authoring
-container).  The reference is pure Python (numpy / scipy / numba); h5py is only used by
-Simulation.save / load (src/var_bayes/simulation.py:1,293,336) and is stubbed when absent."""
+"""Import the unmodified reference (vrettasm/VGPA).  It is not part of this repository: it is found in the
+checkout named by the environment variable VGPA_REFERENCE, else in baseline/_ref (git-ignored).  The
+reference is pure Python (numpy / scipy / numba); h5py is only used by Simulation.save / load
+(src/var_bayes/simulation.py:1,293,336) and is stubbed when absent."""
 import contextlib
 import io
-import shutil
+import os
 import sys
 import types
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 REF_COPY = HERE / "_ref"
-REF_MOUNT = Path("/root/reference")
-
-
-def install_reference(force=False):
-    """Copy the reference tree to baseline/_ref (authoring container only; a no-op elsewhere)."""
-    if not REF_MOUNT.exists():
-        return REF_COPY if REF_COPY.exists() else None
-    if REF_COPY.exists() and not force:
-        return REF_COPY
-    if REF_COPY.exists():
-        shutil.rmtree(REF_COPY)
-    shutil.copytree(REF_MOUNT, REF_COPY, ignore=shutil.ignore_patterns(".git", "__pycache__", "*.pyc"))
-    return REF_COPY
 
 
 def reference_root():
-    for cand in (REF_COPY, REF_MOUNT):
+    env = os.environ.get("VGPA_REFERENCE")
+    for cand in ([Path(env)] if env else []) + [REF_COPY]:
         if (cand / "src" / "var_bayes" / "variational.py").exists():
             return cand
     return None
@@ -36,7 +25,7 @@ def import_reference():
     """dict of the reference's classes, or ImportError with the reason (missing tree, numba, scipy)."""
     root = reference_root()
     if root is None:
-        raise ImportError("baseline/_ref is missing: run __graft_entry__.build() in the authoring container")
+        raise ImportError("the reference tree is missing: set VGPA_REFERENCE to a checkout of vrettasm/VGPA")
     sys.dont_write_bytecode = True
     if str(root) not in sys.path:
         sys.path.insert(0, str(root))

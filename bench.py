@@ -611,6 +611,24 @@ def secondary_configs(torch, local, hbm_peak, with_reference=True):
     return out
 
 
+DUMP_GRAD_ROWS, DUMP_GRAD_COLS = 64, 65536
+
+
+def dump_outputs(out_dir, F_all, G):
+    """What the last timed step handed to its caller, for comparing two builds output for output: F of
+    every problem (gathered over the ranks) as F.npy, and of this rank's gradient (54 GB at 4096
+    problems) a fixed, seeded sample of 64 problems x 65536 entries (32 MB) as grad_sample.npy."""
+    import torch
+    rng = np.random.default_rng([SEED, 99])
+    rows = np.sort(rng.choice(G.shape[0], min(DUMP_GRAD_ROWS, G.shape[0]), replace=False))
+    cols = np.sort(rng.choice(G.shape[1], min(DUMP_GRAD_COLS, G.shape[1]), replace=False))
+    r, c = torch.from_numpy(rows).to(G.device), torch.from_numpy(cols).to(G.device)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "F.npy", F_all.cpu().numpy())
+    np.save(out / "grad_sample.npy", G[r[:, None], c[None, :]].cpu().numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -699,6 +717,8 @@ def run_b200(args):
     ms = float(t.item())
     F_host = F.cpu().numpy()
     assert np.all(np.isfinite(F_host)), "non-finite free energy in the bench batch"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gathered["F_all"], G)
     value = B * world * args.steps / (ms * 1e-3)
     sharded_check = None
     if world > 1:
@@ -886,7 +906,11 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the other BASELINE configs (N = 1 only)")
     ap.add_argument("--scg-problems", type=int, default=444,
                     help="problems per GPU of the device-resident ensemble OPTIMISATION (secondary key ensemble_scg; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write F and a seeded sample of the gradient of the last timed step to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,11 +1,11 @@
 #!/usr/bin/env python
 """
 Generate the golden fixtures under tests/golden/ by running the UNMODIFIED
-reference (vrettasm/VGPA, mounted read-only at /root/reference) in the
-authoring container.  The reference is Python, so it cannot travel to the
-GPU box; its outputs travel instead, as the .npz files this script writes.
+reference (vrettasm/VGPA: a checkout named by VGPA_REFERENCE, or baseline/_ref).
+The reference is not part of this repository; its outputs are, as the .npz
+files this script writes.
 
-Run (authoring container only):
+Run (with the reference checkout):
 
     python tests/golden/make_golden.py            # per-evaluation fixtures
     python tests/golden/make_golden.py --scg      # + SCG convergence traces
@@ -27,6 +27,7 @@ import argparse
 import contextlib
 import io
 import json
+import os
 import sys
 import time
 import types
@@ -34,15 +35,14 @@ from pathlib import Path
 
 import numpy as np
 
-REF = Path("/root/reference")
+REF = Path(os.environ.get("VGPA_REFERENCE", Path(__file__).resolve().parents[2] / "baseline" / "_ref"))
 HERE = Path(__file__).resolve().parent
 SEED = 31415926535
 
 
 def _import_reference():
     if not REF.exists():
-        raise SystemExit("the reference tree is not mounted; goldens can only be "
-                         "regenerated in the authoring container")
+        raise SystemExit("the reference tree is missing: set VGPA_REFERENCE to a checkout of vrettasm/VGPA")
     sys.dont_write_bytecode = True
     sys.path.insert(0, str(REF))
     # h5py is only used by Simulation.save/load (simulation.py:1,293,336).

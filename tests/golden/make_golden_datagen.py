@@ -8,12 +8,13 @@ they consumed.  The draws are recovered by replaying a second numpy Generator wi
 seed through the same sequence of calls, and are STORED, so the tests do not depend on the
 numpy version's Generator stream.
 
-Runs in the authoring container only:
+Runs with the reference checkout (VGPA_REFERENCE, or baseline/_ref):
 
     python tests/golden/make_golden_datagen.py
 """
 import contextlib
 import io
+import os
 import sys
 import types
 from pathlib import Path
@@ -21,7 +22,7 @@ from pathlib import Path
 import numpy as np
 from numpy.random import SeedSequence, default_rng
 
-REF = Path("/root/reference")
+REF = Path(os.environ.get("VGPA_REFERENCE", Path(__file__).resolve().parents[2] / "baseline" / "_ref"))
 HERE = Path(__file__).resolve().parent
 SEED = 31415926535
 
@@ -35,7 +36,7 @@ CASES = {  # model: (sigma, theta, tf, dt, obs density, obs noise)
 
 def main():
     if not REF.exists():
-        raise SystemExit("the reference tree is not mounted")
+        raise SystemExit("the reference tree is missing: set VGPA_REFERENCE to a checkout of vrettasm/VGPA")
     sys.dont_write_bytecode = True
     sys.path.insert(0, str(REF))
     sys.modules.setdefault("h5py", types.ModuleType("h5py"))

@@ -8,25 +8,26 @@ lorenz_96.py:420-434) and dEobs_dr of GaussianLikelihood.gradients (gaussian_lik
 
 Inputs are taken from the existing per-evaluation fixtures (eval_<MODEL>_rk2.npz: A, b from x,
 the marginal moments mt, st, theta, sigma, obs_t, obs_y, R), so the two sets stay consistent.
-Runs the UNMODIFIED reference (authoring container only):
+Runs the UNMODIFIED reference (a checkout named by VGPA_REFERENCE, or baseline/_ref):
 
     python tests/golden/make_golden_hyper.py
 """
 import contextlib
 import io
+import os
 import sys
 import types
 from pathlib import Path
 
 import numpy as np
 
-REF = Path("/root/reference")
+REF = Path(os.environ.get("VGPA_REFERENCE", Path(__file__).resolve().parents[2] / "baseline" / "_ref"))
 HERE = Path(__file__).resolve().parent
 
 
 def main():
     if not REF.exists():
-        raise SystemExit("the reference tree is not mounted")
+        raise SystemExit("the reference tree is missing: set VGPA_REFERENCE to a checkout of vrettasm/VGPA")
     sys.dont_write_bytecode = True
     sys.path.insert(0, str(REF))
     sys.modules.setdefault("h5py", types.ModuleType("h5py"))

@@ -1,12 +1,14 @@
 """
-The drop-in, performed literally (INTEGRATION.md section 1): the UNMODIFIED reference from
-baseline/_ref builds its own Simulation, dynamics, FwdOde, BwdOde, GaussianLikelihood and PriorKL0
+The drop-in, performed literally (INTEGRATION.md section 1): the UNMODIFIED reference (a checkout named
+by VGPA_REFERENCE, or baseline/_ref; these tests skip without one) builds its own Simulation, dynamics,
+FwdOde, BwdOde, GaussianLikelihood and PriorKL0
 (src/var_bayes/simulation.py:92-207), `vgpa_b200.variational.VarGP` takes the place of
 src/var_bayes/variational.py:VarGP in the constructor call of simulation.py:209, and the
 reference's own optimiser (src/numerics/optim_scg.py:75-285) drives free_energy / gradient on the
 CUDA path.  The traces must match the ones the reference recorded with its own VarGP
 (tests/golden/scg_*.npz) within 1e-6 (BASELINE.json), and a single evaluation must match the
-reference's own VarGP, evaluated right here on the box's CPU, to 1e-9 per gradient block.
+reference's own VarGP, evaluated right here on the box's CPU, to 1e-9 per gradient block (and, without
+the reference tree, the outputs it recorded in tests/golden/eval_*.npz).
 """
 import contextlib
 import io
@@ -81,4 +83,25 @@ def test_single_evaluation_against_live_reference(ref, model, method, tf):
     assert rel_err(gr[:na], g_ref[:na]) < 1e-9 and rel_err(gr[na:], g_ref[na:]) < 1e-9
     for k in ("mt", "st", "lamt", "psit"):
         assert rel_err(vgpa.arg_out[k], ref_vgpa.arg_out[k]) < 1e-9, k
+    vgpa.close()
+
+
+@pytest.mark.parametrize("model,method,tf", [("OU", "rk4", None), ("L63", "rk2", 2.0), ("L96", "rk2", 0.2)])
+def test_single_evaluation_against_recorded_reference(model, method, tf):
+    """The check above where the reference tree is absent: the CUDA VarGP, set up by this package's own
+    Simulation, at the evaluation point of tests/golden/eval_<model>_<method>.npz, against what the
+    reference's VarGP returned there."""
+    from vgpa_b200 import Simulation
+    g = np.load(GOLDEN / f"eval_{model}_{method}.npz")
+    sim = Simulation("t")
+    sim.setup(mg.config(model, method, tf))
+    vgpa = sim.build()
+    assert np.array_equal(vgpa.initialization(), g["x0"])
+    F = vgpa.free_energy(g["x"])
+    gr = vgpa.gradient(g["x"])
+    assert abs(F - float(g["F"])) <= 1e-9 * abs(float(g["F"]))
+    na = vgpa.dim_n * vgpa.dim_d * vgpa.dim_d
+    assert rel_err(gr[:na], g["grad"][:na]) < 1e-9 and rel_err(gr[na:], g["grad"][na:]) < 1e-9
+    for k in ("mt", "st", "lamt", "psit"):
+        assert rel_err(vgpa.arg_out[k], g[k]) < 1e-9, k
     vgpa.close()

@@ -64,7 +64,7 @@ def test_two_rank_nccl_matches_single_gpu(tmp_path, total):
     import torch
     import torch.multiprocessing as mp
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
         port = s.getsockname()[1]
@@ -106,7 +106,7 @@ def test_two_rank_sharded_scg_matches_single_gpu(tmp_path):
     import torch.multiprocessing as mp
     from vgpa_b200.batched_scg import BatchedSCG
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     total = 9
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
