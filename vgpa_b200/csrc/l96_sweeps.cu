@@ -123,29 +123,21 @@ struct FwdSmem {
 };
 
 // tile-row product with the left operand in registers (fragment layout):
-//   LK 0: a = A0[n]   LK 1: a = 0.5 (A0[n] + A1[n])   LK 3: a = X[irow][k] from shared (RK2 quirk)
-// the mat-vec always uses the register operand (LK 3: A0).
+//   LK 0: a = A0[n]   LK 1: a = 0.5 (A0[n] + A1[n])
 template <int LK>
 __device__ __forceinline__ void mma_rowa(const double (&A0)[D / 4], const double (&A1)[D / 4],
-                                         const double* __restrict__ X, const double* __restrict__ v, int irow, int g,
+                                         const double* __restrict__ X, const double* __restrict__ v, int g,
                                          int q, double (&acc)[5][2], double& yv)
 {
 #pragma unroll
     for (int J = 0; J < 5; ++J) acc[J][0] = acc[J][1] = 0.0;
     double y = 0.0;
-    const int la = sm_idx(irow, q);
     const int lb = sm_boff(q, g);
 #pragma unroll
     for (int n = 0; n < D / 4; ++n) {
         const int k0 = 4 * n;
-        double a, av;
-        if (LK == 0) a = av = A0[n];
-        else if (LK == 1) a = av = 0.5 * (A0[n] + A1[n]);
-        else {
-            a = X[la + k0];
-            av = A0[n];
-        }
-        y = fma(av, v[k0 + q], y);
+        const double a = LK == 0 ? A0[n] : 0.5 * (A0[n] + A1[n]);
+        y = fma(a, v[k0 + q], y);
         double b[5];
 #pragma unroll
         for (int J = 0; J < 5; ++J) b[J] = X[lb + (n >> 1) * SM_R8 + (n & 1) * SM_BH + 8 * J];
@@ -155,6 +147,58 @@ __device__ __forceinline__ void mma_rowa(const double (&A0)[D / 4], const double
     y += __shfl_xor_sync(0xffffffffu, y, 1);
     y += __shfl_xor_sync(0xffffffffu, y, 2);
     yv = y;
+}
+
+// RK2's inner covariance stage multiplies S by itself (runge_kutta2.py:96).  With S exactly symmetric the
+// product is symmetric bit for bit: entry (j,i) is the same products accumulated in the same order as (i,j).
+// So only the 15 tiles on or below the diagonal are computed, three per warp, and the warp that computes a
+// tile also writes the stage operand at the tile and at its mirror image: 150 DMMAs instead of 250, and no
+// exchange through shared memory.  Warp w computes tiles (a,b), (c,b), (c,d): per k-step two A fragments
+// (tile rows a, c) and two B fragments (tile columns b, d) from S feed its three DMMAs.
+struct SelfTiles { int a, b, c, d; };
+__device__ constexpr SelfTiles kSelfTiles[NMMA] = {{0, 0, 1, 1}, {3, 3, 4, 4}, {2, 0, 3, 1}, {4, 1, 2, 2}, {3, 2, 4, 0}};
+
+// H = S + (dt/2) (Sigma - 2 S S) on this warp's tiles and their mirror images, and the mean's stage
+// operand of row irow: vt[0] = m + (dt/2) (b - A m), with A m from the fragments of A(t) in registers
+__device__ __forceinline__ void rk2_self_stage(FwdSmem& sm, const SelfTiles& tl, const double (&A0)[D / 4], double bc,
+                                               double dt, int irow, int g, int q)
+{
+    const double* X = sm.Sb;
+    const int la = sm_idx(8 * tl.a + g, q), lc = sm_idx(8 * tl.c + g, q);
+    const int lb = sm_boff(q, g) + 8 * tl.b, ld = sm_boff(q, g) + 8 * tl.d;
+    double acc[3][2] = {{0.0, 0.0}, {0.0, 0.0}, {0.0, 0.0}};
+    double y = 0.0;
+#pragma unroll
+    for (int n = 0; n < D / 4; ++n) {
+        const int k0 = 4 * n, kb = (n >> 1) * SM_R8 + (n & 1) * SM_BH;
+        y = fma(A0[n], sm.mv[k0 + q], y);
+        const double fa = X[la + k0], fc = X[lc + k0], fb = X[lb + kb], fd = X[ld + kb];
+        dmma(acc[0][0], acc[0][1], fa, fb);
+        dmma(acc[1][0], acc[1][1], fc, fb);
+        dmma(acc[2][0], acc[2][1], fc, fd);
+    }
+    y += __shfl_xor_sync(0xffffffffu, y, 1);
+    y += __shfl_xor_sync(0xffffffffu, y, 2);
+    const double cdt = next_coef(ODE_RK2, 0) * dt;
+    if (q == 0) sm.vt[0][irow] = sm.mv[irow] + cdt * (-y + bc);
+    const int tr[3] = {tl.a, tl.c, tl.c}, tc[3] = {tl.b, tl.b, tl.d};
+#pragma unroll
+    for (int t = 0; t < 3; ++t) {
+        const int i = 8 * tr[t] + g, j0 = 8 * tc[t] + 2 * q;
+        const double2 sv = *reinterpret_cast<const double2*>(&sm.Sb[sm_idx(i, j0)]);
+        double out[2];
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const int j = j0 + e;
+            const double kk = (i == j ? sm.sig[i] : 0.0) - (acc[t][e] + acc[t][e]);
+            out[e] = (e == 0 ? sv.x : sv.y) + cdt * kk;
+        }
+        *reinterpret_cast<double2*>(&sm.Hb[sm_idx(i, j0)]) = make_double2(out[0], out[1]);
+        if (tr[t] != tc[t]) {   // the mirror image (transposed 8-byte stores: conflict-free in this layout)
+            sm.Hb[sm_idx(j0, i)] = out[0];
+            sm.Hb[sm_idx(j0 + 1, i)] = out[1];
+        }
+    }
 }
 
 template <int METHOD>
@@ -200,6 +244,7 @@ l96_fwd_kernel(Batch b, Scratch s, const double* __restrict__ x, long long xs, i
     __syncthreads();
 
     const bool small_launch = gridDim.x <= SMALL_LAUNCH;
+    const SelfTiles tl = kSelfTiles[w];
     for (int k = 0; k < N - 1; ++k) {
         // launches of at most one CTA per SM (a single SCG run) have nothing to hide the DRAM latency of
         // their only input stream behind: pull this warp's eight rows of A into L2, PF_STEPS indices ahead
@@ -221,20 +266,19 @@ l96_fwd_kernel(Batch b, Scratch s, const double* __restrict__ x, long long xs, i
         double kv = 0.0;     // same for row irow of the mean (replicated over q)
 #pragma unroll
         for (int sidx = 0; sidx < NS; ++sidx) {
-            // the covariance inner stage of RK2 uses S in place of A (runge_kutta2.py:96)
+            if (METHOD == ODE_RK2 && sidx == 0) {   // the covariance inner stage of RK2 uses S in place of A
+                rk2_self_stage(sm, tl, Ac, bc, dt, irow, g, q);
+                __syncthreads();  // Hb, vt[0] complete
+                continue;
+            }
             const int kind = stage_kind(METHOD, sidx);
-            const bool self = (METHOD == ODE_RK2 && sidx == 0);
             const double* X = (sidx == 0) ? sm.Sb : sm.Hb;
             const double* vX = (sidx == 0) ? sm.mv : sm.vt[(sidx - 1) & 1];
             double acc[5][2], yv;
-            if (self)                 mma_rowa<3>(Ac, An, X, vX, irow, g, q, acc, yv);
-            else if (kind == K_CUR)   mma_rowa<0>(Ac, An, X, vX, irow, g, q, acc, yv);
-            else if (kind == K_NEXT)  mma_rowa<0>(An, An, X, vX, irow, g, q, acc, yv);
-            else                      mma_rowa<1>(Ac, An, X, vX, irow, g, q, acc, yv);
-            // RK2's inner covariance stage multiplies S by itself: with S exactly symmetric the product is
-            // too, bit for bit (entry (j,i) is the same products accumulated in the same order), so its
-            // transpose is the accumulator itself: no exchange and no barrier before the epilogue
-            if (!self) row_to_smem(sm.Tb, irow, q, acc);
+            if (kind == K_CUR)        mma_rowa<0>(Ac, An, X, vX, g, q, acc, yv);
+            else if (kind == K_NEXT)  mma_rowa<0>(An, An, X, vX, g, q, acc, yv);
+            else                      mma_rowa<1>(Ac, An, X, vX, g, q, acc, yv);
+            row_to_smem(sm.Tb, irow, q, acc);
             {   // mean stage for row irow: k = -Aop v + bop
                 const double bv = kind == K_CUR ? bc : (kind == K_NEXT ? bn : 0.5 * (bc + bn));
                 const double ks = -yv + bv;
@@ -242,7 +286,7 @@ l96_fwd_kernel(Batch b, Scratch s, const double* __restrict__ x, long long xs, i
                 if (wt != 0.0) kv = (sidx == 0 || (METHOD == ODE_RK2)) ? wt * ks : kv + wt * ks;
                 if (sidx < NS - 1 && q == 0) sm.vt[sidx & 1][irow] = sm.mv[irow] + (next_coef(METHOD, sidx) * dt) * ks;
             }
-            if (!self) __syncthreads();  // T complete
+            __syncthreads();  // T complete
             {
                 const int i = irow;
 #pragma unroll
@@ -253,8 +297,7 @@ l96_fwd_kernel(Batch b, Scratch s, const double* __restrict__ x, long long xs, i
 #pragma unroll
                     for (int e = 0; e < 2; ++e) {
                         const int j = j0 + e;
-                        const double pt = self ? acc[J][e] : sm.Tb[sm_idx(j, i)];
-                        const double kk = (i == j ? sm.sig[i] : 0.0) - (acc[J][e] + pt);
+                        const double kk = (i == j ? sm.sig[i] : 0.0) - (acc[J][e] + sm.Tb[sm_idx(j, i)]);
                         const double wt = ksum_w(METHOD, sidx);
                         if (wt != 0.0) ksum[J][e] = (sidx == 0 || (METHOD == ODE_RK2)) ? wt * kk : ksum[J][e] + wt * kk;
                         const double sold = e == 0 ? sv.x : sv.y;
