@@ -9,6 +9,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/vgpa_b200.h"
@@ -78,9 +79,22 @@ struct BlockCache {
 };
 BlockCache g_block_cache;
 
+// A device allocation that frees itself.  It is destroyed with its owner's device current: the block cache
+// records the current device of a block it keeps.
 struct DevBuf {
     void* p = nullptr;
     size_t bytes = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), bytes(std::exchange(o.bytes, 0)) {}
+    DevBuf& operator=(DevBuf&& o) noexcept
+    {
+        std::swap(p, o.p);
+        std::swap(bytes, o.bytes);
+        return *this;
+    }
+    ~DevBuf() { release(); }
     cudaError_t alloc(size_t n)
     {
         release();
@@ -108,6 +122,84 @@ struct DevBuf {
     template <typename T> T* as() const { return static_cast<T*>(p); }
 };
 
+// Staging of host arrays.  Each helper does nothing once `e` holds an error, so that a run of them stops at
+// the first failure and `e` reports it.  The copies are plain cudaMemcpy (legacy default stream).
+template <typename T = double>
+void alloc(cudaError_t& e, DevBuf& dst, size_t n)
+{
+    if (e == cudaSuccess) e = dst.alloc(sizeof(T) * n);
+}
+template <typename T>
+void to_device(cudaError_t& e, void* dst, const T* src, size_t n)
+{
+    if (e == cudaSuccess) e = cudaMemcpy(dst, src, sizeof(T) * n, cudaMemcpyHostToDevice);
+}
+template <typename T>
+void upload(cudaError_t& e, DevBuf& dst, const T* src, size_t n)
+{
+    alloc<T>(e, dst, n);
+    to_device(e, dst.p, src, n);
+}
+// dst NULL: an output the caller did not ask for
+template <typename T>
+void download(cudaError_t& e, T* dst, const void* src, size_t n)
+{
+    if (e == cudaSuccess && dst != nullptr) e = cudaMemcpy(dst, src, sizeof(T) * n, cudaMemcpyDeviceToHost);
+}
+// `rows` rows of `len` elements, `stride` apart (0 = one row shared by all), into a compact device buffer;
+// *dstride: the row stride there
+void stage_rows(cudaError_t& e, DevBuf& dst, const double* src, long long stride, long long len, int rows,
+                long long* dstride)
+{
+    const int r = stride == 0 ? 1 : rows;
+    alloc(e, dst, (size_t)len * r);
+    if (e != cudaSuccess) return;
+    *dstride = stride == 0 ? 0 : len;
+    if (r == 1 || stride == len) e = cudaMemcpy(dst.p, src, sizeof(double) * (size_t)len * r, cudaMemcpyHostToDevice);
+    else e = cudaMemcpy2D(dst.p, sizeof(double) * len, src, sizeof(double) * stride, sizeof(double) * len, r, cudaMemcpyHostToDevice);
+}
+
+// Trajectory scratch of one pass: `chunk` problems of N time points.
+struct ScratchBufs {
+    DevBuf mt, st, dEm, dEs, esde;
+    cudaError_t alloc(long long chunk, long long N, long long D)
+    {
+        cudaError_t e = cudaSuccess;
+        ::alloc(e, mt, chunk * N * D);
+        ::alloc(e, st, chunk * N * D * D);
+        ::alloc(e, dEm, chunk * N * D);
+        ::alloc(e, dEs, chunk * N * D * D);
+        ::alloc(e, esde, chunk * N);
+        return e;
+    }
+    Scratch view(int* status) const
+    {
+        return Scratch{mt.as<double>(), st.as<double>(), dEm.as<double>(), dEs.as<double>(), esde.as<double>(), status};
+    }
+    size_t bytes() const { return mt.bytes + st.bytes + dEm.bytes + dEs.bytes + esde.bytes; }
+};
+
+std::string vformat(const char* fmt, va_list ap)
+{
+    char buf[512];
+    vsnprintf(buf, sizeof buf, fmt, ap);
+    return buf;
+}
+
+// The error of a call that has no handle (vgpa_last_error(NULL)); returns `code`.
+int set_error(int code, const char* fmt, ...)
+{
+    va_list ap;
+    va_start(ap, fmt);
+    g_create_error = vformat(fmt, ap);
+    va_end(ap);
+    return code;
+}
+int set_cuda_error(cudaError_t e, const char* fn)
+{
+    return set_error(VGPA_ECUDA, "CUDA error in %s: %s", fn, cudaGetErrorString(e));
+}
+
 int n_theta(int model) { return model == VGPA_MODEL_L63 ? 3 : 1; }
 
 }  // namespace
@@ -115,18 +207,10 @@ int n_theta(int model) { return model == VGPA_MODEL_L63 ? 3 : 1; }
 struct vgpa_handle {
     vgpa_desc d{};
     Batch batch{};
-    Scratch scratch{};
     int chunk = 0;
     long long n_x = 0;   // N * D * (D + 1)
     DevBuf theta, sigma, R, obs_t, obs_index, obs_y, m0, s0, E0, status;
-    DevBuf sc_mt, sc_st, sc_dEm, sc_dEs, sc_esde;
-    // second scratch lane: consecutive chunks run on two internal streams so that the
-    // latency-bound energy kernel of one chunk overlaps the sweeps of the other
-    DevBuf sc2_mt, sc2_st, sc2_dEm, sc2_dEs, sc2_esde;
-    Scratch scratch2{};
-    int lanes = 1;
-    cudaStream_t s_lane[2] = {nullptr, nullptr};
-    cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
+    ScratchBufs sc;
     cudaEvent_t ev_done = nullptr;      // end of the last vgpa_eval_device (a call on ANOTHER stream waits for it: one scratch)
     // host-API staging: two slots of one chunk each
     DevBuf st_x[2], st_g[2], st_F;
@@ -169,12 +253,10 @@ struct vgpa_handle {
 
     int fail(int code, const char* fmt, ...)
     {
-        char buf[512];
         va_list ap;
         va_start(ap, fmt);
-        vsnprintf(buf, sizeof buf, fmt, ap);
+        err = vformat(fmt, ap);
         va_end(ap);
-        err = buf;
         return code;
     }
     int cuda_fail(cudaError_t e, const char* what)
@@ -191,30 +273,13 @@ struct vgpa_handle {
 
 namespace {
 
-// upload a per-problem array given with an element stride (0 = shared)
-int upload(vgpa_handle* h, DevBuf& dst, const double* src, long long stride, long long len, int B,
-           const double** dev_ptr, long long* dev_stride, const char* name)
-{
-    if (src == nullptr) return h->fail(VGPA_EINVAL, "descriptor field %s is NULL", name);
-    if (stride != 0 && stride < len) return h->fail(VGPA_EINVAL, "%s_stride %lld < %lld", name, stride, len);
-    const long long copies = (stride == 0) ? 1 : B;
-    std::vector<double> host((size_t)copies * len);
-    for (long long q = 0; q < copies; ++q) memcpy(&host[(size_t)q * len], src + q * stride, sizeof(double) * len);
-    CK(dst.alloc(host.size() * sizeof(double)), "cudaMalloc(params)");
-    CK(cudaMemcpy(dst.p, host.data(), host.size() * sizeof(double), cudaMemcpyHostToDevice), "cudaMemcpy(params)");
-    *dev_ptr = dst.as<double>();
-    *dev_stride = (stride == 0) ? 0 : len;
-    return VGPA_OK;
-}
-
 bool small_model(int model) { return model != VGPA_MODEL_L96; }
 
 // one pass over problems [p0, p0 + count) with device buffers
 void run_chunk(vgpa_handle* h, const double* d_x, long long xs, int want_grad, double* d_F, double* d_grad,
-               long long gs, int p0, int count, const Extra& ex, cudaStream_t st, int lane = 0)
+               long long gs, int p0, int count, const Extra& ex, cudaStream_t st)
 {
-    Scratch sc = lane ? h->scratch2 : h->scratch;
-    sc.status = h->status.as<int>() + p0;
+    const Scratch sc = h->sc.view(h->status.as<int>() + p0);
     const Batch& b = h->batch;
     const bool small = small_model(b.model);
     h->tick(0, st, true);
@@ -296,10 +361,7 @@ const char* vgpa_last_error(const vgpa_handle* h) { return h ? h->err.c_str() : 
 int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
 {
     if (out) *out = nullptr;
-    if (d == nullptr || out == nullptr) {
-        g_create_error = "vgpa_create: NULL argument";
-        return VGPA_EINVAL;
-    }
+    if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create: NULL argument");
     vgpa_handle* h = new vgpa_handle();
     h->d = *d;
     auto bail = [&](int rc) {
@@ -346,10 +408,21 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
     Batch& b = h->batch;
     b.model = d->model; b.method = d->method; b.D = D; b.N = N; b.M = M; b.B = B;
     b.dt = d->dt; b.dt_model = d->dt_model;
+    // a per-problem parameter: one row shared by the batch (stride 0) or B rows `stride` apart
+    auto upload_param = [&](DevBuf& buf, const double* src, long long stride, long long len, const double** dev,
+                            long long* dev_stride, const char* name) -> int {
+        if (src == nullptr) return h->fail(VGPA_EINVAL, "descriptor field %s is NULL", name);
+        if (stride != 0 && stride < len) return h->fail(VGPA_EINVAL, "%s_stride %lld < %lld", name, stride, len);
+        cudaError_t e = cudaSuccess;
+        stage_rows(e, buf, src, stride, len, B, dev_stride);
+        if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_create(params)");
+        *dev = buf.as<double>();
+        return VGPA_OK;
+    };
     int rc;
-#define UP(field, len)                                                                              \
-    if ((rc = upload(h, h->field, d->field, d->field##_stride, (len), B, &b.field, &b.field##_stride, \
-                     #field)) != VGPA_OK)                                                           \
+#define UP(field, len)                                                                                       \
+    if ((rc = upload_param(h->field, d->field, d->field##_stride, (len), &b.field, &b.field##_stride, #field)) \
+        != VGPA_OK)                                                                                          \
         return bail(rc);
     UP(theta, n_theta(d->model));
     UP(sigma, D);
@@ -371,12 +444,10 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
             ot[n] = d->obs_t[n];
             oi[d->obs_t[n]] = n;
         }
-        cudaError_t e;
-        if ((e = h->obs_t.alloc(ot.size() * sizeof(long long))) != cudaSuccess ||
-            (e = h->obs_index.alloc(oi.size() * sizeof(int))) != cudaSuccess ||
-            (e = cudaMemcpy(h->obs_t.p, ot.data(), ot.size() * sizeof(long long), cudaMemcpyHostToDevice)) != cudaSuccess ||
-            (e = cudaMemcpy(h->obs_index.p, oi.data(), oi.size() * sizeof(int), cudaMemcpyHostToDevice)) != cudaSuccess)
-            return bail(h->cuda_fail(e, "upload(obs_t)"));
+        cudaError_t e = cudaSuccess;
+        upload(e, h->obs_t, ot.data(), ot.size());
+        upload(e, h->obs_index, oi.data(), oi.size());
+        if (e != cudaSuccess) return bail(h->cuda_fail(e, "upload(obs_t)"));
         b.obs_t = h->obs_t.as<long long>();
         b.obs_index = h->obs_index.as<int>();
     }
@@ -407,51 +478,11 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
     }
     h->chunk = (int)chunk;
     {
-        cudaError_t e;
-        if ((e = h->sc_mt.alloc(sizeof(double) * chunk * N * D)) != cudaSuccess ||
-            (e = h->sc_st.alloc(sizeof(double) * chunk * N * D * D)) != cudaSuccess ||
-            (e = h->sc_dEm.alloc(sizeof(double) * chunk * N * D)) != cudaSuccess ||
-            (e = h->sc_dEs.alloc(sizeof(double) * chunk * N * D * D)) != cudaSuccess ||
-            (e = h->sc_esde.alloc(sizeof(double) * chunk * N)) != cudaSuccess ||
-            (e = h->status.alloc(sizeof(int) * B)) != cudaSuccess ||
-            (e = cudaMemset(h->status.p, 0, sizeof(int) * B)) != cudaSuccess)
-            return bail(h->cuda_fail(e, "cudaMalloc(scratch)"));
+        cudaError_t e = h->sc.alloc(chunk, N, D);
+        alloc<int>(e, h->status, B);
+        if (e == cudaSuccess) e = cudaMemset(h->status.p, 0, sizeof(int) * B);
+        if (e != cudaSuccess) return bail(h->cuda_fail(e, "cudaMalloc(scratch)"));
     }
-    {
-        const char* env = getenv("VGPA_LANES");
-        int want = env ? atoi(env) : 1;   // VGPA_LANES=2: measured +2 % (18.6k -> 19.0k evals/s) for 2x scratch; off by default
-                                          // (per-kernel timings of overlapping kernels would also stop being meaningful)
-        h->lanes = (!small_model(d->model) && B > chunk && want >= 2) ? 2 : 1;
-        if (h->lanes == 2) {
-            cudaError_t e;
-            if ((e = h->sc2_mt.alloc(sizeof(double) * chunk * N * D)) != cudaSuccess ||
-                (e = h->sc2_st.alloc(sizeof(double) * chunk * N * D * D)) != cudaSuccess ||
-                (e = h->sc2_dEm.alloc(sizeof(double) * chunk * N * D)) != cudaSuccess ||
-                (e = h->sc2_dEs.alloc(sizeof(double) * chunk * N * D * D)) != cudaSuccess ||
-                (e = h->sc2_esde.alloc(sizeof(double) * chunk * N)) != cudaSuccess ||
-                (e = cudaStreamCreateWithFlags(&h->s_lane[0], cudaStreamNonBlocking)) != cudaSuccess ||
-                (e = cudaStreamCreateWithFlags(&h->s_lane[1], cudaStreamNonBlocking)) != cudaSuccess ||
-                (e = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming)) != cudaSuccess ||
-                (e = cudaEventCreateWithFlags(&h->ev_join[0], cudaEventDisableTiming)) != cudaSuccess ||
-                (e = cudaEventCreateWithFlags(&h->ev_join[1], cudaEventDisableTiming)) != cudaSuccess) {
-                cudaGetLastError();
-                h->lanes = 1;   // not enough memory for a second lane: run the chunks back to back
-                for (DevBuf* q : {&h->sc2_mt, &h->sc2_st, &h->sc2_dEm, &h->sc2_dEs, &h->sc2_esde}) q->release();
-            }
-        }
-        h->scratch2.mt = h->sc2_mt.as<double>();
-        h->scratch2.st = h->sc2_st.as<double>();
-        h->scratch2.dEm = h->sc2_dEm.as<double>();
-        h->scratch2.dEs = h->sc2_dEs.as<double>();
-        h->scratch2.esde_t = h->sc2_esde.as<double>();
-        h->scratch2.status = h->status.as<int>();
-    }
-    h->scratch.mt = h->sc_mt.as<double>();
-    h->scratch.st = h->sc_st.as<double>();
-    h->scratch.dEm = h->sc_dEm.as<double>();
-    h->scratch.dEs = h->sc_dEs.as<double>();
-    h->scratch.esde_t = h->sc_esde.as<double>();
-    h->scratch.status = h->status.as<int>();
     {
         cudaError_t e;
         if ((e = cudaStreamCreateWithFlags(&h->s_comp, cudaStreamNonBlocking)) != cudaSuccess ||
@@ -473,11 +504,6 @@ void vgpa_destroy(vgpa_handle* h)
     if (!h) return;
     cudaSetDevice(h->d.device);
     cudaDeviceSynchronize();
-    for (DevBuf* b : {&h->theta, &h->sigma, &h->R, &h->obs_t, &h->obs_index, &h->obs_y, &h->m0, &h->s0, &h->E0,
-                      &h->status, &h->sc_mt, &h->sc_st, &h->sc_dEm, &h->sc_dEs, &h->sc_esde, &h->sc2_mt, &h->sc2_st,
-                      &h->sc2_dEm, &h->sc2_dEs, &h->sc2_esde, &h->st_x[0],
-                      &h->st_x[1], &h->st_g[0], &h->st_g[1], &h->st_F, &h->plist2[0], &h->plist2[1]})
-        b->release();
     if (h->s_aux) cudaStreamDestroy(h->s_aux);
     for (int q = 0; q < 2; ++q)
         if (h->plist_ev[q]) cudaEventDestroy(h->plist_ev[q]);
@@ -491,16 +517,11 @@ void vgpa_destroy(vgpa_handle* h)
             cudaEventDestroy(pr.first);
             cudaEventDestroy(pr.second);
         }
-    for (int q = 0; q < 2; ++q) {
-        if (h->s_lane[q]) cudaStreamDestroy(h->s_lane[q]);
-        if (h->ev_join[q]) cudaEventDestroy(h->ev_join[q]);
-    }
-    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_done) cudaEventDestroy(h->ev_done);
     if (h->s_comp) cudaStreamDestroy(h->s_comp);
     if (h->s_h2d) cudaStreamDestroy(h->s_h2d);
     if (h->s_d2h) cudaStreamDestroy(h->s_d2h);
-    delete h;
+    delete h;   // frees the device buffers, with the handle's device current
 }
 
 int vgpa_eval_device(vgpa_handle* h, const double* d_x, int64_t x_stride, int want_grad, double* d_F,
@@ -523,24 +544,9 @@ int vgpa_eval_device(vgpa_handle* h, const double* d_x, int64_t x_stride, int wa
     CK(cudaMemsetAsync(h->status.p, 0, sizeof(int) * h->d.B, st), "cudaMemsetAsync(status)");
     Extra ex{};
     const int total = (h->n_list >= 0 && h->batch.plist != nullptr) ? h->n_list : h->d.B;   // launch positions
-    if (h->lanes == 2) {
-        CK(cudaEventRecord(h->ev_fork, st), "cudaEventRecord");
-        CK(cudaStreamWaitEvent(h->s_lane[0], h->ev_fork, 0), "cudaStreamWaitEvent");
-        CK(cudaStreamWaitEvent(h->s_lane[1], h->ev_fork, 0), "cudaStreamWaitEvent");
-        int ci = 0;
-        for (int p0 = 0; p0 < total; p0 += h->chunk, ++ci) {
-            const int count = std::min(h->chunk, total - p0);
-            run_chunk(h, d_x, x_stride, want_grad, d_F, d_grad, grad_stride, p0, count, ex, h->s_lane[ci & 1], ci & 1);
-        }
-        for (int q = 0; q < 2; ++q) {
-            CK(cudaEventRecord(h->ev_join[q], h->s_lane[q]), "cudaEventRecord");
-            CK(cudaStreamWaitEvent(st, h->ev_join[q], 0), "cudaStreamWaitEvent");
-        }
-    } else {
-        for (int p0 = 0; p0 < total; p0 += h->chunk) {
-            const int count = std::min(h->chunk, total - p0);
-            run_chunk(h, d_x, x_stride, want_grad, d_F, d_grad, grad_stride, p0, count, ex, st);
-        }
+    for (int p0 = 0; p0 < total; p0 += h->chunk) {
+        const int count = std::min(h->chunk, total - p0);
+        run_chunk(h, d_x, x_stride, want_grad, d_F, d_grad, grad_stride, p0, count, ex, st);
     }
     CK(cudaGetLastError(), "kernel launch");
     if (h->batch.plist != nullptr && h->n_list >= 0) {   // this evaluation reads the current copy of the list
@@ -703,16 +709,16 @@ int vgpa_eval_full(vgpa_handle* h, int64_t problem, const double* x, const vgpa_
     HostCallScope scope(h);
     const long long nx = h->n_x, N = h->d.N, D = h->d.D, nv = N * D, nm = N * D * D;
     DevBuf dx, dg, dF, dl, dp, def, dedf, dparts;
-    auto cleanup = [&]() { for (DevBuf* b : {&dx, &dg, &dF, &dl, &dp, &def, &dedf, &dparts}) b->release(); };
-    cudaError_t e;
-    if ((e = dx.alloc(sizeof(double) * nx)) != cudaSuccess || (e = dg.alloc(sizeof(double) * nx)) != cudaSuccess ||
-        (e = dF.alloc(sizeof(double) * h->d.B)) != cudaSuccess || (e = dl.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dp.alloc(sizeof(double) * nm)) != cudaSuccess || (e = def.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dedf.alloc(sizeof(double) * nm)) != cudaSuccess || (e = dparts.alloc(sizeof(double) * 3)) != cudaSuccess ||
-        (e = cudaMemcpy(dx.p, x, sizeof(double) * nx, cudaMemcpyHostToDevice)) != cudaSuccess) {
-        cleanup();
-        return h->cuda_fail(e, "vgpa_eval_full setup");
-    }
+    cudaError_t e = cudaSuccess;
+    upload(e, dx, x, nx);
+    alloc(e, dg, nx);
+    alloc(e, dF, h->d.B);
+    alloc(e, dl, nv);
+    alloc(e, dp, nm);
+    alloc(e, def, nv);
+    alloc(e, dedf, nm);
+    alloc(e, dparts, 3);
+    if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_eval_full setup");
     Extra ex{};
     ex.lamt = dl.as<double>(); ex.psit = dp.as<double>(); ex.Efx = def.as<double>(); ex.Edf = dedf.as<double>();
     ex.parts = dparts.as<double>();
@@ -722,25 +728,18 @@ int vgpa_eval_full(vgpa_handle* h, int64_t problem, const double* x, const vgpa_
               (int)problem, 1, ex, h->s_comp);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->s_comp);
-    if (e != cudaSuccess) {
-        cleanup();
-        return h->cuda_fail(e, "vgpa_eval_full kernels");
-    }
-    auto back = [&](double* dst, const void* src, long long n) {
-        if (dst && e == cudaSuccess) e = cudaMemcpy(dst, src, sizeof(double) * n, cudaMemcpyDeviceToHost);
-    };
-    back(out->F, dF.as<double>() + problem, 1);
-    back(out->parts, dparts.p, 3);
-    back(out->grad, dg.p, nx);
-    back(out->mt, h->scratch.mt, nv);
-    back(out->st, h->scratch.st, nm);
-    back(out->lamt, dl.p, nv);
-    back(out->psit, dp.p, nm);
-    back(out->Efx, def.p, nv);
-    back(out->Edf, dedf.p, nm);
-    back(out->dEsde_dm, h->scratch.dEm, nv);
-    back(out->dEsde_ds, h->scratch.dEs, nm);
-    cleanup();
+    if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_eval_full kernels");
+    download(e, out->F, dF.as<double>() + problem, 1);
+    download(e, out->parts, dparts.p, 3);
+    download(e, out->grad, dg.p, nx);
+    download(e, out->mt, h->sc.mt.p, nv);
+    download(e, out->st, h->sc.st.p, nm);
+    download(e, out->lamt, dl.p, nv);
+    download(e, out->psit, dp.p, nm);
+    download(e, out->Efx, def.p, nv);
+    download(e, out->Edf, dedf.p, nm);
+    download(e, out->dEsde_dm, h->sc.dEm.p, nv);
+    download(e, out->dEsde_ds, h->sc.dEs.p, nm);
     if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_eval_full copy-back");
     h->status_dirty = true;
     return check_status(h);
@@ -749,36 +748,31 @@ int vgpa_eval_full(vgpa_handle* h, int64_t problem, const double* x, const vgpa_
 // ---- stand-alone sweeps (FwdOde.__call__ / BwdOde.__call__) -------------------------
 static int check_sweep_args(int method, int D, int N, double dt)
 {
-    if (method < 0 || method > 3) { g_create_error = "Integration method is unknown"; return VGPA_EINVAL; }
-    if (D != 1 && D != 3 && D != 40) { g_create_error = "unsupported state dimension (1, 3 or 40)"; return VGPA_EINVAL; }
-    if (N < 2) { g_create_error = "need at least two time points"; return VGPA_EINVAL; }
-    if (!(dt > 0.0)) { g_create_error = "Discrete time step should be strictly positive"; return VGPA_EINVAL; }
+    if (method < 0 || method > 3) return set_error(VGPA_EINVAL, "Integration method is unknown");
+    if (D != 1 && D != 3 && D != 40) return set_error(VGPA_EINVAL, "unsupported state dimension (1, 3 or 40)");
+    if (N < 2) return set_error(VGPA_EINVAL, "need at least two time points");
+    if (!(dt > 0.0)) return set_error(VGPA_EINVAL, "Discrete time step should be strictly positive");
     return VGPA_OK;
 }
 
 int vgpa_solve_fwd(int device, int method, int D, int N, double dt, const double* A, const double* b,
                    const double* m0, const double* s0, const double* sigma, double* mt, double* st)
 {
-    int rc = check_sweep_args(method, D, N, dt);
-    if (rc) return rc;
-    if (!A || !b || !m0 || !s0 || !sigma || !mt || !st) { g_create_error = "NULL argument"; return VGPA_EINVAL; }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+    if (int rc = check_sweep_args(method, D, N, dt)) return rc;
+    if (!A || !b || !m0 || !s0 || !sigma || !mt || !st) return set_error(VGPA_EINVAL, "NULL argument");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const long long nv = (long long)N * D, nm = (long long)N * D * D;
     DevBuf dx, dm0, ds0, dsig, dmt, dst;
-    cudaError_t e;
-    auto cleanup = [&]() { for (DevBuf* q : {&dx, &dm0, &ds0, &dsig, &dmt, &dst}) q->release(); };
-    if ((e = dx.alloc(sizeof(double) * (nm + nv))) != cudaSuccess || (e = dm0.alloc(sizeof(double) * D)) != cudaSuccess ||
-        (e = ds0.alloc(sizeof(double) * D * D)) != cudaSuccess || (e = dsig.alloc(sizeof(double) * D)) != cudaSuccess ||
-        (e = dmt.alloc(sizeof(double) * nv)) != cudaSuccess || (e = dst.alloc(sizeof(double) * nm)) != cudaSuccess ||
-        (e = cudaMemcpy(dx.p, A, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dx.as<double>() + nm, b, sizeof(double) * nv, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dm0.p, m0, sizeof(double) * D, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(ds0.p, s0, sizeof(double) * D * D, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dsig.p, sigma, sizeof(double) * D, cudaMemcpyHostToDevice)) != cudaSuccess) {
-        cleanup();
-        g_create_error = std::string("CUDA error in vgpa_solve_fwd: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    cudaError_t e = cudaSuccess;
+    alloc(e, dx, nm + nv);
+    to_device(e, dx.as<double>(), A, nm);
+    to_device(e, dx.as<double>() + nm, b, nv);
+    upload(e, dm0, m0, D);
+    upload(e, ds0, s0, (size_t)D * D);
+    upload(e, dsig, sigma, D);
+    alloc(e, dmt, nv);
+    alloc(e, dst, nm);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_solve_fwd");
     Batch bt{};
     bt.model = (D == 40) ? MODEL_L96 : (D == 3 ? MODEL_L63 : MODEL_OU);
     bt.method = method; bt.D = D; bt.N = N; bt.B = 1; bt.dt = dt; bt.dt_model = dt;
@@ -789,96 +783,73 @@ int vgpa_solve_fwd(int device, int method, int D, int N, double dt, const double
     else launch_small_fwd(bt, sc, dx.as<double>(), 0, 0, 1, nullptr);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
-    if (e == cudaSuccess) e = cudaMemcpy(mt, dmt.p, sizeof(double) * nv, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(st, dst.p, sizeof(double) * nm, cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) {
-        g_create_error = std::string("CUDA error in vgpa_solve_fwd: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
-    return VGPA_OK;
+    download(e, mt, dmt.p, nv);
+    download(e, st, dst.p, nm);
+    return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_solve_fwd");
 }
 
 int vgpa_solve_bwd(int device, int method, int D, int N, double dt, const double* A, const double* dEm,
                    const double* dEs, const double* jm, const double* js, double* lam, double* psi)
 {
-    int rc = check_sweep_args(method, D, N, dt);
-    if (rc) return rc;
-    if (!A || !dEm || !dEs || !jm || !js || !lam || !psi) { g_create_error = "NULL argument"; return VGPA_EINVAL; }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+    if (int rc = check_sweep_args(method, D, N, dt)) return rc;
+    if (!A || !dEm || !dEs || !jm || !js || !lam || !psi) return set_error(VGPA_EINVAL, "NULL argument");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const long long nv = (long long)N * D, nm = (long long)N * D * D;
     DevBuf dA, dgm, dgs, djm, djs, dl, dp;
-    cudaError_t e;
-    auto cleanup = [&]() { for (DevBuf* q : {&dA, &dgm, &dgs, &djm, &djs, &dl, &dp}) q->release(); };
-    if ((e = dA.alloc(sizeof(double) * nm)) != cudaSuccess || (e = dgm.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dgs.alloc(sizeof(double) * nm)) != cudaSuccess || (e = djm.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = djs.alloc(sizeof(double) * nm)) != cudaSuccess || (e = dl.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dp.alloc(sizeof(double) * nm)) != cudaSuccess ||
-        (e = cudaMemcpy(dA.p, A, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dgm.p, dEm, sizeof(double) * nv, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dgs.p, dEs, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(djm.p, jm, sizeof(double) * nv, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(djs.p, js, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess) {
-        cleanup();
-        g_create_error = std::string("CUDA error in vgpa_solve_bwd: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    cudaError_t e = cudaSuccess;
+    upload(e, dA, A, nm);
+    upload(e, dgm, dEm, nv);
+    upload(e, dgs, dEs, nm);
+    upload(e, djm, jm, nv);
+    upload(e, djs, js, nm);
+    alloc(e, dl, nv);
+    alloc(e, dp, nm);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_solve_bwd");
     launch_bwd_dense(method, D, N, dt, dA.as<double>(), dgm.as<double>(), dgs.as<double>(), djm.as<double>(),
                      djs.as<double>(), dl.as<double>(), dp.as<double>(), nullptr);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
-    if (e == cudaSuccess) e = cudaMemcpy(lam, dl.p, sizeof(double) * nv, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(psi, dp.p, sizeof(double) * nm, cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) {
-        g_create_error = std::string("CUDA error in vgpa_solve_bwd: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
-    return VGPA_OK;
+    download(e, lam, dl.p, nv);
+    download(e, psi, dp.p, nm);
+    return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_solve_bwd");
 }
 
 int vgpa_model_energy(int device, int model, int D, int N, double dt_model, const double* theta,
                       const double* sigma, const double* A, const double* b, const double* m, const double* S,
                       double* Esde, double* Ef, double* Edf, double* dEm, double* dEs, double* dEth, double* dEsig)
 {
-    if (model < 0 || model > 3) { g_create_error = "Unknown stochastic model"; return VGPA_EINVAL; }
+    if (model < 0 || model > 3) return set_error(VGPA_EINVAL, "Unknown stochastic model");
     const int needD = (model == VGPA_MODEL_L63) ? 3 : (model == VGPA_MODEL_L96 ? 40 : 1);
-    if (D != needD || N < 2 || !(dt_model > 0.0)) { g_create_error = "Wrong dimensions for model.energy"; return VGPA_EINVAL; }
-    if (!theta || !sigma || !A || !b || !m || !S || !Esde || !Ef || !Edf || !dEm || !dEs) {
-        g_create_error = "NULL argument";
-        return VGPA_EINVAL;
-    }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+    if (D != needD || N < 2 || !(dt_model > 0.0)) return set_error(VGPA_EINVAL, "Wrong dimensions for model.energy");
+    if (!theta || !sigma || !A || !b || !m || !S || !Esde || !Ef || !Edf || !dEm || !dEs)
+        return set_error(VGPA_EINVAL, "NULL argument");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const long long nv = (long long)N * D, nm = (long long)N * D * D;
     const int nth = n_theta(model);
     DevBuf dx, dth, dsig, dmt, dst, dgm, dgs, des, def, dedf, dparts, dzero, dF, dstat, dft, dfs, dhth, dhsig;
-    auto cleanup = [&]() {
-        for (DevBuf* q : {&dx, &dth, &dsig, &dmt, &dst, &dgm, &dgs, &des, &def, &dedf, &dparts, &dzero, &dF, &dstat,
-                          &dft, &dfs, &dhth, &dhsig})
-            q->release();
-    };
     const bool hyper = (dEth != nullptr) || (dEsig != nullptr);
     const int nhth = (model == VGPA_MODEL_L96) ? D : nth;   // lorenz_96.py:431: one entry per state dimension
     const long long nsig = (D == 1) ? 1 : (long long)D * D;
-    cudaError_t e;
-    if ((e = dx.alloc(sizeof(double) * (nm + nv))) != cudaSuccess || (e = dth.alloc(sizeof(double) * nth)) != cudaSuccess ||
-        (e = dsig.alloc(sizeof(double) * D)) != cudaSuccess || (e = dmt.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dst.alloc(sizeof(double) * nm)) != cudaSuccess || (e = dgm.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dgs.alloc(sizeof(double) * nm)) != cudaSuccess || (e = des.alloc(sizeof(double) * N)) != cudaSuccess ||
-        (e = def.alloc(sizeof(double) * nv)) != cudaSuccess || (e = dedf.alloc(sizeof(double) * nm)) != cudaSuccess ||
-        (e = dparts.alloc(sizeof(double) * 3)) != cudaSuccess || (e = dzero.alloc(sizeof(double))) != cudaSuccess ||
-        (e = dF.alloc(sizeof(double))) != cudaSuccess || (e = dstat.alloc(sizeof(int))) != cudaSuccess ||
-        (e = cudaMemset(dzero.p, 0, sizeof(double))) != cudaSuccess || (e = cudaMemset(dstat.p, 0, sizeof(int))) != cudaSuccess ||
-        (e = cudaMemcpy(dx.p, A, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dx.as<double>() + nm, b, sizeof(double) * nv, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dth.p, theta, sizeof(double) * nth, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dsig.p, sigma, sizeof(double) * D, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dmt.p, m, sizeof(double) * nv, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dst.p, S, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess) {
-        cleanup();
-        g_create_error = std::string("CUDA error in vgpa_model_energy: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    cudaError_t e = cudaSuccess;
+    alloc(e, dx, nm + nv);
+    to_device(e, dx.as<double>(), A, nm);
+    to_device(e, dx.as<double>() + nm, b, nv);
+    upload(e, dth, theta, nth);
+    upload(e, dsig, sigma, D);
+    upload(e, dmt, m, nv);
+    upload(e, dst, S, nm);
+    alloc(e, dgm, nv);
+    alloc(e, dgs, nm);
+    alloc(e, des, N);
+    alloc(e, def, nv);
+    alloc(e, dedf, nm);
+    alloc(e, dparts, 3);
+    alloc(e, dzero, 1);
+    alloc(e, dF, 1);
+    alloc<int>(e, dstat, 1);
+    if (e == cudaSuccess) e = cudaMemset(dzero.p, 0, sizeof(double));
+    if (e == cudaSuccess) e = cudaMemset(dstat.p, 0, sizeof(int));
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_model_energy");
     Batch bt{};
     bt.model = model; bt.method = ODE_EULER; bt.D = D; bt.N = N; bt.M = 0; bt.B = 1;
     bt.dt = dt_model; bt.dt_model = dt_model;
@@ -893,12 +864,11 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
     else launch_small_energy(bt, sc, dx.as<double>(), 0, 0, 1, ex, nullptr);
     launch_finalize(bt, sc, dF.as<double>(), 0, 1, ex, nullptr);
     if (hyper) {
-        if ((e = dft.alloc(sizeof(double) * (size_t)N * nhth)) != cudaSuccess || (e = dfs.alloc(sizeof(double) * nv)) != cudaSuccess ||
-            (e = dhth.alloc(sizeof(double) * nhth)) != cudaSuccess || (e = dhsig.alloc(sizeof(double) * nsig)) != cudaSuccess) {
-            cleanup();
-            g_create_error = std::string("CUDA error in vgpa_model_energy: ") + cudaGetErrorString(e);
-            return VGPA_ECUDA;
-        }
+        alloc(e, dft, (size_t)N * nhth);
+        alloc(e, dfs, nv);
+        alloc(e, dhth, nhth);
+        alloc(e, dhsig, nsig);
+        if (e != cudaSuccess) return set_cuda_error(e, "vgpa_model_energy");
         // parts[1] = Esde (written by finalize on the same stream)
         launch_hyper(model, D, N, dt_model, dth.as<double>(), dsig.as<double>(), dx.as<double>(), dmt.as<double>(),
                      dst.as<double>(), dparts.as<double>() + 1, dft.as<double>(), dfs.as<double>(),
@@ -908,25 +878,16 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     double parts[3] = {0, 0, 0};
     int stat = 0;
-    if (e == cudaSuccess) e = cudaMemcpy(parts, dparts.p, sizeof parts, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(&stat, dstat.p, sizeof stat, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && dEth) e = cudaMemcpy(dEth, dhth.p, sizeof(double) * nhth, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && dEsig) e = cudaMemcpy(dEsig, dhsig.p, sizeof(double) * nsig, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(Ef, def.p, sizeof(double) * nv, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(Edf, dedf.p, sizeof(double) * nm, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(dEm, dgm.p, sizeof(double) * nv, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(dEs, dgs.p, sizeof(double) * nm, cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) {
-        g_create_error = std::string("CUDA error in vgpa_model_energy: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
-    if (stat != 0) {
-        char buf[128];
-        snprintf(buf, sizeof buf, "Matrix is not positive definite: S(t) at time index %d", stat - 1);
-        g_create_error = buf;
-        return VGPA_ENOTPD;
-    }
+    download(e, parts, dparts.p, 3);
+    download(e, &stat, dstat.p, 1);
+    download(e, dEth, dhth.p, nhth);
+    download(e, dEsig, dhsig.p, nsig);
+    download(e, Ef, def.p, nv);
+    download(e, Edf, dedf.p, nm);
+    download(e, dEm, dgm.p, nv);
+    download(e, dEs, dgs.p, nm);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_model_energy");
+    if (stat != 0) return set_error(VGPA_ENOTPD, "Matrix is not positive definite: S(t) at time index %d", stat - 1);
     *Esde = parts[1];
     return VGPA_OK;
 }
@@ -934,33 +895,31 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
 int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const double* obs_y, const double* R,
                     const double* mt, const double* st, double* Eobs, double* jm, double* js, double* dr)
 {
-    if ((D != 1 && D != 3 && D != 40) || N < 2 || M < 0 || M > N) { g_create_error = "Wrong dimensions for the likelihood"; return VGPA_EINVAL; }
-    if ((M > 0 && (!obs_t || !obs_y)) || !R || !mt || !st || !Eobs || !jm || !js) { g_create_error = "NULL argument"; return VGPA_EINVAL; }
+    if ((D != 1 && D != 3 && D != 40) || N < 2 || M < 0 || M > N) return set_error(VGPA_EINVAL, "Wrong dimensions for the likelihood");
+    if ((M > 0 && (!obs_t || !obs_y)) || !R || !mt || !st || !Eobs || !jm || !js) return set_error(VGPA_EINVAL, "NULL argument");
     for (int n = 0; n < M; ++n)
-        if (obs_t[n] < 0 || obs_t[n] >= N) { g_create_error = "observation index out of range"; return VGPA_EINVAL; }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+        if (obs_t[n] < 0 || obs_t[n] >= N) return set_error(VGPA_EINVAL, "observation index out of range");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const long long nv = (long long)N * D, nm = (long long)N * D * D;
     DevBuf dot, doy, dR, dmt, dst, djm, djs, des, dparts, dzero, dF, ddr;
-    auto cleanup = [&]() { for (DevBuf* q : {&dot, &doy, &dR, &dmt, &dst, &djm, &djs, &des, &dparts, &dzero, &dF, &ddr}) q->release(); };
     std::vector<long long> ot(std::max(M, 1), 0);
     for (int n = 0; n < M; ++n) ot[n] = obs_t[n];
-    cudaError_t e;
-    if ((e = dot.alloc(sizeof(long long) * ot.size())) != cudaSuccess || (e = doy.alloc(sizeof(double) * std::max(M, 1) * D)) != cudaSuccess ||
-        (e = dR.alloc(sizeof(double) * D)) != cudaSuccess || (e = dmt.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = dst.alloc(sizeof(double) * nm)) != cudaSuccess || (e = djm.alloc(sizeof(double) * nv)) != cudaSuccess ||
-        (e = djs.alloc(sizeof(double) * nm)) != cudaSuccess || (e = des.alloc(sizeof(double) * N)) != cudaSuccess ||
-        (e = dparts.alloc(sizeof(double) * 3)) != cudaSuccess || (e = dzero.alloc(sizeof(double))) != cudaSuccess ||
-        (e = dF.alloc(sizeof(double))) != cudaSuccess ||
-        (e = cudaMemset(dzero.p, 0, sizeof(double))) != cudaSuccess || (e = cudaMemset(des.p, 0, sizeof(double) * N)) != cudaSuccess ||
-        (e = cudaMemcpy(dot.p, ot.data(), sizeof(long long) * ot.size(), cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (M > 0 && (e = cudaMemcpy(doy.p, obs_y, sizeof(double) * M * D, cudaMemcpyHostToDevice)) != cudaSuccess) ||
-        (e = cudaMemcpy(dR.p, R, sizeof(double) * D, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dmt.p, mt, sizeof(double) * nv, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = cudaMemcpy(dst.p, st, sizeof(double) * nm, cudaMemcpyHostToDevice)) != cudaSuccess) {
-        cleanup();
-        g_create_error = std::string("CUDA error in vgpa_obs_energy: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    cudaError_t e = cudaSuccess;
+    upload(e, dot, ot.data(), ot.size());
+    alloc(e, doy, (size_t)std::max(M, 1) * D);
+    if (M > 0) to_device(e, doy.p, obs_y, (size_t)M * D);
+    upload(e, dR, R, D);
+    upload(e, dmt, mt, nv);
+    upload(e, dst, st, nm);
+    alloc(e, djm, nv);
+    alloc(e, djs, nm);
+    alloc(e, des, N);
+    alloc(e, dparts, 3);
+    alloc(e, dzero, 1);
+    alloc(e, dF, 1);
+    if (e == cudaSuccess) e = cudaMemset(dzero.p, 0, sizeof(double));
+    if (e == cudaSuccess) e = cudaMemset(des.p, 0, sizeof(double) * N);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_obs_energy");
     Batch bt{};
     bt.model = (D == 1) ? MODEL_OU : (D == 3 ? MODEL_L63 : MODEL_L96);
     bt.D = D; bt.N = N; bt.M = M; bt.B = 1; bt.dt = 1.0; bt.dt_model = 1.0;
@@ -974,29 +933,22 @@ int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const
     launch_jump_tables(D, N, M, dot.as<long long>(), doy.as<double>(), dR.as<double>(), dmt.as<double>(),
                        djm.as<double>(), djs.as<double>(), nullptr);
     if (dr != nullptr && D == 1) {
-        if ((e = ddr.alloc(sizeof(double) * N)) != cudaSuccess) {
-            cleanup();
-            g_create_error = std::string("CUDA error in vgpa_obs_energy: ") + cudaGetErrorString(e);
-            return VGPA_ECUDA;
-        }
+        alloc(e, ddr, N);
+        if (e != cudaSuccess) return set_cuda_error(e, "vgpa_obs_energy");
         launch_obs_dr(N, M, dot.as<long long>(), doy.as<double>(), dR.as<double>(), dmt.as<double>(), dst.as<double>(),
                       ddr.as<double>(), nullptr);
     }
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     double parts[3] = {0, 0, 0};
-    if (e == cudaSuccess) e = cudaMemcpy(parts, dparts.p, sizeof parts, cudaMemcpyDeviceToHost);
+    download(e, parts, dparts.p, 3);
     if (e == cudaSuccess && dr != nullptr) {
-        if (D == 1) e = cudaMemcpy(dr, ddr.p, sizeof(double) * N, cudaMemcpyDeviceToHost);
+        if (D == 1) download(e, dr, ddr.p, N);
         else std::fill(dr, dr + (size_t)N * M * M, 0.0);   // the reference's n-D branch returns zeros (gaussian_like.py:226)
     }
-    if (e == cudaSuccess) e = cudaMemcpy(jm, djm.p, sizeof(double) * nv, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(js, djs.p, sizeof(double) * nm, cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) {
-        g_create_error = std::string("CUDA error in vgpa_obs_energy: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    download(e, jm, djm.p, nv);
+    download(e, js, djs.p, nm);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_obs_energy");
     *Eobs = parts[2];
     return VGPA_OK;
 }
@@ -1017,19 +969,17 @@ int vgpa_initialization(vgpa_handle* h, double t0, double* d_x, int64_t x_stride
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int B = h->d.B, D = h->d.D, n = h->d.M + 2;
     DevBuf scratch, err;
-    cudaError_t e;
-    if ((e = scratch.alloc(sizeof(double) * (size_t)B * D * 2 * n)) != cudaSuccess || (e = err.alloc(sizeof(int))) != cudaSuccess ||
-        (e = cudaMemsetAsync(err.p, 0, sizeof(int), st)) != cudaSuccess) {
-        scratch.release(); err.release();
-        return h->cuda_fail(e, "vgpa_initialization");
-    }
+    cudaError_t e = cudaSuccess;
+    alloc(e, scratch, (size_t)B * D * 2 * n);
+    alloc<int>(e, err, 1);
+    if (e == cudaSuccess) e = cudaMemsetAsync(err.p, 0, sizeof(int), st);
+    if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_initialization");
     launch_initialization(h->batch, 0, B, t0, scratch.as<double>(), d_x, x_stride, err.as<int>(), st);
     h->launches += 2;
     int bad = 0;
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(&bad, err.p, sizeof(int), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // the scratch is released below
-    scratch.release(); err.release();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // the scratch is released on return
     if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_initialization");
     if (bad) return h->fail(VGPA_EINVAL, "`x` must be strictly increasing sequence: an observation sits at the first or last grid index");
     return VGPA_OK;
@@ -1044,13 +994,12 @@ int vgpa_initialization_host(vgpa_handle* h, double t0, double* x, int64_t x_str
     const long long nx = h->n_x;
     const int C = std::max(1, std::min(B, 64));
     DevBuf scratch, err, dx;
-    auto cleanup = [&]() { scratch.release(); err.release(); dx.release(); };
-    cudaError_t e;
-    if ((e = scratch.alloc(sizeof(double) * (size_t)C * D * 2 * n)) != cudaSuccess || (e = err.alloc(sizeof(int))) != cudaSuccess ||
-        (e = dx.alloc(sizeof(double) * (size_t)C * nx)) != cudaSuccess || (e = cudaMemset(err.p, 0, sizeof(int))) != cudaSuccess) {
-        cleanup();
-        return h->cuda_fail(e, "vgpa_initialization_host");
-    }
+    cudaError_t e = cudaSuccess;
+    alloc(e, scratch, (size_t)C * D * 2 * n);
+    alloc<int>(e, err, 1);
+    alloc(e, dx, (size_t)C * nx);
+    if (e == cudaSuccess) e = cudaMemset(err.p, 0, sizeof(int));
+    if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_initialization_host");
     for (int p0 = 0; p0 < B && e == cudaSuccess; p0 += C) {
         const int count = std::min(C, B - p0);
         // kernels index problems globally: offset the staging pointer accordingly
@@ -1064,8 +1013,7 @@ int vgpa_initialization_host(vgpa_handle* h, double t0, double* x, int64_t x_str
         if (e == cudaSuccess) e = cudaStreamSynchronize(h->s_comp);
     }
     int bad = 0;
-    if (e == cudaSuccess) e = cudaMemcpy(&bad, err.p, sizeof(int), cudaMemcpyDeviceToHost);
-    cleanup();
+    download(e, &bad, err.p, 1);
     if (e != cudaSuccess) return h->cuda_fail(e, "vgpa_initialization_host");
     if (bad) return h->fail(VGPA_EINVAL, "`x` must be strictly increasing sequence: an observation sits at the first or last grid index");
     return VGPA_OK;
@@ -1078,15 +1026,14 @@ static int traj_ntheta(int model) { return model == VGPA_MODEL_L63 ? 3 : (model 
 static int check_traj_args(int model, int N, int B, double dt, const void* theta, const void* sigma,
                            const void* x_init, const void* z, const void* path, int64_t z_stride, int64_t path_stride)
 {
-    if (model < 0 || model > 3) { g_create_error = "Unknown stochastic model"; return VGPA_EINVAL; }
+    if (model < 0 || model > 3) return set_error(VGPA_EINVAL, "Unknown stochastic model");
     const int D = model_dim(model);
-    if (N < 1 || B < 1) { g_create_error = "need N >= 1 time points and B >= 1 paths"; return VGPA_EINVAL; }
-    if (!(dt > 0.0)) { g_create_error = "Discrete time step should be strictly positive"; return VGPA_EINVAL; }
-    if (!theta || !sigma || !z || !path) { g_create_error = "NULL argument"; return VGPA_EINVAL; }
-    if (D == 1 && !x_init) { g_create_error = "x_init is required for the 1-D models"; return VGPA_EINVAL; }
-    if ((z_stride != 0 && z_stride < (int64_t)N * D) || (B > 1 && path_stride < (int64_t)N * D)) {
-        g_create_error = "z_stride / path_stride shorter than one path"; return VGPA_EINVAL;
-    }
+    if (N < 1 || B < 1) return set_error(VGPA_EINVAL, "need N >= 1 time points and B >= 1 paths");
+    if (!(dt > 0.0)) return set_error(VGPA_EINVAL, "Discrete time step should be strictly positive");
+    if (!theta || !sigma || !z || !path) return set_error(VGPA_EINVAL, "NULL argument");
+    if (D == 1 && !x_init) return set_error(VGPA_EINVAL, "x_init is required for the 1-D models");
+    if ((z_stride != 0 && z_stride < (int64_t)N * D) || (B > 1 && path_stride < (int64_t)N * D))
+        return set_error(VGPA_EINVAL, "z_stride / path_stride shorter than one path");
     return VGPA_OK;
 }
 
@@ -1095,24 +1042,12 @@ int vgpa_make_trajectory_device(int device, int model, int N, int B, double dt, 
                                 const double* d_z, int64_t z_stride, double* d_path, int64_t path_stride, void* stream)
 {
     if (int rc = check_traj_args(model, N, B, dt, d_theta, d_sigma, d_x_init, d_z, d_path, z_stride, path_stride)) return rc;
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     TrajArgs a{model, model_dim(model), N, B, dt, d_theta, theta_stride, d_sigma, sigma_stride, d_x_init, x_init_stride,
                d_z, z_stride, d_path, path_stride};
     launch_trajectories(a, static_cast<cudaStream_t>(stream));
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { g_create_error = std::string("CUDA error in vgpa_make_trajectory_device: ") + cudaGetErrorString(e); return VGPA_ECUDA; }
-    return VGPA_OK;
-}
-
-// copy `rows` rows of `len` elements, `stride` apart (0 = one shared row), to a compact device buffer
-static cudaError_t stage_rows(DevBuf& dst, const double* src, int64_t stride, int64_t len, int rows, long long* dstride)
-{
-    const int r = stride == 0 ? 1 : rows;
-    cudaError_t e = dst.alloc(sizeof(double) * (size_t)len * r);
-    if (e != cudaSuccess) return e;
-    *dstride = stride == 0 ? 0 : len;
-    if (r == 1 || stride == len) return cudaMemcpy(dst.p, src, sizeof(double) * (size_t)len * r, cudaMemcpyHostToDevice);
-    return cudaMemcpy2D(dst.p, sizeof(double) * len, src, sizeof(double) * stride, sizeof(double) * len, r, cudaMemcpyHostToDevice);
+    return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_make_trajectory_device");
 }
 
 int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const double* theta, int64_t theta_stride,
@@ -1121,27 +1056,21 @@ int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const d
 {
     if (int rc = check_traj_args(model, N, B, dt, theta, sigma, x_init, z, path, z_stride, path_stride)) return rc;
     if ((theta_stride != 0 && theta_stride < traj_ntheta(model)) || (sigma_stride != 0 && sigma_stride < model_dim(model)) ||
-        (x_init && x_init_stride != 0 && x_init_stride < model_dim(model))) {
-        g_create_error = "theta_stride / sigma_stride / x_init_stride shorter than one entry (0 = shared)";
-        return VGPA_EINVAL;
-    }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+        (x_init && x_init_stride != 0 && x_init_stride < model_dim(model)))
+        return set_error(VGPA_EINVAL, "theta_stride / sigma_stride / x_init_stride shorter than one entry (0 = shared)");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const int D = model_dim(model);
     const int64_t len = (int64_t)N * D;
     DevBuf dth, dsg, dxi, dz, dp;
-    auto cleanup = [&]() { for (DevBuf* q : {&dth, &dsg, &dxi, &dz, &dp}) q->release(); };
     TrajArgs a{};
     a.model = model; a.D = D; a.N = N; a.B = B; a.dt = dt;
-    cudaError_t e;
-    if ((e = stage_rows(dth, theta, theta_stride, traj_ntheta(model), B, &a.theta_stride)) != cudaSuccess ||
-        (e = stage_rows(dsg, sigma, sigma_stride, D, B, &a.sigma_stride)) != cudaSuccess ||
-        (x_init && (e = stage_rows(dxi, x_init, x_init_stride, D, B, &a.x_init_stride)) != cudaSuccess) ||
-        (e = stage_rows(dz, z, z_stride, len, B, &a.z_stride)) != cudaSuccess ||
-        (e = dp.alloc(sizeof(double) * (size_t)len * B)) != cudaSuccess) {
-        cleanup();
-        g_create_error = std::string("CUDA error in vgpa_make_trajectory: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    cudaError_t e = cudaSuccess;
+    stage_rows(e, dth, theta, theta_stride, traj_ntheta(model), B, &a.theta_stride);
+    stage_rows(e, dsg, sigma, sigma_stride, D, B, &a.sigma_stride);
+    if (x_init) stage_rows(e, dxi, x_init, x_init_stride, D, B, &a.x_init_stride);
+    stage_rows(e, dz, z, z_stride, len, B, &a.z_stride);
+    alloc(e, dp, (size_t)len * B);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_make_trajectory");
     a.theta = dth.as<double>(); a.sigma = dsg.as<double>(); a.x_init = x_init ? dxi.as<double>() : nullptr;
     a.z = dz.as<double>(); a.path = dp.as<double>(); a.path_stride = len;
     launch_trajectories(a, nullptr);
@@ -1150,17 +1079,15 @@ int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const d
     if (e == cudaSuccess)
         e = cudaMemcpy2D(path, sizeof(double) * (B > 1 ? path_stride : len), dp.p, sizeof(double) * len, sizeof(double) * len, B,
                          cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) { g_create_error = std::string("CUDA error in vgpa_make_trajectory: ") + cudaGetErrorString(e); return VGPA_ECUDA; }
-    return VGPA_OK;
+    return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_make_trajectory");
 }
 
 static int check_obs_args(int D, int N, int M, int B, const int64_t* obs_t /* host, or NULL = not checked */)
 {
-    if (D != 1 && D != 3 && D != 40) { g_create_error = "unsupported state dimension (1, 3 or 40)"; return VGPA_EINVAL; }
-    if (N < 1 || M < 0 || B < 1) { g_create_error = "need N >= 1, M >= 0, B >= 1"; return VGPA_EINVAL; }
+    if (D != 1 && D != 3 && D != 40) return set_error(VGPA_EINVAL, "unsupported state dimension (1, 3 or 40)");
+    if (N < 1 || M < 0 || B < 1) return set_error(VGPA_EINVAL, "need N >= 1, M >= 0, B >= 1");
     for (int j = 0; obs_t && j < M; ++j)
-        if (obs_t[j] < 0 || obs_t[j] >= N) { g_create_error = "observation index outside the time grid"; return VGPA_EINVAL; }
+        if (obs_t[j] < 0 || obs_t[j] >= N) return set_error(VGPA_EINVAL, "observation index outside the time grid");
     return VGPA_OK;
 }
 
@@ -1169,45 +1096,37 @@ int vgpa_collect_obs_device(int device, int D, int N, int M, int B, const int64_
                             double* d_obs_y, int64_t obs_y_stride, void* stream)
 {
     if (int rc = check_obs_args(D, N, M, B, nullptr)) return rc;
-    if (!d_obs_t || !d_R || !d_path || !d_xi || !d_obs_y) { g_create_error = "NULL argument"; return VGPA_EINVAL; }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+    if (!d_obs_t || !d_R || !d_path || !d_xi || !d_obs_y) return set_error(VGPA_EINVAL, "NULL argument");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     ObsArgs a{D, N, M, B, reinterpret_cast<const long long*>(d_obs_t), d_R, R_stride, d_path, path_stride, d_xi, xi_stride,
               d_obs_y, obs_y_stride};
     launch_collect_obs(a, static_cast<cudaStream_t>(stream));
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { g_create_error = std::string("CUDA error in vgpa_collect_obs_device: ") + cudaGetErrorString(e); return VGPA_ECUDA; }
-    return VGPA_OK;
+    return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_collect_obs_device");
 }
 
 int vgpa_collect_obs(int device, int D, int N, int M, int B, const int64_t* obs_t, const double* R, int64_t R_stride,
                      const double* path, int64_t path_stride, const double* xi, int64_t xi_stride, double* obs_y,
                      int64_t obs_y_stride)
 {
-    if (!obs_t || !R || !path || !xi || !obs_y) { g_create_error = "NULL argument"; return VGPA_EINVAL; }
+    if (!obs_t || !R || !path || !xi || !obs_y) return set_error(VGPA_EINVAL, "NULL argument");
     if (int rc = check_obs_args(D, N, M, B, obs_t)) return rc;
     if (M == 0) return VGPA_OK;
     if ((R_stride != 0 && R_stride < D) || (path_stride != 0 && path_stride < (int64_t)N * D) ||
-        (xi_stride != 0 && xi_stride < (int64_t)M * D) || (B > 1 && obs_y_stride < (int64_t)M * D)) {
-        g_create_error = "R_stride / path_stride / xi_stride / obs_y_stride shorter than one entry (0 = shared)";
-        return VGPA_EINVAL;
-    }
-    if (cudaSetDevice(device) != cudaSuccess) { g_create_error = "cudaSetDevice failed"; return VGPA_ECUDA; }
+        (xi_stride != 0 && xi_stride < (int64_t)M * D) || (B > 1 && obs_y_stride < (int64_t)M * D))
+        return set_error(VGPA_EINVAL, "R_stride / path_stride / xi_stride / obs_y_stride shorter than one entry (0 = shared)");
+    if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const int64_t plen = (int64_t)N * D, olen = (int64_t)M * D;
     DevBuf dt_, dR, dp, dx, dy;
-    auto cleanup = [&]() { for (DevBuf* q : {&dt_, &dR, &dp, &dx, &dy}) q->release(); };
     ObsArgs a{};
     a.D = D; a.N = N; a.M = M; a.B = B;
-    cudaError_t e;
-    if ((e = dt_.alloc(sizeof(int64_t) * M)) != cudaSuccess ||
-        (e = cudaMemcpy(dt_.p, obs_t, sizeof(int64_t) * M, cudaMemcpyHostToDevice)) != cudaSuccess ||
-        (e = stage_rows(dR, R, R_stride, D, B, &a.R_stride)) != cudaSuccess ||
-        (e = stage_rows(dp, path, path_stride, plen, B, &a.path_stride)) != cudaSuccess ||
-        (e = stage_rows(dx, xi, xi_stride, olen, B, &a.xi_stride)) != cudaSuccess ||
-        (e = dy.alloc(sizeof(double) * (size_t)olen * B)) != cudaSuccess) {
-        cleanup();
-        g_create_error = std::string("CUDA error in vgpa_collect_obs: ") + cudaGetErrorString(e);
-        return VGPA_ECUDA;
-    }
+    cudaError_t e = cudaSuccess;
+    upload(e, dt_, obs_t, M);
+    stage_rows(e, dR, R, R_stride, D, B, &a.R_stride);
+    stage_rows(e, dp, path, path_stride, plen, B, &a.path_stride);
+    stage_rows(e, dx, xi, xi_stride, olen, B, &a.xi_stride);
+    alloc(e, dy, (size_t)olen * B);
+    if (e != cudaSuccess) return set_cuda_error(e, "vgpa_collect_obs");
     a.obs_t = dt_.as<long long>(); a.R = dR.as<double>(); a.path = dp.as<double>(); a.xi = dx.as<double>();
     a.obs_y = dy.as<double>(); a.obs_y_stride = olen;
     launch_collect_obs(a, nullptr);
@@ -1216,9 +1135,7 @@ int vgpa_collect_obs(int device, int D, int N, int M, int B, const int64_t* obs_
     if (e == cudaSuccess)
         e = cudaMemcpy2D(obs_y, sizeof(double) * (B > 1 ? obs_y_stride : olen), dy.p, sizeof(double) * olen, sizeof(double) * olen,
                          B, cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) { g_create_error = std::string("CUDA error in vgpa_collect_obs: ") + cudaGetErrorString(e); return VGPA_ECUDA; }
-    return VGPA_OK;
+    return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_collect_obs");
 }
 
 void* vgpa_host_alloc(int64_t bytes)
@@ -1315,8 +1232,7 @@ int64_t vgpa_chunk_size(const vgpa_handle* h) { return h ? h->chunk : 0; }
 int64_t vgpa_scratch_in_use(const vgpa_handle* h)
 {
     if (!h) return 0;
-    return (int64_t)(h->sc_mt.bytes + h->sc_st.bytes + h->sc_dEm.bytes + h->sc_dEs.bytes + h->sc_esde.bytes +
-                     h->sc2_mt.bytes + h->sc2_st.bytes + h->sc2_dEm.bytes + h->sc2_dEs.bytes + h->sc2_esde.bytes);
+    return (int64_t)h->sc.bytes();
 }
 
 }  // extern "C"

@@ -1,12 +1,33 @@
 // common.cuh -- shared declarations of the sm_100a VGPA kernels.
 #pragma once
+#include <cstddef>
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 
 namespace vgpa {
 
 enum Model { MODEL_DW = 0, MODEL_OU = 1, MODEL_L63 = 2, MODEL_L96 = 3 };
 enum Method { ODE_EULER = 0, ODE_HEUN = 1, ODE_RK2 = 2, ODE_RK4 = 3 };
+
+// Solver dispatch of the launchers: f(std::integral_constant<int, METHOD>{}) for the run-time method, so that
+// f instantiates its kernel for that method.  Values out of range take RK4.
+template <typename F>
+void with_method(int method, F&& f)
+{
+    switch (method) {
+    case ODE_EULER: f(std::integral_constant<int, ODE_EULER>{}); break;
+    case ODE_HEUN:  f(std::integral_constant<int, ODE_HEUN>{}); break;
+    case ODE_RK2:   f(std::integral_constant<int, ODE_RK2>{}); break;
+    default:        f(std::integral_constant<int, ODE_RK4>{}); break;
+    }
+}
+
+template <typename K>
+void set_smem(K kernel, size_t bytes)
+{
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
 
 // Device-resident description of a problem batch (all pointers are device
 // pointers; *_stride in elements, 0 = shared by every problem).

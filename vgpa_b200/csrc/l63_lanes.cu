@@ -380,24 +380,14 @@ void launch_l63_fwd_lanes(const Batch& b, const Scratch& s, const double* x, lon
                           cudaStream_t st)
 {
     const int th = 32, bl = (count + 1) / 2;     // one warp = one CTA = two problems
-    switch (b.method) {
-    case ODE_EULER: l63_fwd_lanes_kernel<ODE_EULER><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    case ODE_HEUN:  l63_fwd_lanes_kernel<ODE_HEUN><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    case ODE_RK2:   l63_fwd_lanes_kernel<ODE_RK2><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    default:        l63_fwd_lanes_kernel<ODE_RK4><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    }
+    with_method(b.method, [&](auto m) { l63_fwd_lanes_kernel<m><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); });
 }
 
 void launch_l63_bwd_lanes(const Batch& b, const Scratch& s, const double* x, long long xs, double* grad, long long gs,
                           int p0, int count, cudaStream_t st)
 {
     const int th = 32, bl = (count + 1) / 2;
-    switch (b.method) {
-    case ODE_EULER: l63_bwd_lanes_kernel<ODE_EULER><<<bl, th, 0, st>>>(b, s, x, xs, grad, gs, p0, count); break;
-    case ODE_HEUN:  l63_bwd_lanes_kernel<ODE_HEUN><<<bl, th, 0, st>>>(b, s, x, xs, grad, gs, p0, count); break;
-    case ODE_RK2:   l63_bwd_lanes_kernel<ODE_RK2><<<bl, th, 0, st>>>(b, s, x, xs, grad, gs, p0, count); break;
-    default:        l63_bwd_lanes_kernel<ODE_RK4><<<bl, th, 0, st>>>(b, s, x, xs, grad, gs, p0, count); break;
-    }
+    with_method(b.method, [&](auto m) { l63_bwd_lanes_kernel<m><<<bl, th, 0, st>>>(b, s, x, xs, grad, gs, p0, count); });
 }
 
 }  // namespace vgpa

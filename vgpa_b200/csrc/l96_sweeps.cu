@@ -695,35 +695,25 @@ l96_bwd_kernel(Batch b, BwdArgs a, int p0)
     }
 }
 
-template <typename K>
-void set_smem(K kernel, size_t bytes)
-{
-    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-}
-
 }  // namespace
 
 void launch_l96_fwd(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count,
                     cudaStream_t st)
 {
     const size_t sh = sizeof(FwdSmem);
-    switch (b.method) {
-    case ODE_EULER: set_smem(l96_fwd_kernel<ODE_EULER>, sh); l96_fwd_kernel<ODE_EULER><<<count, NTH, sh, st>>>(b, s, x, xs, p0); break;
-    case ODE_HEUN:  set_smem(l96_fwd_kernel<ODE_HEUN>, sh);  l96_fwd_kernel<ODE_HEUN><<<count, NTH, sh, st>>>(b, s, x, xs, p0); break;
-    case ODE_RK2:   set_smem(l96_fwd_kernel<ODE_RK2>, sh);   l96_fwd_kernel<ODE_RK2><<<count, NTH, sh, st>>>(b, s, x, xs, p0); break;
-    default:        set_smem(l96_fwd_kernel<ODE_RK4>, sh);   l96_fwd_kernel<ODE_RK4><<<count, NTH, sh, st>>>(b, s, x, xs, p0); break;
-    }
+    with_method(b.method, [&](auto m) {
+        set_smem(l96_fwd_kernel<m>, sh);
+        l96_fwd_kernel<m><<<count, NTH, sh, st>>>(b, s, x, xs, p0);
+    });
 }
 
 static void bwd_launch(const Batch& b, const BwdArgs& a, int p0, int count, cudaStream_t st)
 {
     const size_t sh = sizeof(BwdSmem);
-    switch (b.method) {
-    case ODE_EULER: set_smem(l96_bwd_kernel<ODE_EULER>, sh); l96_bwd_kernel<ODE_EULER><<<count, NTH, sh, st>>>(b, a, p0); break;
-    case ODE_HEUN:  set_smem(l96_bwd_kernel<ODE_HEUN>, sh);  l96_bwd_kernel<ODE_HEUN><<<count, NTH, sh, st>>>(b, a, p0); break;
-    case ODE_RK2:   set_smem(l96_bwd_kernel<ODE_RK2>, sh);   l96_bwd_kernel<ODE_RK2><<<count, NTH, sh, st>>>(b, a, p0); break;
-    default:        set_smem(l96_bwd_kernel<ODE_RK4>, sh);   l96_bwd_kernel<ODE_RK4><<<count, NTH, sh, st>>>(b, a, p0); break;
-    }
+    with_method(b.method, [&](auto m) {
+        set_smem(l96_bwd_kernel<m>, sh);
+        l96_bwd_kernel<m><<<count, NTH, sh, st>>>(b, a, p0);
+    });
 }
 
 void launch_l96_bwd(const Batch& b, const Scratch& s, const double* x, long long xs, double* grad,

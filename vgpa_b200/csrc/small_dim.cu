@@ -1218,18 +1218,10 @@ static void fwd_dispatch(const Batch& b, const Scratch& s, const double* x, long
     if constexpr (D == 1) {
         const size_t sh = scan_fwd_bytes(b.N, b.method);
         if (count <= (b.method == ODE_RK2 ? SCAN_RK2_MAX_BATCH : SCAN_MAX_BATCH) && sh <= SCAN_MAX_SMEM && !scan_disabled()) {
-#define VGPA_SCAN_FWD(M)                                                                                  \
-    do {                                                                                                  \
-        cudaFuncSetAttribute(scan1_fwd_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh);  \
-        scan1_fwd_kernel<M><<<count, SCAN_THREADS, sh, st>>>(b, s, x, xs, p0, count);                     \
-    } while (0)
-            switch (b.method) {
-            case ODE_EULER: VGPA_SCAN_FWD(ODE_EULER); break;
-            case ODE_HEUN:  VGPA_SCAN_FWD(ODE_HEUN); break;
-            case ODE_RK2:   VGPA_SCAN_FWD(ODE_RK2); break;
-            default:        VGPA_SCAN_FWD(ODE_RK4); break;
-            }
-#undef VGPA_SCAN_FWD
+            with_method(b.method, [&](auto m) {
+                set_smem(scan1_fwd_kernel<m>, sh);
+                scan1_fwd_kernel<m><<<count, SCAN_THREADS, sh, st>>>(b, s, x, xs, p0, count);
+            });
             return;
         }
     }
@@ -1237,28 +1229,15 @@ static void fwd_dispatch(const Batch& b, const Scratch& s, const double* x, long
         constexpr int TB = (D == 1) ? 16 : 8;
         const size_t sh = fwd_stage_bytes<D, TB>();
         const int bl = (count + 31) / 32;
-#define VGPA_FWD_STAGED(M)                                                                              \
-    do {                                                                                                \
-        cudaFuncSetAttribute(small_fwd_staged_kernel<D, M, TB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh); \
-        small_fwd_staged_kernel<D, M, TB><<<bl, 32, sh, st>>>(b, s, x, xs, p0, count);                  \
-    } while (0)
-        switch (b.method) {
-        case ODE_EULER: VGPA_FWD_STAGED(ODE_EULER); break;
-        case ODE_HEUN:  VGPA_FWD_STAGED(ODE_HEUN); break;
-        case ODE_RK2:   VGPA_FWD_STAGED(ODE_RK2); break;
-        default:        VGPA_FWD_STAGED(ODE_RK4); break;
-        }
-#undef VGPA_FWD_STAGED
+        with_method(b.method, [&](auto m) {
+            set_smem(small_fwd_staged_kernel<D, m, TB>, sh);
+            small_fwd_staged_kernel<D, m, TB><<<bl, 32, sh, st>>>(b, s, x, xs, p0, count);
+        });
         return;
     }
     // one thread per problem: small CTAs spread a small batch over more SMs (more load streams in flight)
     const int th = (count <= 148 * 64) ? 32 : 64, bl = (count + th - 1) / th;
-    switch (b.method) {
-    case ODE_EULER: small_fwd_kernel<D, ODE_EULER><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    case ODE_HEUN:  small_fwd_kernel<D, ODE_HEUN><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    case ODE_RK2:   small_fwd_kernel<D, ODE_RK2><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    default:        small_fwd_kernel<D, ODE_RK4><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); break;
-    }
+    with_method(b.method, [&](auto m) { small_fwd_kernel<D, m><<<bl, th, 0, st>>>(b, s, x, xs, p0, count); });
 }
 void launch_small_fwd(const Batch& b, const Scratch& s, const double* x, long long xs, int p0,
                       int count, cudaStream_t st)
@@ -1277,27 +1256,11 @@ bool launch_small_fused(const Batch& b, const double* x, long long xs, double* F
         (b.method == ODE_RK2 && count > SCAN_RK2_MAX_BATCH) ||
         ex.lamt != nullptr || ex.Efx != nullptr || ex.parts != nullptr)
         return false;
-#define VGPA_SCAN_EVAL(MODEL, M)                                                                                  \
-    do {                                                                                                          \
-        cudaFuncSetAttribute(scan1_eval_kernel<MODEL, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh);  \
-        scan1_eval_kernel<MODEL, M><<<count, SCAN_THREADS, sh, st>>>(b, x, xs, F, g, gs, p0, count);              \
-    } while (0)
-    if (b.model == MODEL_DW) {
-        switch (b.method) {
-        case ODE_EULER: VGPA_SCAN_EVAL(MODEL_DW, ODE_EULER); break;
-        case ODE_HEUN:  VGPA_SCAN_EVAL(MODEL_DW, ODE_HEUN); break;
-        case ODE_RK2:   VGPA_SCAN_EVAL(MODEL_DW, ODE_RK2); break;
-        default:        VGPA_SCAN_EVAL(MODEL_DW, ODE_RK4); break;
-        }
-    } else {
-        switch (b.method) {
-        case ODE_EULER: VGPA_SCAN_EVAL(MODEL_OU, ODE_EULER); break;
-        case ODE_HEUN:  VGPA_SCAN_EVAL(MODEL_OU, ODE_HEUN); break;
-        case ODE_RK2:   VGPA_SCAN_EVAL(MODEL_OU, ODE_RK2); break;
-        default:        VGPA_SCAN_EVAL(MODEL_OU, ODE_RK4); break;
-        }
-    }
-#undef VGPA_SCAN_EVAL
+    with_method(b.method, [&](auto m) {
+        const auto kernel = (b.model == MODEL_DW) ? scan1_eval_kernel<MODEL_DW, m> : scan1_eval_kernel<MODEL_OU, m>;
+        set_smem(kernel, sh);
+        kernel<<<count, SCAN_THREADS, sh, st>>>(b, x, xs, F, g, gs, p0, count);
+    });
     return true;
 }
 
@@ -1320,28 +1283,15 @@ static void bwd_dispatch(const Batch& b, const Scratch& s, const SmallBwdArgs& a
         const size_t sh = scan_bwd_bytes(b.N);
         if (a.grad != nullptr && a.jm_dense == nullptr && ex.lamt == nullptr && count <= SCAN_MAX_BATCH &&
             sh <= SCAN_MAX_SMEM && !scan_disabled()) {   // time-parallel
-#define VGPA_SCAN_BWD(M)                                                                                        \
-    do {                                                                                                        \
-        cudaFuncSetAttribute(scan1_bwd_kernel<MODEL, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh); \
-        scan1_bwd_kernel<MODEL, M><<<count, SCAN_THREADS, sh, st>>>(b, s, a, p0, count);                        \
-    } while (0)
-            switch (b.method) {
-            case ODE_EULER: VGPA_SCAN_BWD(ODE_EULER); break;
-            case ODE_HEUN:  VGPA_SCAN_BWD(ODE_HEUN); break;
-            case ODE_RK2:   VGPA_SCAN_BWD(ODE_RK2); break;
-            default:        VGPA_SCAN_BWD(ODE_RK4); break;
-            }
-#undef VGPA_SCAN_BWD
+            with_method(b.method, [&](auto m) {
+                set_smem(scan1_bwd_kernel<MODEL, m>, sh);
+                scan1_bwd_kernel<MODEL, m><<<count, SCAN_THREADS, sh, st>>>(b, s, a, p0, count);
+            });
             return;
         }
     }
     const int th = (count <= 148 * 64) ? 32 : 64, bl = (count + th - 1) / th;
-    switch (b.method) {
-    case ODE_EULER: small_bwd_kernel<MODEL, D, ODE_EULER><<<bl, th, 0, st>>>(b, s, a, p0, count, ex); break;
-    case ODE_HEUN:  small_bwd_kernel<MODEL, D, ODE_HEUN><<<bl, th, 0, st>>>(b, s, a, p0, count, ex); break;
-    case ODE_RK2:   small_bwd_kernel<MODEL, D, ODE_RK2><<<bl, th, 0, st>>>(b, s, a, p0, count, ex); break;
-    default:        small_bwd_kernel<MODEL, D, ODE_RK4><<<bl, th, 0, st>>>(b, s, a, p0, count, ex); break;
-    }
+    with_method(b.method, [&](auto m) { small_bwd_kernel<MODEL, D, m><<<bl, th, 0, st>>>(b, s, a, p0, count, ex); });
 }
 void launch_small_bwd(const Batch& b, const Scratch& s, const double* x, long long xs, double* g,
                       long long gs, int p0, int count, const Extra& ex, cudaStream_t st)

@@ -15,14 +15,13 @@ from . import _lib
 from ._lib import MODELS, METHODS, MODEL_DIM, VgpaDesc, VgpaFullOut, dptr, f64, lib, raise_for
 
 
-def _per_problem(a, B, shape, name):
-    """Accept either one array of `shape` (shared) or B of them."""
-    a = f64(a)
-    n = int(np.prod(shape)) if shape else 1
+def _rows(a, B, n, name):
+    """n values shared by the B problems, or B x n: returns the flat array and its row stride (0 = shared)."""
+    a = f64(a).reshape(-1)
     if a.size == n:
-        return a.reshape(-1), 0
+        return a, 0
     if a.size == B * n:
-        return a.reshape(-1), n
+        return a, n
     raise ValueError(f"{name}: expected {n} or {B}x{n} values, got {a.size}")
 
 
@@ -57,12 +56,11 @@ class BatchEvaluator:
         d.device = self.device
         d.dt = float(dt)
         d.dt_model = float(dt if dt_model is None else dt_model)
-        for name, val, shape in (("theta", theta, (nth,)), ("sigma", sigma, (D,)), ("R", R, (D,)),
-                                 ("obs_y", obs_y, (M, D)), ("m0", m0, (D,)), ("s0", s0, (D, D)),
-                                 ("E0", E0, ())):
+        for name, val, n in (("theta", theta, nth), ("sigma", sigma, D), ("R", R, D), ("obs_y", obs_y, M * D),
+                             ("m0", m0, D), ("s0", s0, D * D), ("E0", E0, 1)):
             if name == "obs_y" and M == 0:
                 continue
-            arr, stride = _per_problem(val, self.B, shape, name)
+            arr, stride = _rows(val, self.B, n, name)
             keep[name] = arr
             setattr(d, name, dptr(arr))
             setattr(d, name + "_stride", stride)
@@ -279,16 +277,6 @@ def obs_energy(obs_t, obs_y, R_diag, m, s, device=0, with_dr=False):
 
 
 # -- batched data generation (SURVEY 8 f4; host buffers) ------------------------------
-def _rows(a, B, n, name):
-    """(n,) shared by the B paths, or (B, n): returns the flat array and its row stride."""
-    a = f64(a).reshape(-1)
-    if a.size == n:
-        return a, 0
-    if a.size == B * n:
-        return a, n
-    raise ValueError(f"{name}: expected {n} or {B}x{n} values, got {a.size}")
-
-
 def make_trajectories(model, N, dt, theta, sigma_diag, z, x_init=None, device=0):
     """B sample paths by the Euler-Maruyama loop of <Model>.make_trajectory, on the GPU.
     z: (B, D, N) standard-normal draws in the reference's (D, N) layout ((B, N) for the 1-D models);
