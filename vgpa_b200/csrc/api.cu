@@ -219,8 +219,10 @@ struct vgpa_handle {
     cudaStream_t s_aux = nullptr;       //   non-blocking stream of the list upload
     cudaEvent_t plist_ev[2] = {nullptr, nullptr};   //   end of the last evaluation that read each copy
     bool plist_used[2] = {false, false};
-    std::vector<int> plist_host;        // ... and the host copy (error messages name the problem, not the position)
+    std::vector<int> plist_host;        // ... and the host copy
     int n_list = -1;                    // < 0: no list, every problem
+    std::vector<int> status_map;        // status word k belongs to problem status_map[k] (the list of the compacted
+                                        //   evaluation that wrote it); empty: to problem k
     cudaStream_t s_comp = nullptr, s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_h2d[2]{}, ev_comp[2]{}, ev_d2h[2]{};
     cudaStream_t last_stream = nullptr;
@@ -320,6 +322,7 @@ struct HostCallScope {
         if (h->status_dirty) cudaStreamSynchronize(h->last_stream);
         h->batch.active = nullptr;
         h->batch.plist = nullptr;
+        h->status_map.clear();
     }
     ~HostCallScope()
     {
@@ -343,7 +346,7 @@ int check_status(vgpa_handle* h)
     for (int p = 0; p < h->d.B; ++p)
         if (st[p] != 0) {
             // under a compacted launch the status words are indexed by launch position
-            const int prob = (h->n_list >= 0 && p < (int)h->plist_host.size()) ? h->plist_host[p] : p;
+            const int prob = (p < (int)h->status_map.size()) ? h->status_map[p] : p;
             return h->fail(VGPA_ENOTPD, "Matrix is not positive definite: S(t) of problem %d at time index %d",
                            prob, st[p] - 1);
         }
@@ -543,13 +546,16 @@ int vgpa_eval_device(vgpa_handle* h, const double* d_x, int64_t x_stride, int wa
         CK(cudaStreamWaitEvent(st, h->ev_done, 0), "cudaStreamWaitEvent");
     CK(cudaMemsetAsync(h->status.p, 0, sizeof(int) * h->d.B, st), "cudaMemsetAsync(status)");
     Extra ex{};
-    const int total = (h->n_list >= 0 && h->batch.plist != nullptr) ? h->n_list : h->d.B;   // launch positions
+    const bool compacted = h->n_list >= 0 && h->batch.plist != nullptr;
+    const int total = compacted ? h->n_list : h->d.B;   // launch positions
+    if (compacted) h->status_map = h->plist_host;     // vgpa_sync names problems by this list, even if it changes first
+    else h->status_map.clear();
     for (int p0 = 0; p0 < total; p0 += h->chunk) {
         const int count = std::min(h->chunk, total - p0);
         run_chunk(h, d_x, x_stride, want_grad, d_F, d_grad, grad_stride, p0, count, ex, st);
     }
     CK(cudaGetLastError(), "kernel launch");
-    if (h->batch.plist != nullptr && h->n_list >= 0) {   // this evaluation reads the current copy of the list
+    if (compacted) {   // this evaluation reads the current copy of the list
         const int q = h->plist_flip;
         if (h->plist_ev[q] == nullptr) CK(cudaEventCreateWithFlags(&h->plist_ev[q], cudaEventDisableTiming), "cudaEventCreate");
         CK(cudaEventRecord(h->plist_ev[q], st), "cudaEventRecord");
