@@ -132,6 +132,22 @@ int vgpa_eval_device(vgpa_handle *h, const double *d_x, int64_t x_stride, int wa
                      double *d_F, double *d_grad, int64_t grad_stride, void *stream);
 int vgpa_sync(vgpa_handle *h);
 
+/* model.energy's hyper-parameter gradients for EVERY problem of the handle, each at its own x row
+ * (d_x + p * x_stride; 0 = one x shared by all).  DEVICE buffers, asynchronous on `stream`; vgpa_sync
+ * waits and reports a non-positive-definite S(t) exactly as after vgpa_eval_device.  Any output may be NULL.
+ *   F[p]                           free energy (bitwise what vgpa_eval_device returns for the same x)
+ *   Esde[p]                        Esde as energy() returns it (= parts[1] of vgpa_eval_full)
+ *   dtheta + p * dtheta_stride     dEsde_dtheta: 1 (DW, OU), 3 (L63), D (L96) values
+ *   dsigma + p * dsigma_stride     dEsde_dsigma: 1 value (D = 1) or D x D (diagonal; off-diagonals written as 0)
+ * x is 16-byte aligned with an even stride; an output stride is at least the length of its row (0 only when
+ * B = 1).  dEsde_dtheta and dEsde_dsigma are the partial derivatives at the problem's m(t), S(t): for DW, OU
+ * and L63, dEsde_dtheta is dF/dtheta at fixed x.  Ordering against other calls on the handle is that of
+ * vgpa_eval_device.  The active set and the compacted list are suspended for the call (every problem is
+ * served) and stay installed for later vgpa_eval_device calls. */
+int vgpa_hyper_device(vgpa_handle *h, const double *d_x, int64_t x_stride, double *d_F, double *d_Esde,
+                      double *d_dtheta, int64_t dtheta_stride, double *d_dsigma, int64_t dsigma_stride,
+                      void *stream);
+
 /*
  * One problem, everything: F, its three parts, the gradient and every
  * intermediate the reference caches in VarGP.output (variational.py:189-196,
@@ -174,7 +190,8 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
 /* dEsde_dtheta / dEsde_dsigma: the hyper-parameter gradients that energy() returns last
  * (double_well.py:251-257, ornstein_uhlenbeck.py:223-229, lorenz_63.py:327-343 + :572-633,
  * lorenz_96.py:420-434) and VarGP discards.  Both may be NULL (not computed).  Sizes:
- * dEsde_dtheta 1 (DW, OU), 3 (L63), D (L96); dEsde_dsigma 1 (D = 1) or D x D. */
+ * dEsde_dtheta 1 (DW, OU), 3 (L63), D (L96); dEsde_dsigma 1 (D = 1) or D x D.  The kernels are those of
+ * vgpa_hyper_device with one problem. */
 
 /* GaussianLikelihood.__call__ and .gradients (gaussian_like.py:39-243) on their
  * own: one problem, HOST buffers, identity operator, diagonal R (D values).

@@ -61,6 +61,9 @@ def _load():
     lib.vgpa_eval_device.restype = C.c_int
     lib.vgpa_eval_device.argtypes = [H, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
                                      C.c_int64, C.c_void_p]
+    lib.vgpa_hyper_device.restype = C.c_int
+    lib.vgpa_hyper_device.argtypes = [H, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                      C.c_void_p, C.c_int64, C.c_void_p]
     lib.vgpa_initialization.restype = C.c_int
     lib.vgpa_initialization.argtypes = [H, C.c_double, C.c_void_p, C.c_int64, C.c_void_p]
     lib.vgpa_initialization_host.restype = C.c_int

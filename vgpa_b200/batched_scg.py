@@ -369,7 +369,7 @@ class ShardedBatchedSCG:
         per_problem = 5 * 8 * n_x + scratch_per_problem + 64
         return max(1, int(free * self.mem_fraction // per_problem))
 
-    def run(self, t0=0.0, x0_fn=None, keep=(), concurrent=1):
+    def run(self, t0=0.0, x0_fn=None, keep=(), concurrent=1, hyper=False):
         """Optimise the local block.  x0_fn(lo, hi, X) fills the (hi - lo, n) device tensor X with starting
         points (default: the on-device VarGP.initialization).  keep: global problem indices whose optimised
         x is returned (host).  concurrent: sub-batches optimised AT THE SAME TIME, each by its own host thread
@@ -378,7 +378,10 @@ class ShardedBatchedSCG:
         evaluation as a full wave) can overlap the full waves of another.  (Measured on one B200, Lorenz-96:
         1776 problems as two sub-batches of 888, 177-200 optimisations/s one after the other, 217-235 concurrently;
         888 problems as one sub-batch 229, as two concurrent halves 176 -- concurrency only pays between sub-batches
-        that each fill the GPU, so the default stays 1.)  Returns the dict that `save` writes,
+        that each fill the GPU, so the default stays 1.)  hyper=True: each sub-batch also computes model.energy's
+        hyper-parameter gradients at its optimised x (one vgpa_hyper_device call before x is freed), returned
+        as Esde (total,), dEsde_dtheta (total, n_theta) and dEsde_dsigma_diag (total, D) -- the diagonal only,
+        dEsde_dsigma is diagonal (the full D x D of 32768 Lorenz-96 problems is 420 MB).  Returns the dict that `save` writes,
         identical on every rank (except `kept` entries, which each rank holds for its own problems until the
         gather)."""
         import time
@@ -391,6 +394,7 @@ class ShardedBatchedSCG:
         n_it = np.zeros(n_local, dtype=np.int64)
         f_eval = np.zeros(n_local)
         kept = {}
+        hyp = None
         sub = self.sub_batch
         if sub is None and n_local > 0:   # from the evaluator's shape: what fits the free HBM, shared by the workers
             ev = self.make_evaluator(self.lo, min(self.hi, self.lo + 1))
@@ -430,6 +434,8 @@ class ShardedBatchedSCG:
                     res = {"range": rng_, "optimise_seconds": t_opt, "create_seconds": t_create, "x0_seconds": t_x0, "fx": fxb, "n_it": opt.stats["MaxIt"], "f_eval": opt.stats["f_eval"],
                            "evaluations": opt.stats["evaluations"] * b, "syncs": opt.host_syncs,
                            "kept": {k: Xf[k - lo_].cpu().numpy() for k in keep if lo_ <= k < hi_}}
+                    if hyper:
+                        res["hyper"] = self._hyper_at(ev, Xf, stream)
                     t_free = time.perf_counter()
                     del opt, Xf, X
                 return res
@@ -481,6 +487,11 @@ class ShardedBatchedSCG:
             create_seconds += r["create_seconds"]
             x0_seconds += r["x0_seconds"]
             kept.update(r["kept"])
+            if hyper:
+                if hyp is None:
+                    hyp = {k: np.zeros((n_local,) + v.shape[1:]) for k, v in r["hyper"].items()}
+                for k, v in r["hyper"].items():
+                    hyp[k][sl] = v
         # gather of the per-problem results (the only collective)
         def gather(v):
             if self.world == 1 or not (dist.is_available() and dist.is_initialized()):
@@ -491,6 +502,9 @@ class ShardedBatchedSCG:
         out = {"fx": gather(fx), "n_it": gather(n_it.astype(np.float64)).astype(np.int64), "f_eval": gather(f_eval),
                "rank_seconds": seconds, "rank_optimise_seconds": optimise_seconds, "rank_problem_evaluations": evaluations, "rank_host_syncs": syncs,
                "sub_batch": sub, "concurrent": concurrent, "kept": kept}
+        if hyper:
+            for k, v in hyp.items():     # gathered like fx, one column at a time
+                out[k] = gather(v) if v.ndim == 1 else np.stack([gather(v[:, j]) for j in range(v.shape[1])], axis=1)
         out["rank_phase_seconds"] = {"create_evaluators": round(create_seconds, 4), "starting_points": round(x0_seconds, 4),
                                      "optimise": round(optimise_seconds, 4), "whole_loop": round(seconds, 4),
                                      "close_evaluators": round(sum(r.get("free_seconds", 0.0) for r in results), 4),
@@ -500,11 +514,29 @@ class ShardedBatchedSCG:
         _start_release()
         return out
 
+    @staticmethod
+    def _hyper_at(ev, X, stream):
+        """Esde, dEsde_dtheta and the diagonal of dEsde_dsigma of every problem of `ev` at the rows of X (host arrays)."""
+        import torch
+        b, D, nth = ev.B, ev.D, ev.n_theta
+        nsig = 1 if D == 1 else D * D
+        Esde = torch.empty(b, dtype=torch.float64, device=X.device)
+        dth = torch.empty((b, nth), dtype=torch.float64, device=X.device)
+        dsig = torch.empty((b, nsig), dtype=torch.float64, device=X.device)
+        ev.hyper_device(X.data_ptr(), ev.n_x, None, Esde.data_ptr(), dth.data_ptr(), nth, dsig.data_ptr(), nsig,
+                        stream.cuda_stream)
+        ev.sync()
+        diag = dsig if D == 1 else dsig[:, ::D + 1]
+        return {"Esde": Esde.cpu().numpy(), "dEsde_dtheta": dth.cpu().numpy(), "dEsde_dsigma_diag": diag.cpu().numpy()}
+
     def save(self, name, N, D):
         """Rank-local file `<name>_rank<r>` in the reference's key convention (save_ensemble)."""
         r = self.result
         ks = sorted(r["kept"])
         out = {"fx": r["fx"], "n_it": r["n_it"], "f_eval": r["f_eval"], "problem": np.array(ks, dtype=np.int64)}
+        for k in ("Esde", "dEsde_dtheta", "dEsde_dsigma_diag"):
+            if k in r:
+                out[k] = r[k]
         if ks:
             xs = np.stack([r["kept"][k] for k in ks])
             if D == 1:

@@ -1,6 +1,7 @@
 // api.cu -- the C ABI of libvgpa_b200.so (include/vgpa_b200.h): handle management,
 // chunked three-phase evaluation (forward sweep -> time-parallel energy -> backward
-// sweep fused with the gradient), host staging with copy/compute overlap.
+// sweep fused with the gradient), the batched hyper-parameter gradients, host staging
+// with copy/compute overlap.
 #include <algorithm>
 #include <cstdarg>
 #include <cstdio>
@@ -310,6 +311,29 @@ void run_chunk(vgpa_handle* h, const double* d_x, long long xs, int want_grad, d
     }
 }
 
+// one pass of vgpa_hyper_device over problems [p0, p0 + count): the forward sweep, the energy stage with the
+// hyper integrands (into the pass's dEs scratch, which nothing after them reads), F, the per-problem reduction
+void run_hyper_chunk(vgpa_handle* h, const double* d_x, long long xs, double* d_F, const HyperOut& o, int p0, int count,
+                     cudaStream_t st)
+{
+    const Scratch sc = h->sc.view(h->status.as<int>() + p0);
+    const Batch& b = h->batch;
+    const bool small = small_model(b.model);
+    h->tick(0, st, true);
+    if (small) launch_small_fwd(b, sc, d_x, xs, p0, count, st);
+    else launch_l96_fwd(b, sc, d_x, xs, p0, count, st);
+    h->tick(0, st, false);
+    h->tick(1, st, true);
+    if (small) launch_small_energy(b, sc, d_x, xs, p0, count, Extra{}, st);
+    launch_hyper_terms(b, sc, d_x, xs, p0, count, st);
+    h->tick(1, st, false);
+    h->tick(2, st, true);
+    if (d_F != nullptr) launch_finalize(b, sc, d_F, p0, count, Extra{}, st);
+    launch_hyper_reduce(b, sc, p0, count, o, st);
+    h->tick(2, st, false);
+    h->launches += (small ? 4 : 3) + (d_F != nullptr ? 1 : 0);
+}
+
 // The host-buffer entry points (vgpa_eval, vgpa_eval_full) always serve EVERY problem: the active set
 // and the compacted list installed for vgpa_eval_device are suspended for the call (a masked problem
 // would otherwise return whatever the staging buffers hold), and a device evaluation still pending on
@@ -561,6 +585,45 @@ int vgpa_eval_device(vgpa_handle* h, const double* d_x, int64_t x_stride, int wa
         CK(cudaEventRecord(h->plist_ev[q], st), "cudaEventRecord");
         h->plist_used[q] = true;
     }
+    if (h->ev_done == nullptr) CK(cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming), "cudaEventCreate");
+    CK(cudaEventRecord(h->ev_done, st), "cudaEventRecord");
+    h->last_stream = st;
+    h->status_dirty = true;
+    return VGPA_OK;
+}
+
+int vgpa_hyper_device(vgpa_handle* h, const double* d_x, int64_t x_stride, double* d_F, double* d_Esde,
+                      double* d_dtheta, int64_t dtheta_stride, double* d_dsigma, int64_t dsigma_stride, void* stream)
+{
+    if (!h) return VGPA_EINVAL;
+    if (d_x == nullptr) return h->fail(VGPA_EINVAL, "x is NULL");
+    if (x_stride != 0 && x_stride < h->n_x) return h->fail(VGPA_EINVAL, "x_stride %lld < %lld", (long long)x_stride, h->n_x);
+    if (((uintptr_t)d_x & 15) || (x_stride & 1))
+        return h->fail(VGPA_EINVAL, "device buffers must be 16-byte aligned with even strides");
+    const int D = h->d.D, B = h->d.B;
+    const long long nth = hyper_ntheta(h->batch.model, D), nsig = (D == 1) ? 1 : (long long)D * D;
+    if (d_dtheta != nullptr && dtheta_stride < nth && !(B == 1 && dtheta_stride == 0))
+        return h->fail(VGPA_EINVAL, "dtheta_stride %lld < %lld", (long long)dtheta_stride, nth);
+    if (d_dsigma != nullptr && dsigma_stride < nsig && !(B == 1 && dsigma_stride == 0))
+        return h->fail(VGPA_EINVAL, "dsigma_stride %lld < %lld", (long long)dsigma_stride, nsig);
+    CK(cudaSetDevice(h->d.device), "cudaSetDevice");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // one scratch, one set of status words: ordered after the previous evaluation as in vgpa_eval_device
+    if (h->ev_done != nullptr && h->status_dirty && st != h->last_stream)
+        CK(cudaStreamWaitEvent(st, h->ev_done, 0), "cudaStreamWaitEvent");
+    CK(cudaMemsetAsync(h->status.p, 0, sizeof(int) * B, st), "cudaMemsetAsync(status)");
+    // every problem is served, its status word indexed by problem; the kernels take the Batch by value, so the
+    // active set and the list are back in place for later calls as soon as the launches are enqueued
+    const int *active = h->batch.active, *plist = h->batch.plist;
+    h->batch.active = nullptr;
+    h->batch.plist = nullptr;
+    h->status_map.clear();
+    const HyperOut o{d_Esde, d_dtheta, dtheta_stride, d_dsigma, dsigma_stride};
+    for (int p0 = 0; p0 < B; p0 += h->chunk)
+        run_hyper_chunk(h, d_x, x_stride, d_F, o, p0, std::min(h->chunk, B - p0), st);
+    h->batch.active = active;
+    h->batch.plist = plist;
+    CK(cudaGetLastError(), "kernel launch");
     if (h->ev_done == nullptr) CK(cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming), "cudaEventCreate");
     CK(cudaEventRecord(h->ev_done, st), "cudaEventRecord");
     h->last_stream = st;
@@ -832,9 +895,9 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
     if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const long long nv = (long long)N * D, nm = (long long)N * D * D;
     const int nth = n_theta(model);
-    DevBuf dx, dth, dsig, dmt, dst, dgm, dgs, des, def, dedf, dparts, dzero, dF, dstat, dft, dfs, dhth, dhsig;
+    DevBuf dx, dth, dsig, dmt, dst, dgm, dgs, des, def, dedf, dparts, dzero, dF, dstat, dterms, dhth, dhsig;
     const bool hyper = (dEth != nullptr) || (dEsig != nullptr);
-    const int nhth = (model == VGPA_MODEL_L96) ? D : nth;   // lorenz_96.py:431: one entry per state dimension
+    const int nhth = hyper_ntheta(model, D);
     const long long nsig = (D == 1) ? 1 : (long long)D * D;
     cudaError_t e = cudaSuccess;
     alloc(e, dx, nm + nv);
@@ -869,16 +932,15 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
     if (model == VGPA_MODEL_L96) launch_l96_energy(bt, sc, dx.as<double>(), 0, 0, 1, ex, nullptr);
     else launch_small_energy(bt, sc, dx.as<double>(), 0, 0, 1, ex, nullptr);
     launch_finalize(bt, sc, dF.as<double>(), 0, 1, ex, nullptr);
-    if (hyper) {
-        alloc(e, dft, (size_t)N * nhth);
-        alloc(e, dfs, nv);
+    if (hyper) {   // the launchers of vgpa_hyper_device with B = 1; the integrands go to a buffer of their own
+        alloc(e, dterms, (size_t)N * (nhth + (D == 1 ? 0 : D)));
         alloc(e, dhth, nhth);
         alloc(e, dhsig, nsig);
         if (e != cudaSuccess) return set_cuda_error(e, "vgpa_model_energy");
-        // parts[1] = Esde (written by finalize on the same stream)
-        launch_hyper(model, D, N, dt_model, dth.as<double>(), dsig.as<double>(), dx.as<double>(), dmt.as<double>(),
-                     dst.as<double>(), dparts.as<double>() + 1, dft.as<double>(), dfs.as<double>(),
-                     dhth.as<double>(), dhsig.as<double>(), dstat.as<int>(), nullptr);
+        Scratch hs = sc;
+        hs.dEs = dterms.as<double>();
+        launch_hyper_terms(bt, hs, dx.as<double>(), 0, 0, 1, nullptr);
+        launch_hyper_reduce(bt, hs, 0, 1, HyperOut{nullptr, dhth.as<double>(), 0, dhsig.as<double>(), 0}, nullptr);
     }
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();

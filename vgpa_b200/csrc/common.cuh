@@ -53,6 +53,38 @@ struct Batch {
 // problem served by launch position `pos` (= p0 + local index)
 __device__ __forceinline__ int problem_at(const Batch& b, int pos) { return b.plist != nullptr ? b.plist[pos] : pos; }
 
+// Sum over the CTA in a fixed order (every thread gets it); sh: blockDim.x doubles, blockDim.x a power of two.
+__device__ __forceinline__ double block_sum(double v, double* sh)
+{
+    const int tid = threadIdx.x;
+    sh[tid] = v;
+    __syncthreads();
+    for (int o = blockDim.x >> 1; o > 0; o >>= 1) {
+        if (tid < o) sh[tid] += sh[tid + o];
+        __syncthreads();
+    }
+    const double r = sh[0];
+    __syncthreads();
+    return r;
+}
+
+// Esde of problem p from its integrand f(t) (utilities.py:144-201: composite trapezoid, sum(dx * (f[i+1] + f[i]) / 2)).
+// Every thread of the CTA calls it.  The partial sums are taken by the first ESDE_THREADS threads whatever the CTA
+// size (the rest add zeros to the reduction tree), so that Esde and F are the same bits from finalize_kernel, from
+// the fused D = 1 evaluation (SCAN_THREADS) and from the hyper-parameter reduction.
+constexpr int ESDE_THREADS = 128;
+__device__ __forceinline__ double esde_of(const Batch& b, int p, const double* f, double* sh)
+{
+    const int tid = threadIdx.x, N = b.N;
+    double acc = 0.0;
+    if (tid < ESDE_THREADS)
+        for (int i = tid; i < N - 1; i += ESDE_THREADS) acc += b.dt_model * (f[i + 1] + f[i]) / 2.0;
+    double Esde = block_sum(acc, sh);
+    if (b.model == MODEL_DW || b.model == MODEL_OU)  // double_well.py:217, ornstein_uhlenbeck.py:208
+        Esde = 0.5 * Esde / b.sigma[p * b.sigma_stride];
+    return Esde;
+}
+
 // Per-pass (chunk) scratch: trajectories of the marginal moments, the SDE-energy
 // gradients and the per-time-step energy.  Problem-major: [p][t][...].
 struct Scratch {
@@ -153,10 +185,24 @@ void launch_bwd_dense(int method, int D, int N, double dt, const double* A, cons
 void launch_initialization(const Batch& b, int p0, int count, double t0, double* scratch, double* x,
                            long long x_stride, int* err, cudaStream_t st);
 
-// Hyper-parameter gradients of model.energy (hyper.cu); all pointers are device pointers.
-void launch_hyper(int model, int D, int N, double dt_model, const double* theta, const double* sigma,
-                  const double* x, const double* mt, const double* st, const double* esde, double* ft,
-                  double* fs, double* dth, double* dsig, int* status, cudaStream_t stream);
+// Hyper-parameter gradients of model.energy (hyper.cu).  dEsde/dtheta has one entry per theta value, and for
+// Lorenz-96 one per state dimension (lorenz_96.py:431).
+__host__ __device__ inline int hyper_ntheta(int model, int D) { return model == MODEL_L63 ? 3 : (model == MODEL_L96 ? D : 1); }
+// Per-problem outputs of the reduction: device rows p * stride, any pointer may be null.
+struct HyperOut {
+    double* Esde;                          // (B)
+    double* dth;  long long dth_stride;    // hyper_ntheta values
+    double* dsig; long long dsig_stride;   // 1 (D = 1) or D x D (diagonal; off-diagonals written as 0)
+};
+// The integrands of problems p0 .. p0 + count - 1 at their moments in s.mt, s.st into s.dEs (nth + D values per
+// (problem, t); ft only for D = 1).  D = 1 and 3 read s.esde_t later and need the energy stage first; D = 40 runs the
+// energy kernel's HYPER instantiation, which writes s.esde_t and the status words itself.
+void launch_hyper_terms(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count,
+                        cudaStream_t st);
+void launch_l96_hyper(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count,
+                      cudaStream_t st);
+// Esde, dEsde/dtheta, dEsde/dSigma of those problems from s.esde_t and the integrands: one CTA per problem.
+void launch_hyper_reduce(const Batch& b, const Scratch& s, int p0, int count, const HyperOut& o, cudaStream_t st);
 // dEobs_dr of the 1-D likelihood (N values, zero except at obs_t).
 void launch_obs_dr(int N, int M, const long long* obs_t, const double* obs_y, const double* R,
                    const double* mt, const double* st, double* dr, cudaStream_t stream);

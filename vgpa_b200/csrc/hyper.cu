@@ -1,44 +1,51 @@
 // hyper.cu -- hyper-parameter gradients of model.energy: dEsde/dtheta and dEsde/dSigma, the last two
 // entries of the third return value of StochasticProcess.energy.  The reference's hot path computes
-// them on every evaluation and discards them (variational.py:175); here they are produced only
-// when vgpa_model_energy is asked for them, by small kernels off the hot path:
+// them on every evaluation and discards them (variational.py:175); here they are produced on request,
+// for one problem (vgpa_model_energy) or for every problem of a handle (vgpa_hyper_device):
 //   DW   double_well.py:251-257        OU   ornstein_uhlenbeck.py:223-229
 //   L63  lorenz_63.py:327-343, Efg_drift_theta :572-633, Efg :414-432
 //   L96  lorenz_96.py:420-434 (m_bar of ut_approx, utilities.py:239-310; flattened roll :27-32)
-// Per time index the integrands go to scratch (ft: theta integrand, fs: Sigma integrand); one CTA
-// then integrates every component with the composite trapezoid (utilities.py:144-201) in a fixed
-// order and applies the final scalings.
+// Per (problem, time index) the integrands go to the pass's dEs scratch, nth + D values each (ft: theta
+// integrand, nth values; fs: Sigma integrand, D values; for D = 1 ft only, dEsde/dSigma = -Esde / sigma): one thread per (problem, t)
+// for D = 1 and D = 3 (below), the HYPER instantiation of the energy kernel for D = 40 (l96_energy.cu).
+// Then one CTA per problem integrates every component with the composite trapezoid
+// (utilities.py:144-201) in an order fixed by N alone and applies the final scalings.
 #include "common.cuh"
 
 namespace vgpa {
 namespace {
 
-// ---- D = 1 (DW, OU) and D = 3 (L63): one thread per time index -----------------------------
+// ---- D = 1 (DW, OU) and D = 3 (L63): one thread per (problem, time index) -------------------
 template <int MODEL>
 __global__ void __launch_bounds__(128)
-hyper_small_kernel(int N, const double* __restrict__ theta, const double* __restrict__ x,
-                   const double* __restrict__ mt, const double* __restrict__ st, double* __restrict__ ft,
-                   double* __restrict__ fs)
+hyper_small_kernel(Batch b, Scratch s, const double* __restrict__ x, long long xs, int p0, int count)
 {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= N) return;
+    constexpr int D = (MODEL == MODEL_L63) ? 3 : 1, DD = D * D, W = (MODEL == MODEL_L63) ? 6 : 1;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int N = b.N;
+    if (idx >= (long long)count * N) return;
+    const int lp = (int)(idx / N), t = (int)(idx % N), p = p0 + lp;
+    const double* xp = x + (long long)p * xs;
+    const double* theta = b.theta + p * b.theta_stride;
+    const double* m = s.mt + ((long long)lp * N + t) * D;
+    const double* S = s.st + ((long long)lp * N + t) * DD;
+    double* ft = s.dEs + ((long long)lp * N + t) * W;
     if (MODEL == MODEL_DW || MODEL == MODEL_OU) {
-        const double a = x[t], b = x[N + t], m = mt[t], v = st[t], th = theta[0];
-        const double m2 = m * m, E2 = m2 + v;
+        const double a = xp[t], bb = xp[N + t], mm = m[0], v = S[0], th = theta[0];
+        const double m2 = mm * mm, E2 = m2 + v;
         if (MODEL == MODEL_DW) {
             const double c = 4.0 * th + a;
             const double E4 = m2 * m2 + 6 * m2 * v + 3 * v * v;
-            ft[t] = c * E2 - 4.0 * E4 - b * m;                 // double_well.py:251
+            ft[0] = c * E2 - 4.0 * E4 - bb * mm;               // double_well.py:251
         } else {
-            ft[t] = E2 * (th - a) + m * b;                     // ornstein_uhlenbeck.py:223
+            ft[0] = E2 * (th - a) + mm * bb;                   // ornstein_uhlenbeck.py:223
         }
         return;
     }
     // Lorenz 63
-    const double* A = x + (long long)t * 9;
-    const double* bt = x + (long long)N * 9 + (long long)t * 3;
-    const double* m = mt + (long long)t * 3;
-    const double* S = st + (long long)t * 9;
+    const double* A = xp + (long long)t * 9;
+    const double* bt = xp + (long long)N * 9 + (long long)t * 3;
+    double* fs = ft + 3;
     const double vS = theta[0], vR = theta[1], vB = theta[2];
     const double mx = m[0], my = m[1], mz = m[2];
     // the reference reads the UPPER triangle of S (lorenz_63.py:388-390, :601-606)
@@ -48,10 +55,10 @@ hyper_small_kernel(int N, const double* __restrict__ theta, const double* __rest
     const double Exxz = Sxx * mz + 2 * Sxz * mx + (mx * mx) * mz;
     const double Exyz = Sxy * mz + Sxz * my + Syz * mx + mx * my * mz;
     // Efg_drift_theta, lorenz_63.py:622-631
-    ft[t * 3 + 0] = Eyy * (vS + A[1]) + Exx * (vS - A[0]) + Exy * (A[0] - 2 * vS - A[1]) + A[2] * (Eyz - Exz) +
+    ft[0] = Eyy * (vS + A[1]) + Exx * (vS - A[0]) + Exy * (A[0] - 2 * vS - A[1]) + A[2] * (Eyz - Exz) +
                     bt[0] * (mx - my);
-    ft[t * 3 + 1] = vR * Exx - Exy - Exxz + A[3] * Exx + A[4] * Exy + A[5] * Exz - bt[1] * mx;
-    ft[t * 3 + 2] = -Exyz + vB * Ezz - A[6] * Exz - A[7] * Eyz - A[8] * Ezz + bt[2] * mz;
+    ft[1] = vR * Exx - Exy - Exxz + A[3] * Exx + A[4] * Exy + A[5] * Exz - bt[1] * mx;
+    ft[2] = -Exyz + vB * Ezz - A[6] * Exz - A[7] * Eyz - A[8] * Ezz + bt[2] * mz;
     // Efg_i = <r_i^2> of the quadratic residual r_i = c + l.x + s x_a x_b (see small_dim.cu: l63_energy)
     const double U[9] = {Sxx, Sxy, Sxz, Sxy, Syy, Syz, Sxz, Syz, Szz};
     const double l[9] = {A[0] - vS, A[1] + vS, A[2], A[3] + vR, A[4] - 1.0, A[5], A[6], A[7], A[8] - vB};
@@ -73,132 +80,45 @@ hyper_small_kernel(int N, const double* __restrict__ theta, const double* __rest
         double q = 0.0;
 #pragma unroll
         for (int r = 0; r < 3; ++r) q += u[r] * (U[r * 3 + 0] * u[0] + U[r * 3 + 1] * u[1] + U[r * 3 + 2] * u[2]);
-        fs[t * 3 + i] = mu * mu + q + extra;
+        fs[i] = mu * mu + q + extra;
     }
 }
 
-// ---- Lorenz 96 (D = 40): one CTA of 128 threads per time index ---------------------------
-// Plain shared-memory code (this kernel is not on the hot path): L = chol(c S) column by column,
-// A L and A m by row loops, then thread i walks the 81 sigma points for component i of the
-// squared residual.  The flattened roll of the reference wraps entries 0, 1 and 39 into the
-// neighbouring sigma points.
-constexpr int HD = 40;
-__global__ void __launch_bounds__(128)
-hyper_l96_kernel(int N, const double* __restrict__ theta, const double* __restrict__ x,
-                 const double* __restrict__ mt, const double* __restrict__ st, double* __restrict__ ft,
-                 double* __restrict__ fs, int* __restrict__ status)
+// ---- trapezoid over t for every component + final scalings: one CTA of 128 threads per problem ----
+// Esde comes from esde_t exactly as finalize computes it (esde_of).  Component c is integrated by warp
+// c % 4: lane l adds the intervals l, l + 32, ... in order, then a fixed xor tree; the order depends on N only.
+__global__ void __launch_bounds__(ESDE_THREADS)
+hyper_reduce_kernel(Batch b, Scratch s, int p0, int count, HyperOut o)
 {
-    __shared__ double L[HD][HD + 1], AL[HD][HD + 1], Am[HD], mv[HD];
-    __shared__ int bad;
-    const int t = blockIdx.x, tid = threadIdx.x;
-    const double* A = x + (long long)t * HD * HD;
-    const double* bt = x + (long long)N * HD * HD + (long long)t * HD;
-    const double* m = mt + (long long)t * HD;
-    const double* S = st + (long long)t * HD * HD;
-    const double th = theta[0];
-    const double kap = 1.05 * HD, c = HD + kap;               // utilities.py:271
-    const double w0 = kap / c, wi = 1.0 / (2.0 * c);          // :290-291
-    if (tid == 0) bad = 0;
-    for (int e = tid; e < HD * HD; e += blockDim.x) {
-        const int i = e / HD, j = e % HD;
-        L[i][j] = (j <= i) ? c * S[i * HD + j] : 0.0;           // lower triangle of c S
-    }
-    if (tid < HD) mv[tid] = m[tid];
-    __syncthreads();
-    for (int k = 0; k < HD; ++k) {                            // right-looking Cholesky
-        if (tid == 0) {
-            const double d = L[k][k];
-            if (!(d > 0.0)) bad = 1;
-            L[k][k] = sqrt(d);
+    __shared__ double sh[ESDE_THREADS];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lp = blockIdx.x, p = p0 + lp, N = b.N, D = b.D;
+    const int nth = hyper_ntheta(b.model, D), W = nth + (D == 1 ? 0 : D);
+    const double* f = s.dEs + (long long)lp * N * W;
+    const double* sg = b.sigma + p * b.sigma_stride;
+    double* dth = o.dth ? o.dth + p * o.dth_stride : nullptr;
+    double* dsig = o.dsig ? o.dsig + p * o.dsig_stride : nullptr;
+    const double Esde = esde_of(b, p, s.esde_t + (long long)lp * N, sh);
+    if (tid == 0 && o.Esde) o.Esde[p] = Esde;
+    for (int c = warp; c < W; c += ESDE_THREADS / 32) {
+        double tz = 0.0;
+        for (int i = lane; i < N - 1; i += 32) tz += b.dt_model * (f[(long long)(i + 1) * W + c] + f[(long long)i * W + c]) / 2.0;
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) tz += __shfl_xor_sync(0xffffffffu, tz, off);
+        if (lane != 0) continue;
+        if (c < nth) {
+            if (dth) dth[c] = (D == 1) ? (b.model == MODEL_DW ? 4.0 * tz : tz) / sg[0] : (1.0 / sg[c]) * tz;
+        } else if (dsig) {
+            const int i = c - nth;
+            dsig[i * D + i] = -0.5 * (1.0 / sg[i]) * tz * (1.0 / sg[i]);
         }
-        __syncthreads();
-        const double dk = L[k][k];
-        for (int i = k + 1 + tid; i < HD; i += blockDim.x) L[i][k] /= dk;
-        __syncthreads();
-        for (int e = tid; e < (HD - k - 1) * (HD - k - 1); e += blockDim.x) {
-            const int i = k + 1 + e / (HD - k - 1), j = k + 1 + e % (HD - k - 1);
-            if (j <= i) L[i][j] -= L[i][k] * L[j][k];
-        }
-        __syncthreads();
     }
-    for (int e = tid; e < HD * HD; e += blockDim.x) {          // A L (L lower) and A m
-        const int i = e / HD, j = e % HD;
-        double a = 0.0;
-        for (int k = j; k < HD; ++k) a = fma(A[i * HD + k], L[k][j], a);
-        AL[i][j] = a;
-    }
-    if (tid < HD) {
-        double a = 0.0;
-        for (int k = 0; k < HD; ++k) a = fma(A[tid * HD + k], mv[k], a);
-        Am[tid] = a;
-    }
-    __syncthreads();
-    if (tid < HD) {
-        const int i = tid, K = 2 * HD + 1;
-        const int f1 = (i + 1) % HD, b1 = (i + HD - 1) % HD, b2 = (i + HD - 2) % HD;
-        // sigma point k: chi_k = m (k = 0), m + L[:, k-1] (k <= D), m - L[:, k-1-D]
-        auto chi = [&](int k, int j) -> double {
-            k = (k + K) % K;
-            if (k == 0) return mv[j];
-            return (k <= HD) ? mv[j] + L[j][k - 1] : mv[j] - L[j][k - 1 - HD];
-        };
-        double mbar = 0.0;
-        for (int k = 0; k < K; ++k) {
-            // flattened np.roll (lorenz_96.py:27-32): neighbours of entry i of row k in the 81 x 40 matrix
-            const double xp1 = (i + 1 < HD) ? chi(k, i + 1) : chi(k + 1, 0);
-            const double xm1 = (i >= 1) ? chi(k, i - 1) : chi(k - 1, HD - 1);
-            const double xm2 = (i >= 2) ? chi(k, i - 2) : chi(k - 1, HD - 2 + i);
-            const double fx = (xp1 - xm2) * xm1 - chi(k, i) + th;
-            double ax = Am[i];
-            if (k >= 1) ax += (k <= HD) ? AL[i][k - 1] : -AL[i][k - 1 - HD];
-            const double r = fx + ax - bt[i];
-            mbar += (k == 0 ? w0 : wi) * (r * r);
-        }
-        fs[(long long)t * HD + i] = mbar;                                       // lorenz_96.py:423
-        const double Ef = (S[f1 * HD + b1] - S[b2 * HD + b1]) + (mv[f1] - mv[b2]) * mv[b1] - mv[i] + th;
-        ft[(long long)t * HD + i] = Ef + Am[i] - bt[i];                         // :420
-    }
-    if (tid == 0 && bad) atomicCAS(status, 0, 1 + t);
-}
-
-// ---- trapezoid over t for every component + final scalings: one CTA -------------------------
-__global__ void __launch_bounds__(256)
-hyper_reduce_kernel(int model, int D, int N, int nth, double dt, const double* __restrict__ sigma,
-                    const double* __restrict__ ft, const double* __restrict__ fs,
-                    const double* __restrict__ esde, double* __restrict__ dth, double* __restrict__ dsig)
-{
-    __shared__ double sh[256];
-    const int tid = threadIdx.x;
-    auto trapz = [&](const double* f, int stride) {
-        double acc = 0.0;
-        for (int i = tid; i < N - 1; i += blockDim.x) acc += dt * (f[(long long)(i + 1) * stride] + f[(long long)i * stride]) / 2.0;
-        sh[tid] = acc;
-        __syncthreads();
-        for (int o = blockDim.x >> 1; o > 0; o >>= 1) {
-            if (tid < o) sh[tid] += sh[tid + o];
-            __syncthreads();
-        }
-        const double r = sh[0];
-        __syncthreads();
-        return r;
-    };
+    if (dsig == nullptr) return;
     if (D == 1) {
-        const double tz = trapz(ft, 1);
-        if (tid == 0) {
-            dth[0] = (model == MODEL_DW ? 4.0 * tz : tz) / sigma[0];
-            dsig[0] = -esde[0] / sigma[0];
-        }
-        return;
-    }
-    for (int e = tid; e < D * D; e += blockDim.x) dsig[e] = 0.0;
-    __syncthreads();
-    for (int i = 0; i < nth; ++i) {
-        const double tz = trapz(ft + i, nth);
-        if (tid == 0) dth[i] = (1.0 / sigma[i]) * tz;
-    }
-    for (int i = 0; i < D; ++i) {
-        const double tz = trapz(fs + i, D);
-        if (tid == 0) dsig[i * D + i] = -0.5 * (1.0 / sigma[i]) * tz * (1.0 / sigma[i]);
+        if (tid == 0) dsig[0] = -Esde / sg[0];
+    } else {
+        for (int e = tid; e < D * D; e += ESDE_THREADS)
+            if (e / D != e % D) dsig[e] = 0.0;
     }
 }
 
@@ -223,20 +143,22 @@ void launch_obs_dr(int N, int M, const long long* obs_t, const double* obs_y, co
     if (M > 0) obs_dr_kernel<<<(M + 127) / 128, 128, 0, stream>>>(M, obs_t, obs_y, R, mt, st, dr);
 }
 
-// ft: N * nth doubles, fs: N * D doubles of device scratch; esde: device pointer to Esde (1-D models);
-// dth (nth values) and dsig (1 or D*D values) are device outputs; status: one int, set to 1 + t when
-// S(t) is not positive definite (L96).
-void launch_hyper(int model, int D, int N, double dt_model, const double* theta, const double* sigma,
-                  const double* x, const double* mt, const double* st, const double* esde, double* ft,
-                  double* fs, double* dth, double* dsig, int* status, cudaStream_t stream)
+void launch_hyper_terms(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count,
+                        cudaStream_t st)
 {
-    const int nth = (model == MODEL_L63) ? 3 : (model == MODEL_L96 ? D : 1);
-    const int bl = (N + 127) / 128;
-    if (model == MODEL_DW) hyper_small_kernel<MODEL_DW><<<bl, 128, 0, stream>>>(N, theta, x, mt, st, ft, fs);
-    else if (model == MODEL_OU) hyper_small_kernel<MODEL_OU><<<bl, 128, 0, stream>>>(N, theta, x, mt, st, ft, fs);
-    else if (model == MODEL_L63) hyper_small_kernel<MODEL_L63><<<bl, 128, 0, stream>>>(N, theta, x, mt, st, ft, fs);
-    else hyper_l96_kernel<<<N, 128, 0, stream>>>(N, theta, x, mt, st, ft, fs, status);
-    hyper_reduce_kernel<<<1, 256, 0, stream>>>(model, D, N, nth, dt_model, sigma, ft, fs, esde, dth, dsig);
+    if (b.model == MODEL_L96) {
+        launch_l96_hyper(b, s, x, xs, p0, count, st);
+        return;
+    }
+    const unsigned bl = (unsigned)(((long long)count * b.N + 127) / 128);
+    if (b.model == MODEL_DW)      hyper_small_kernel<MODEL_DW><<<bl, 128, 0, st>>>(b, s, x, xs, p0, count);
+    else if (b.model == MODEL_OU) hyper_small_kernel<MODEL_OU><<<bl, 128, 0, st>>>(b, s, x, xs, p0, count);
+    else                          hyper_small_kernel<MODEL_L63><<<bl, 128, 0, st>>>(b, s, x, xs, p0, count);
+}
+
+void launch_hyper_reduce(const Batch& b, const Scratch& s, int p0, int count, const HyperOut& o, cudaStream_t st)
+{
+    hyper_reduce_kernel<<<count, ESDE_THREADS, 0, st>>>(b, s, p0, count, o);
 }
 
 }  // namespace vgpa

@@ -847,39 +847,19 @@ small_bwd_kernel(Batch b, Scratch s, SmallBwdArgs a, int p0, int count, Extra ex
 // ---------------------------------------------------------------------------
 // F = E0 + Esde + Eobs : one CTA per problem, fixed-order reductions (bitwise
 // reproducible, so a sharded batch returns the same F as a single-GPU one).
+// block_sum and esde_of: common.cuh.
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ double block_sum(double v, double* sh)
-{
-    const int tid = threadIdx.x;
-    sh[tid] = v;
-    __syncthreads();
-    for (int o = blockDim.x >> 1; o > 0; o >>= 1) {
-        if (tid < o) sh[tid] += sh[tid + o];
-        __syncthreads();
-    }
-    const double r = sh[0];
-    __syncthreads();
-    return r;
-}
 
 // The free energy of problem p from its Esde integrand f(t) and its moments (global or shared memory); every
 // thread of the CTA (128 threads or more) calls it, every thread gets the value.  parts: E0, Esde, Eobs (or null).
 __device__ __forceinline__ double free_energy_of(const Batch& b, int p, const double* f, const double* mt,
                                                  const double* st, double* sh, double* parts)
 {
-    // The partial sums are taken by the first 128 threads whatever the CTA size (the rest add zeros to the
-    // reduction tree), so that F is the same bits from finalize_kernel (128 threads) and from the fused D = 1
-    // evaluation (SCAN_THREADS).
-    constexpr int W = 128;
+    constexpr int W = ESDE_THREADS;
     const int tid = threadIdx.x;
-    const int N = b.N, D = b.D, M = b.M, DD = D * D;
-    // utilities.py:144-201: composite trapezoid, sum(dx * (f[i+1] + f[i]) / 2)
-    double acc = 0.0;
-    if (tid < W)
-        for (int i = tid; i < N - 1; i += W) acc += b.dt_model * (f[i + 1] + f[i]) / 2.0;
-    double Esde = block_sum(acc, sh);
-    if (b.model == MODEL_DW || b.model == MODEL_OU)  // double_well.py:217, ornstein_uhlenbeck.py:208
-        Esde = 0.5 * Esde / b.sigma[p * b.sigma_stride];
+    const int D = b.D, M = b.M, DD = D * D;
+    const double Esde = esde_of(b, p, f, sh);
+    double acc;
     // observation energy
     const double* oy = b.obs_y + p * b.obs_y_stride;
     const double* R = b.R + p * b.R_stride;

@@ -121,6 +121,52 @@ class BatchEvaluator:
     def sync(self):
         raise_for(lib.vgpa_sync(self._h), self._h)
 
+    @property
+    def n_theta(self):
+        """Entries of dEsde_dtheta per problem: 1 (DW, OU), 3 (L63), D (L96, lorenz_96.py:431)."""
+        return {"DW": 1, "OU": 1, "L63": 3, "L96": self.D}[self.model]
+
+    def hyper_device(self, x_ptr, x_stride, F_ptr=None, Esde_ptr=None, dtheta_ptr=None, dtheta_stride=None,
+                     dsigma_ptr=None, dsigma_stride=None, stream=0):
+        """model.energy's hyper-parameter gradients for every problem at its x row (vgpa_hyper_device): device
+        pointers (ints), asynchronous on `stream`; call sync() afterwards.  Any output may be None; default strides
+        are compact rows (n_theta and 1 or D*D values)."""
+        nsig = 1 if self.D == 1 else self.D * self.D
+        rc = lib.vgpa_hyper_device(self._h, x_ptr, x_stride, F_ptr, Esde_ptr, dtheta_ptr,
+                                   self.n_theta if dtheta_stride is None else dtheta_stride, dsigma_ptr,
+                                   nsig if dsigma_stride is None else dsigma_stride, stream or None)
+        raise_for(rc, self._h)
+
+    def hyper(self, X):
+        """F, Esde, dEsde_dtheta and dEsde_dsigma of every problem at its x: X (n_x,) shared by all problems or
+        (B, n_x), a host array or a CUDA tensor.  Returns a dict of host arrays; each problem's entries have the
+        shapes StochasticProcess.energy returns: F, Esde (B,); dEsde_dtheta (B,) for D = 1, else (B, n_theta);
+        dEsde_dsigma (B,) for D = 1, else (B, D, D)."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        Xt = torch.as_tensor(X, dtype=torch.float64, device=dev)
+        if Xt.numel() == self.n_x:
+            Xt, xs = Xt.reshape(1, self.n_x).contiguous(), 0
+        elif Xt.numel() == self.B * self.n_x:
+            Xt, xs = Xt.reshape(self.B, self.n_x).contiguous(), self.n_x
+        else:
+            raise ValueError(f"x: expected {self.n_x} or {self.B}x{self.n_x} values, got {Xt.numel()}")
+        B, D, nth = self.B, self.D, self.n_theta
+        F, Esde = (torch.empty(B, dtype=torch.float64, device=dev) for _ in range(2))
+        dth = torch.empty((B, nth), dtype=torch.float64, device=dev)
+        dsig = torch.empty((B, 1 if D == 1 else D * D), dtype=torch.float64, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        self.hyper_device(Xt.data_ptr(), xs, F.data_ptr(), Esde.data_ptr(), dth.data_ptr(), nth, dsig.data_ptr(),
+                          dsig.shape[1], stream)
+        self.sync()
+        out = {"F": F.cpu().numpy(), "Esde": Esde.cpu().numpy(), "dEsde_dtheta": dth.cpu().numpy(),
+               "dEsde_dsigma": dsig.cpu().numpy()}
+        if D == 1:
+            out["dEsde_dtheta"], out["dEsde_dsigma"] = out["dEsde_dtheta"][:, 0], out["dEsde_dsigma"][:, 0]
+        else:
+            out["dEsde_dsigma"] = out["dEsde_dsigma"].reshape(B, D, D)
+        return out
+
     def set_active(self, mask_ptr=None):
         """Device pointer to B int32 flags (0 = skip the problem in the following eval_device calls:
         its F and gradient row stay untouched), or None for every problem."""
