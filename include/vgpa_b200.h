@@ -16,8 +16,9 @@
  *
  * Scope: diagonal system noise Sigma, diagonal observation noise R, identity
  * observation operator -- everything the sim_params JSON schema can express
- * (vgpa_main.py:38-40, simulation.py:107-176).  L96 is built for D = 40
- * (the only size simulation.py:20,134 can construct).
+ * (vgpa_main.py:38-40, simulation.py:107-176).  L96 takes any 10 <= D <= 64
+ * (lorenz_96.py:104-140 accepts dim_d >= 10): D = 40, the only size simulation.py:20,134
+ * constructs, runs hand-tuned kernels, every other D a run-time-D kernel family.
  *
  * Return codes (mapped to the exceptions the reference raises):
  *     VGPA_OK            0
@@ -61,7 +62,7 @@ typedef struct vgpa_handle vgpa_handle;
 typedef struct {
     int32_t model;   /* VGPA_MODEL_*                                              */
     int32_t method;  /* VGPA_ODE_*                                                */
-    int32_t D;       /* state dimension (1, 3 or 40)                              */
+    int32_t D;       /* state dimension (DW, OU: 1; L63: 3; L96: 10 <= D <= 64)   */
     int32_t N;       /* number of time-grid points = len(np.arange(t0,tf+dt,dt))  */
     int32_t M;       /* number of observations                                    */
     int32_t B;       /* number of independent problems in the batch               */
@@ -112,7 +113,7 @@ int vgpa_eval(vgpa_handle *h, const double *x, int64_t x_stride, int want_grad,
  * problems that have converged. */
 int vgpa_set_active(vgpa_handle *h, const int32_t *d_active);
 
-/* Compacted launches for thinned-out ensembles (Lorenz-96, D = 40 only): `list` = n problem indices in
+/* Compacted launches for thinned-out ensembles (Lorenz-96 handles only): `list` = n problem indices in
  * HOST memory (copied), or NULL / n < 0 to switch the mode off.  The following vgpa_eval_device calls
  * evaluate exactly the listed problems, chunked by list position, so that every pass still fills whole
  * waves of the GPU when most problems of a batch have converged (an active-flag mask alone leaves the
@@ -223,7 +224,9 @@ int vgpa_initialization_host(vgpa_handle *h, double t0, double *x, int64_t x_str
  *           (their start consumes the generator, double_well.py:145-151), NULL for L63 / L96 = the
  *           reference's 5000-step burn-in from its fixed starting point
  *   path  : (N, D) per path, row stride path_stride
- * vgpa_make_trajectory: HOST buffers, synchronous.  _device: DEVICE buffers, asynchronous on `stream`. */
+ * vgpa_make_trajectory: HOST buffers, synchronous.  _device: DEVICE buffers, asynchronous on `stream`.
+ * Both take D from the model (L96: 40); the _dim variants take it as an argument (L96: 10 <= D <= 64,
+ * the burn-in perturbs component int(D / 2); the other models: their fixed D). */
 int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const double *theta,
                          int64_t theta_stride, const double *sigma, int64_t sigma_stride,
                          const double *x_init, int64_t x_init_stride, const double *z, int64_t z_stride,
@@ -232,6 +235,14 @@ int vgpa_make_trajectory_device(int device, int model, int N, int B, double dt, 
                                 int64_t theta_stride, const double *d_sigma, int64_t sigma_stride,
                                 const double *d_x_init, int64_t x_init_stride, const double *d_z,
                                 int64_t z_stride, double *d_path, int64_t path_stride, void *stream);
+int vgpa_make_trajectory_dim(int device, int model, int D, int N, int B, double dt, const double *theta,
+                             int64_t theta_stride, const double *sigma, int64_t sigma_stride,
+                             const double *x_init, int64_t x_init_stride, const double *z, int64_t z_stride,
+                             double *path, int64_t path_stride);
+int vgpa_make_trajectory_device_dim(int device, int model, int D, int N, int B, double dt, const double *d_theta,
+                                    int64_t theta_stride, const double *d_sigma, int64_t sigma_stride,
+                                    const double *d_x_init, int64_t x_init_stride, const double *d_z,
+                                    int64_t z_stride, double *d_path, int64_t path_stride, void *stream);
 
 /* StochasticProcess.collect_obs (stochastic_process.py:130-230) for B observation sets:
  * obs_y[p][j][i] = path[p][obs_t[j]][i] + sqrt(R[p][i]) * xi[p][i][j]   (xi: (D, M) draws, the

@@ -16,7 +16,24 @@ LIB_PATH = Path(os.environ["VGPA_LIB"]) if os.environ.get("VGPA_LIB") else PKG /
 VGPA_OK, VGPA_EINVAL, VGPA_ENOTPD, VGPA_ECUDA = 0, 1, 2, 3
 MODELS = {"DW": 0, "OU": 1, "L63": 2, "L96": 3}
 METHODS = {"euler": 0, "heun": 1, "rk2": 2, "rk4": 3}
-MODEL_DIM = {"DW": 1, "OU": 1, "L63": 3, "L96": 40}
+MODEL_DIM = {"DW": 1, "OU": 1, "L63": 3, "L96": 40}   # the default D; Lorenz 96 takes any 10 <= D <= 64
+L96_DIMS = (10, 64)
+
+
+def model_dim(key, D=None):
+    """State dimension of a model: its fixed D, or for L96 the given D (default 40) checked against
+    10 <= D <= 64."""
+    if D is None:
+        return MODEL_DIM[key]
+    D = int(D)
+    if key == "L96":
+        if D < L96_DIMS[0]:
+            raise ValueError(f" Lorenz96: Insufficient state vector dimensions: {D}")
+        if D > L96_DIMS[1]:
+            raise ValueError(f" Lorenz96: dim_d = {D} is outside the supported range {L96_DIMS[0]} <= dim_d <= {L96_DIMS[1]}")
+    elif D != MODEL_DIM[key]:
+        raise ValueError(f" {key}: state dimension {D}, expected {MODEL_DIM[key]}")
+    return D
 
 _dp = C.POINTER(C.c_double)
 _ip = C.POINTER(C.c_int64)
@@ -87,7 +104,10 @@ def _load():
     i64 = C.c_int64
     traj = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double] + [C.c_void_p, i64] * 5
     obs = [C.c_int] * 5 + [C.c_void_p] + [C.c_void_p, i64] * 4
+    traj_dim = traj[:2] + [C.c_int] + traj[2:]
     for name, args in (("vgpa_make_trajectory", traj), ("vgpa_make_trajectory_device", traj + [C.c_void_p]),
+                       ("vgpa_make_trajectory_dim", traj_dim),
+                       ("vgpa_make_trajectory_device_dim", traj_dim + [C.c_void_p]),
                        ("vgpa_collect_obs", obs), ("vgpa_collect_obs_device", obs + [C.c_void_p])):
         fn = getattr(lib, name)
         fn.restype = C.c_int

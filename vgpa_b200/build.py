@@ -15,7 +15,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libvgpa_b200.so"
 SOURCES = ["api.cu", "small_dim.cu", "l63_lanes.cu", "l96_sweeps.cu", "l96_energy.cu", "vecops.cu", "hyper.cu", "init.cu",
-           "datagen.cu"]
+           "datagen.cu", "l96_dyn.cu"]
 HEADERS = ["common.cuh", "ptx.cuh", "l63_grad.cuh", "../../include/vgpa_b200.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]

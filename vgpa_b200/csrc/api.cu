@@ -278,6 +278,25 @@ namespace {
 
 bool small_model(int model) { return model != VGPA_MODEL_L96; }
 
+// Lorenz 96: the tuned kernels at D = 40, the run-time-D family (l96_dyn.cu) at every other D
+void l96_fwd(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count, cudaStream_t st)
+{
+    if (l96_tuned(b.D)) launch_l96_fwd(b, s, x, xs, p0, count, st);
+    else launch_l96d_fwd(b, s, x, xs, p0, count, st);
+}
+void l96_energy(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count, const Extra& ex,
+                cudaStream_t st)
+{
+    if (l96_tuned(b.D)) launch_l96_energy(b, s, x, xs, p0, count, ex, st);
+    else launch_l96d_energy(b, s, x, xs, p0, count, ex, st);
+}
+void l96_bwd(const Batch& b, const Scratch& s, const double* x, long long xs, double* g, long long gs, int p0, int count,
+             const Extra& ex, cudaStream_t st)
+{
+    if (l96_tuned(b.D)) launch_l96_bwd(b, s, x, xs, g, gs, p0, count, ex, st);
+    else launch_l96d_bwd(b, s, x, xs, g, gs, p0, count, ex, st);
+}
+
 // one pass over problems [p0, p0 + count) with device buffers
 void run_chunk(vgpa_handle* h, const double* d_x, long long xs, int want_grad, double* d_F, double* d_grad,
                long long gs, int p0, int count, const Extra& ex, cudaStream_t st)
@@ -292,11 +311,11 @@ void run_chunk(vgpa_handle* h, const double* d_x, long long xs, int want_grad, d
         return;
     }
     if (small) launch_small_fwd(b, sc, d_x, xs, p0, count, st);
-    else launch_l96_fwd(b, sc, d_x, xs, p0, count, st);
+    else l96_fwd(b, sc, d_x, xs, p0, count, st);
     h->tick(0, st, false);
     h->tick(1, st, true);
     if (small) launch_small_energy(b, sc, d_x, xs, p0, count, ex, st);
-    else launch_l96_energy(b, sc, d_x, xs, p0, count, ex, st);
+    else l96_energy(b, sc, d_x, xs, p0, count, ex, st);
     h->tick(1, st, false);
     h->tick(2, st, true);
     launch_finalize(b, sc, d_F, p0, count, ex, st);
@@ -305,7 +324,7 @@ void run_chunk(vgpa_handle* h, const double* d_x, long long xs, int want_grad, d
     if (want_grad) {
         h->tick(3, st, true);
         if (small) launch_small_bwd(b, sc, d_x, xs, d_grad, gs, p0, count, ex, st);
-        else launch_l96_bwd(b, sc, d_x, xs, d_grad, gs, p0, count, ex, st);
+        else l96_bwd(b, sc, d_x, xs, d_grad, gs, p0, count, ex, st);
         h->tick(3, st, false);
         h->launches += 1;
     }
@@ -321,7 +340,7 @@ void run_hyper_chunk(vgpa_handle* h, const double* d_x, long long xs, double* d_
     const bool small = small_model(b.model);
     h->tick(0, st, true);
     if (small) launch_small_fwd(b, sc, d_x, xs, p0, count, st);
-    else launch_l96_fwd(b, sc, d_x, xs, p0, count, st);
+    else l96_fwd(b, sc, d_x, xs, p0, count, st);
     h->tick(0, st, false);
     h->tick(1, st, true);
     if (small) launch_small_energy(b, sc, d_x, xs, p0, count, Extra{}, st);
@@ -400,8 +419,14 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
     if (d->model < 0 || d->model > 3) return bail(h->fail(VGPA_EINVAL, "Unknown stochastic model -> %d", d->model));
     if (d->method < 0 || d->method > 3)
         return bail(h->fail(VGPA_EINVAL, "Integration method is unknown -> %d", d->method));
-    const int needD = (d->model == VGPA_MODEL_L63) ? 3 : (d->model == VGPA_MODEL_L96 ? 40 : 1);
-    if (d->D != needD) return bail(h->fail(VGPA_EINVAL, "Wrong state dimension %d for model %d (need %d)", d->D, d->model, needD));
+    if (d->model == VGPA_MODEL_L96) {
+        if (d->D < 10) return bail(h->fail(VGPA_EINVAL, " Lorenz96: Insufficient state vector dimensions: %d", d->D));
+        if (d->D > 64)
+            return bail(h->fail(VGPA_EINVAL, "Wrong state dimension %d for Lorenz 96 (supported: 10 <= D <= 64)", d->D));
+    } else {
+        const int needD = (d->model == VGPA_MODEL_L63) ? 3 : 1;
+        if (d->D != needD) return bail(h->fail(VGPA_EINVAL, "Wrong state dimension %d for model %d (need %d)", d->D, d->model, needD));
+    }
     if (d->N < 2) return bail(h->fail(VGPA_EINVAL, "Need at least two time points, got %d", d->N));
     if (d->M < 0 || d->B < 1) return bail(h->fail(VGPA_EINVAL, "Wrong sizes M=%d B=%d", d->M, d->B));
     if (!(d->dt > 0.0) || !(d->dt_model > 0.0))
@@ -485,8 +510,9 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
     long long budget = d->scratch_bytes > 0 ? d->scratch_bytes : std::min<long long>(56LL << 30, (long long)(free_b * 0.35));
     long long chunk = std::max<long long>(1, std::min<long long>(B, budget / per));
     if (!small_model(d->model) && chunk < B) {
-        if (d->scratch_bytes > 0) {
-            // caller-given budget: whole waves (multiples of 6 * 148: 3 backward / 4 forward CTAs per SM) when it allows
+        if (d->scratch_bytes > 0 && l96_tuned(D)) {
+            // caller-given budget: whole waves (multiples of 6 * 148: 3 backward / 4 forward CTAs per SM of the D = 40
+            // kernels) when it allows
             const long long wave = 148 * 6;
             if (chunk >= wave) chunk = (chunk / wave) * wave;
             else if (chunk >= 148) chunk = (chunk / 148) * 148;
@@ -648,7 +674,7 @@ int vgpa_set_active_list(vgpa_handle* h, const int32_t* list, int32_t n)
         return VGPA_OK;
     }
     if (h->batch.model != MODEL_L96)
-        return h->fail(VGPA_EINVAL, "vgpa_set_active_list: compacted launches exist for the D = 40 kernels only "
+        return h->fail(VGPA_EINVAL, "vgpa_set_active_list: compacted launches exist for the Lorenz-96 kernels only "
                                     "(use vgpa_set_active for the small models)");
     if (n > h->d.B) return h->fail(VGPA_EINVAL, "vgpa_set_active_list: %d entries for %d problems", (int)n, h->d.B);
     for (int k = 0; k < n; ++k)
@@ -818,7 +844,8 @@ int vgpa_eval_full(vgpa_handle* h, int64_t problem, const double* x, const vgpa_
 static int check_sweep_args(int method, int D, int N, double dt)
 {
     if (method < 0 || method > 3) return set_error(VGPA_EINVAL, "Integration method is unknown");
-    if (D != 1 && D != 3 && D != 40) return set_error(VGPA_EINVAL, "unsupported state dimension (1, 3 or 40)");
+    if (D != 1 && D != 3 && (D < 10 || D > 64))
+        return set_error(VGPA_EINVAL, "unsupported state dimension %d (1, 3 or 10 <= D <= 64)", D);
     if (N < 2) return set_error(VGPA_EINVAL, "need at least two time points");
     if (!(dt > 0.0)) return set_error(VGPA_EINVAL, "Discrete time step should be strictly positive");
     return VGPA_OK;
@@ -843,12 +870,12 @@ int vgpa_solve_fwd(int device, int method, int D, int N, double dt, const double
     alloc(e, dst, nm);
     if (e != cudaSuccess) return set_cuda_error(e, "vgpa_solve_fwd");
     Batch bt{};
-    bt.model = (D == 40) ? MODEL_L96 : (D == 3 ? MODEL_L63 : MODEL_OU);
+    bt.model = (D >= 10) ? MODEL_L96 : (D == 3 ? MODEL_L63 : MODEL_OU);
     bt.method = method; bt.D = D; bt.N = N; bt.B = 1; bt.dt = dt; bt.dt_model = dt;
     bt.sigma = dsig.as<double>(); bt.m0 = dm0.as<double>(); bt.s0 = ds0.as<double>();
     Scratch sc{};
     sc.mt = dmt.as<double>(); sc.st = dst.as<double>();
-    if (D == 40) launch_l96_fwd(bt, sc, dx.as<double>(), 0, 0, 1, nullptr);
+    if (D >= 10) l96_fwd(bt, sc, dx.as<double>(), 0, 0, 1, nullptr);
     else launch_small_fwd(bt, sc, dx.as<double>(), 0, 0, 1, nullptr);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
@@ -888,8 +915,8 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
                       double* Esde, double* Ef, double* Edf, double* dEm, double* dEs, double* dEth, double* dEsig)
 {
     if (model < 0 || model > 3) return set_error(VGPA_EINVAL, "Unknown stochastic model");
-    const int needD = (model == VGPA_MODEL_L63) ? 3 : (model == VGPA_MODEL_L96 ? 40 : 1);
-    if (D != needD || N < 2 || !(dt_model > 0.0)) return set_error(VGPA_EINVAL, "Wrong dimensions for model.energy");
+    const bool okD = (model == VGPA_MODEL_L96) ? (D >= 10 && D <= 64) : (D == ((model == VGPA_MODEL_L63) ? 3 : 1));
+    if (!okD || N < 2 || !(dt_model > 0.0)) return set_error(VGPA_EINVAL, "Wrong dimensions for model.energy");
     if (!theta || !sigma || !A || !b || !m || !S || !Esde || !Ef || !Edf || !dEm || !dEs)
         return set_error(VGPA_EINVAL, "NULL argument");
     if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
@@ -929,7 +956,7 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
     sc.esde_t = des.as<double>(); sc.status = dstat.as<int>();
     Extra ex{};
     ex.Efx = def.as<double>(); ex.Edf = dedf.as<double>(); ex.parts = dparts.as<double>();
-    if (model == VGPA_MODEL_L96) launch_l96_energy(bt, sc, dx.as<double>(), 0, 0, 1, ex, nullptr);
+    if (model == VGPA_MODEL_L96) l96_energy(bt, sc, dx.as<double>(), 0, 0, 1, ex, nullptr);
     else launch_small_energy(bt, sc, dx.as<double>(), 0, 0, 1, ex, nullptr);
     launch_finalize(bt, sc, dF.as<double>(), 0, 1, ex, nullptr);
     if (hyper) {   // the launchers of vgpa_hyper_device with B = 1; the integrands go to a buffer of their own
@@ -963,7 +990,8 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
 int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const double* obs_y, const double* R,
                     const double* mt, const double* st, double* Eobs, double* jm, double* js, double* dr)
 {
-    if ((D != 1 && D != 3 && D != 40) || N < 2 || M < 0 || M > N) return set_error(VGPA_EINVAL, "Wrong dimensions for the likelihood");
+    if ((D != 1 && D != 3 && (D < 10 || D > 64)) || N < 2 || M < 0 || M > N)
+        return set_error(VGPA_EINVAL, "Wrong dimensions for the likelihood");
     if ((M > 0 && (!obs_t || !obs_y)) || !R || !mt || !st || !Eobs || !jm || !js) return set_error(VGPA_EINVAL, "NULL argument");
     for (int n = 0; n < M; ++n)
         if (obs_t[n] < 0 || obs_t[n] >= N) return set_error(VGPA_EINVAL, "observation index out of range");
@@ -1091,11 +1119,15 @@ int vgpa_initialization_host(vgpa_handle* h, double t0, double* x, int64_t x_str
 static int model_dim(int model) { return model == VGPA_MODEL_L96 ? 40 : (model == VGPA_MODEL_L63 ? 3 : 1); }
 static int traj_ntheta(int model) { return model == VGPA_MODEL_L63 ? 3 : (model == VGPA_MODEL_OU ? 2 : 1); }
 
-static int check_traj_args(int model, int N, int B, double dt, const void* theta, const void* sigma,
+static int check_traj_args(int model, int D, int N, int B, double dt, const void* theta, const void* sigma,
                            const void* x_init, const void* z, const void* path, int64_t z_stride, int64_t path_stride)
 {
     if (model < 0 || model > 3) return set_error(VGPA_EINVAL, "Unknown stochastic model");
-    const int D = model_dim(model);
+    if (model == VGPA_MODEL_L96 && D < 10) return set_error(VGPA_EINVAL, " Lorenz96: Insufficient state vector dimensions: %d", D);
+    if (model == VGPA_MODEL_L96 && D > 64)
+        return set_error(VGPA_EINVAL, "Wrong state dimension %d for Lorenz 96 (supported: 10 <= D <= 64)", D);
+    if (model != VGPA_MODEL_L96 && D != model_dim(model))
+        return set_error(VGPA_EINVAL, "Wrong state dimension %d for model %d (need %d)", D, model, model_dim(model));
     if (N < 1 || B < 1) return set_error(VGPA_EINVAL, "need N >= 1 time points and B >= 1 paths");
     if (!(dt > 0.0)) return set_error(VGPA_EINVAL, "Discrete time step should be strictly positive");
     if (!theta || !sigma || !z || !path) return set_error(VGPA_EINVAL, "NULL argument");
@@ -1105,29 +1137,37 @@ static int check_traj_args(int model, int N, int B, double dt, const void* theta
     return VGPA_OK;
 }
 
-int vgpa_make_trajectory_device(int device, int model, int N, int B, double dt, const double* d_theta, int64_t theta_stride,
-                                const double* d_sigma, int64_t sigma_stride, const double* d_x_init, int64_t x_init_stride,
-                                const double* d_z, int64_t z_stride, double* d_path, int64_t path_stride, void* stream)
+int vgpa_make_trajectory_device_dim(int device, int model, int D, int N, int B, double dt, const double* d_theta,
+                                    int64_t theta_stride, const double* d_sigma, int64_t sigma_stride, const double* d_x_init,
+                                    int64_t x_init_stride, const double* d_z, int64_t z_stride, double* d_path,
+                                    int64_t path_stride, void* stream)
 {
-    if (int rc = check_traj_args(model, N, B, dt, d_theta, d_sigma, d_x_init, d_z, d_path, z_stride, path_stride)) return rc;
+    if (int rc = check_traj_args(model, D, N, B, dt, d_theta, d_sigma, d_x_init, d_z, d_path, z_stride, path_stride)) return rc;
     if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
-    TrajArgs a{model, model_dim(model), N, B, dt, d_theta, theta_stride, d_sigma, sigma_stride, d_x_init, x_init_stride,
+    TrajArgs a{model, D, N, B, dt, d_theta, theta_stride, d_sigma, sigma_stride, d_x_init, x_init_stride,
                d_z, z_stride, d_path, path_stride};
     launch_trajectories(a, static_cast<cudaStream_t>(stream));
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_make_trajectory_device");
 }
 
-int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const double* theta, int64_t theta_stride,
-                         const double* sigma, int64_t sigma_stride, const double* x_init, int64_t x_init_stride,
-                         const double* z, int64_t z_stride, double* path, int64_t path_stride)
+int vgpa_make_trajectory_device(int device, int model, int N, int B, double dt, const double* d_theta, int64_t theta_stride,
+                                const double* d_sigma, int64_t sigma_stride, const double* d_x_init, int64_t x_init_stride,
+                                const double* d_z, int64_t z_stride, double* d_path, int64_t path_stride, void* stream)
 {
-    if (int rc = check_traj_args(model, N, B, dt, theta, sigma, x_init, z, path, z_stride, path_stride)) return rc;
-    if ((theta_stride != 0 && theta_stride < traj_ntheta(model)) || (sigma_stride != 0 && sigma_stride < model_dim(model)) ||
-        (x_init && x_init_stride != 0 && x_init_stride < model_dim(model)))
+    return vgpa_make_trajectory_device_dim(device, model, model_dim(model), N, B, dt, d_theta, theta_stride, d_sigma,
+                                           sigma_stride, d_x_init, x_init_stride, d_z, z_stride, d_path, path_stride, stream);
+}
+
+int vgpa_make_trajectory_dim(int device, int model, int D, int N, int B, double dt, const double* theta,
+                             int64_t theta_stride, const double* sigma, int64_t sigma_stride, const double* x_init,
+                             int64_t x_init_stride, const double* z, int64_t z_stride, double* path, int64_t path_stride)
+{
+    if (int rc = check_traj_args(model, D, N, B, dt, theta, sigma, x_init, z, path, z_stride, path_stride)) return rc;
+    if ((theta_stride != 0 && theta_stride < traj_ntheta(model)) || (sigma_stride != 0 && sigma_stride < D) ||
+        (x_init && x_init_stride != 0 && x_init_stride < D))
         return set_error(VGPA_EINVAL, "theta_stride / sigma_stride / x_init_stride shorter than one entry (0 = shared)");
     if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
-    const int D = model_dim(model);
     const int64_t len = (int64_t)N * D;
     DevBuf dth, dsg, dxi, dz, dp;
     TrajArgs a{};
@@ -1150,9 +1190,18 @@ int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const d
     return e == cudaSuccess ? VGPA_OK : set_cuda_error(e, "vgpa_make_trajectory");
 }
 
+int vgpa_make_trajectory(int device, int model, int N, int B, double dt, const double* theta, int64_t theta_stride,
+                         const double* sigma, int64_t sigma_stride, const double* x_init, int64_t x_init_stride,
+                         const double* z, int64_t z_stride, double* path, int64_t path_stride)
+{
+    return vgpa_make_trajectory_dim(device, model, model_dim(model), N, B, dt, theta, theta_stride, sigma, sigma_stride,
+                                    x_init, x_init_stride, z, z_stride, path, path_stride);
+}
+
 static int check_obs_args(int D, int N, int M, int B, const int64_t* obs_t /* host, or NULL = not checked */)
 {
-    if (D != 1 && D != 3 && D != 40) return set_error(VGPA_EINVAL, "unsupported state dimension (1, 3 or 40)");
+    if (D != 1 && D != 3 && (D < 10 || D > 64))
+        return set_error(VGPA_EINVAL, "unsupported state dimension %d (1, 3 or 10 <= D <= 64)", D);
     if (N < 1 || M < 0 || B < 1) return set_error(VGPA_EINVAL, "need N >= 1, M >= 0, B >= 1");
     for (int j = 0; obs_t && j < M; ++j)
         if (obs_t[j] < 0 || obs_t[j] >= N) return set_error(VGPA_EINVAL, "observation index outside the time grid");

@@ -45,7 +45,7 @@ struct Batch {
     const double* E0;     long long E0_stride;
     const int* active;        // B flags or null: problems whose flag is 0 are skipped by every kernel
                               // (their F, gradient and scratch rows are left untouched)
-    const int* plist;         // or null.  Compacted launches of the D = 40 kernels (vgpa_set_active_list): the
+    const int* plist;         // or null.  Compacted launches of the Lorenz-96 kernels (vgpa_set_active_list): the
                               // pass covers list positions [p0, p0 + count) and the problem at position k is
                               // plist[k], so that a thinned-out ensemble still fills whole waves
 };
@@ -171,6 +171,22 @@ void launch_l96_energy(const Batch& b, const Scratch& s, const double* x, long l
 void launch_l96_bwd(const Batch& b, const Scratch& s, const double* x, long long x_stride,
                     double* grad, long long grad_stride, int p0, int count, const Extra& ex,
                     cudaStream_t st);
+
+// Lorenz 96 at a run-time 10 <= D <= 64 other than 40 (l96_dyn.cu); the same contracts as the D = 40 launchers.
+// D = 40 always runs the tuned kernels above.
+__host__ __device__ inline bool l96_tuned(int D) { return D == 40; }
+void launch_l96d_fwd(const Batch& b, const Scratch& s, const double* x, long long x_stride,
+                     int p0, int count, cudaStream_t st);
+void launch_l96d_energy(const Batch& b, const Scratch& s, const double* x, long long x_stride,
+                        int p0, int count, const Extra& ex, cudaStream_t st);
+void launch_l96d_hyper(const Batch& b, const Scratch& s, const double* x, long long xs, int p0, int count,
+                       cudaStream_t st);
+void launch_l96d_bwd(const Batch& b, const Scratch& s, const double* x, long long x_stride,
+                     double* grad, long long grad_stride, int p0, int count, const Extra& ex,
+                     cudaStream_t st);
+void launch_bwd_dense_l96d(int method, int D, int N, double dt, const double* A, const double* dEm,
+                           const double* dEs, const double* jm, const double* js, double* lam, double* psi,
+                           cudaStream_t st);
 
 // F[p] = E0 + trapz(esde_t) (/sigma for DW, OU) + Eobs.
 void launch_finalize(const Batch& b, const Scratch& s, double* F, int p0, int count,

@@ -12,8 +12,8 @@
 // generator) produces the stream and the device does the arithmetic.  Every operation is a single
 // correctly rounded IEEE operation in the reference's evaluation order (no FMA contraction), so a
 // path is bit-identical to the numpy loop given the same draws.  The recurrences are sequential in t:
-// one thread per path for D = 1, 3, one 64-thread CTA per path for D = 40 (neighbour exchange
-// through a double-buffered shared-memory state, one barrier per step).
+// one thread per path for D = 1, 3, one 64-thread CTA per path for Lorenz 96 (D = 40, and any other
+// 10 <= D <= 64; neighbour exchange through a double-buffered shared-memory state, one barrier per step).
 #include "common.cuh"
 
 namespace vgpa {
@@ -120,6 +120,46 @@ traj_l96_kernel(TrajArgs a)
     }
 }
 
+// Lorenz 96 at a run-time D <= 64 other than 40 (the D = 40 kernel above stays as it is): the same loop,
+// thread i owns component i; the burn-in perturbs component int(D / 2) (lorenz_96.py:269-275).
+__global__ void __launch_bounds__(64)
+traj_l96d_kernel(TrajArgs a)
+{
+    __shared__ double xs[2][64];
+    const int D = a.D, p = blockIdx.x, i = threadIdx.x;
+    const bool on = i < D;
+    const int N = a.N;
+    const double u = a.theta[p * a.theta_stride];
+    const double* z = a.z + p * a.z_stride + (long long)(on ? i : 0) * N;
+    double* out = a.path + p * a.path_stride;
+    const int ip1 = (i + 1) % D, im1 = (i + D - 1) % D, im2 = (i + D - 2) % D;
+    double x = 0.0;
+    int par = 0;
+    auto drift = [&](double xi) {
+        if (on) xs[par][i] = xi;
+        __syncthreads();
+        double f = 0.0;
+        if (on) f = add(sub(mul(sub(xs[par][ip1], xs[par][im2]), xs[par][im1]), xi), u);
+        par ^= 1;
+        return f;
+    };
+    if (a.x_init) {
+        if (on) x = a.x_init[p * a.x_init_stride + i];
+    } else {
+        x = (i == D / 2) ? add(u, 1.0e-3) : u;
+        for (int k = 0; k < 5000; ++k) x = add(x, mul(drift(x), 1.0e-3));
+    }
+    const double sq = on ? sqrt(mul(a.sigma[p * a.sigma_stride + i], a.dt)) : 0.0;
+    if (on) out[i] = x;
+    double zn = (on && N > 1) ? z[1] : 0.0;
+    for (int t = 1; t < N; ++t) {
+        const double zt = zn;
+        if (on && t + 1 < N) zn = z[t + 1];
+        x = add(add(x, mul(drift(x), a.dt)), mul(sq, zt));       // lorenz_96.py:305-307
+        if (on) out[(long long)t * D + i] = x;
+    }
+}
+
 // stochastic_process.py:177-226: obs_y = path[obs_t] + sqrt(R) * xi, xi in (D, M) layout.
 __global__ void __launch_bounds__(128)
 collect_obs_kernel(ObsArgs a)
@@ -139,7 +179,8 @@ collect_obs_kernel(ObsArgs a)
 void launch_trajectories(const TrajArgs& a, cudaStream_t st)
 {
     if (a.B <= 0) return;
-    if (a.D == 40) traj_l96_kernel<<<a.B, 64, 0, st>>>(a);
+    if (a.model == MODEL_L96 && a.D == 40) traj_l96_kernel<<<a.B, 64, 0, st>>>(a);
+    else if (a.model == MODEL_L96) traj_l96d_kernel<<<a.B, 64, 0, st>>>(a);
     else traj_small_kernel<<<(a.B + 31) / 32, 32, 0, st>>>(a);
 }
 

@@ -7,7 +7,8 @@
 //   L96  lorenz_96.py:420-434 (m_bar of ut_approx, utilities.py:239-310; flattened roll :27-32)
 // Per (problem, time index) the integrands go to the pass's dEs scratch, nth + D values each (ft: theta
 // integrand, nth values; fs: Sigma integrand, D values; for D = 1 ft only, dEsde/dSigma = -Esde / sigma): one thread per (problem, t)
-// for D = 1 and D = 3 (below), the HYPER instantiation of the energy kernel for D = 40 (l96_energy.cu).
+// for D = 1 and D = 3 (below), the HYPER instantiation of the energy kernel for Lorenz 96 (l96_energy.cu for
+// D = 40, l96_dyn.cu for the other D).
 // Then one CTA per problem integrates every component with the composite trapezoid
 // (utilities.py:144-201) in an order fixed by N alone and applies the final scalings.
 #include "common.cuh"
@@ -147,7 +148,8 @@ void launch_hyper_terms(const Batch& b, const Scratch& s, const double* x, long 
                         cudaStream_t st)
 {
     if (b.model == MODEL_L96) {
-        launch_l96_hyper(b, s, x, xs, p0, count, st);
+        if (l96_tuned(b.D)) launch_l96_hyper(b, s, x, xs, p0, count, st);
+        else launch_l96d_hyper(b, s, x, xs, p0, count, st);
         return;
     }
     const unsigned bl = (unsigned)(((long long)count * b.N + 127) / 128);

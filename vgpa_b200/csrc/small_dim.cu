@@ -1298,6 +1298,10 @@ void launch_bwd_dense(int method, int D, int N, double dt, const double* A, cons
         launch_bwd_dense_l96(method, N, dt, A, dEm, dEs, jm, js, lam, psi, st);
         return;
     }
+    if (D != 1 && D != 3) {   // Lorenz 96 at any other D
+        launch_bwd_dense_l96d(method, D, N, dt, A, dEm, dEs, jm, js, lam, psi, st);
+        return;
+    }
     Batch b{};
     b.model = (D == 1) ? MODEL_OU : MODEL_L63;
     b.method = method; b.D = D; b.N = N; b.B = 1; b.dt = dt; b.dt_model = dt;

@@ -19,6 +19,7 @@ import numpy as np
 from numpy.random import SeedSequence, default_rng
 
 from . import engine
+from ._lib import L96_DIMS
 
 
 class StochasticProcess(object):
@@ -312,10 +313,10 @@ class Lorenz96(_VectorND):
         StochasticProcess.__init__(self, r_seed, single_dim=False)
         if dim_d < 10:
             raise ValueError(f" {self.__class__.__name__}: Insufficient state vector dimensions: {dim_d}")
-        if dim_d != 40:
-            raise ValueError(f" {self.__class__.__name__}: the CUDA path is built for dim_d = 40"
-                             f" (the only size the reference's Simulation can construct).")
-        self.dim_d = dim_d
+        if dim_d > L96_DIMS[1]:
+            raise ValueError(f" {self.__class__.__name__}: dim_d = {dim_d} is outside the range the CUDA path"
+                             f" supports ({L96_DIMS[0]} <= dim_d <= {L96_DIMS[1]}).")
+        self.dim_d = int(dim_d)
         self._set_sigma(sigma)
         self._theta = np.asarray(theta, dtype=float)
 

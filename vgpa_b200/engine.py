@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import MODELS, METHODS, MODEL_DIM, VgpaDesc, VgpaFullOut, dptr, f64, lib, raise_for
+from ._lib import MODELS, METHODS, MODEL_DIM, VgpaDesc, model_dim, VgpaFullOut, dptr, f64, lib, raise_for
 
 
 def _rows(a, B, n, name):
@@ -33,17 +33,18 @@ class BatchEvaluator:
     :param theta, sigma (D diag), R (D diag), obs_y (M,D), m0 (D), s0 (D,D), E0:
            one value set shared by the batch, or B of them stacked on axis 0
     :param obs_t: (M,) sorted unique observation indices, shared by the batch
+    :param D: state dimension; None = the model's (L96: 40).  L96 takes any 10 <= D <= 64
     """
 
     def __init__(self, model, method, N, dt, theta, sigma, R, obs_t, obs_y, m0, s0, E0,
-                 B=1, dt_model=None, device=0, scratch_bytes=0):
+                 B=1, dt_model=None, device=0, scratch_bytes=0, D=None):
         key = str(model).upper()
         if key not in MODELS:
             raise ValueError(f" Unknown stochastic model -> {key}")
         mkey = str(method).lower()
         if mkey not in METHODS:
             raise ValueError(f" Integration method is unknown -> {method}.")
-        D = MODEL_DIM[key]
+        D = model_dim(key, D)
         self.model, self.method, self.D, self.N, self.B = key, mkey, D, int(N), int(B)
         self.n_x = self.N * D * (D + 1)
         self.device = int(device)
@@ -275,9 +276,9 @@ def model_energy(model, theta, sigma_diag, A, b, m, S, dt_model, device=0, hyper
     """model.energy(A, b, m, S, obs_t) of the reference's StochasticProcess classes.
     Returns Esde, Ef, Edf, dEsde_dm, dEsde_ds (+ dEsde_dtheta, dEsde_dsigma with hyper=True)."""
     key = str(model).upper()
-    D = MODEL_DIM[key]
     b = f64(b)
     N = b.shape[0]
+    D = model_dim(key, (b.size // N) if key == "L96" else None)
     A, m, S = f64(A), f64(m), f64(S)
     th, sg = f64(np.atleast_1d(theta)), f64(np.atleast_1d(sigma_diag))
     if A.size != N * D * D or m.size != N * D or S.size != N * D * D or b.size != N * D or sg.size != D:
@@ -331,9 +332,10 @@ def make_trajectories(model, N, dt, theta, sigma_diag, z, x_init=None, device=0)
     key = str(model).upper()
     if key not in MODELS:
         raise ValueError(f" Unknown stochastic model -> {key}")
-    D = MODEL_DIM[key]
     N = int(N)
     z = f64(z)
+    # L96: D from the draws' (B, D, N) shape (a single path's (D, N) too), 40 when that is ambiguous
+    D = model_dim(key, z.shape[-2] if key == "L96" and z.ndim >= 2 else None)
     if z.size % (N * D) or z.size == 0:
         raise ValueError(f"z: expected B x {D} x {N} values, got {z.size}")
     B = z.size // (N * D)
@@ -342,7 +344,7 @@ def make_trajectories(model, N, dt, theta, sigma_diag, z, x_init=None, device=0)
     sg, sgs = _rows(sigma_diag, B, D, "sigma")
     xi, xis = (None, 0) if x_init is None else _rows(x_init, B, D, "x_init")
     path = np.empty((B, N) if D == 1 else (B, N, D))
-    rc = lib.vgpa_make_trajectory(device, MODELS[key], N, B, float(dt), th.ctypes.data, ths, sg.ctypes.data, sgs,
+    rc = lib.vgpa_make_trajectory_dim(device, MODELS[key], D, N, B, float(dt), th.ctypes.data, ths, sg.ctypes.data, sgs,
                                   None if xi is None else xi.ctypes.data, xis, z.ctypes.data, N * D,
                                   path.ctypes.data, N * D)
     raise_for(rc, None)

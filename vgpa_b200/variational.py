@@ -143,7 +143,7 @@ class VarGP(object):
                 m0=np.atleast_1d(np.asarray(m0, dtype=float)),
                 s0=np.asarray(s0, dtype=float).reshape(D, D),
                 E0=float(np.asarray(self.kl0(m0, s0))),              # constant: variational.py:183-185
-                B=1, dt_model=float(self.dt), device=self._device)
+                B=1, dt_model=float(self.dt), device=self._device, D=D)
         return self._ev_obj
 
     # -- variational.py:73-139 (host-side set-up, not on the per-iteration path) ------
