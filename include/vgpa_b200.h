@@ -77,7 +77,8 @@ typedef struct {
     const double *R;      int64_t R_stride;      /* D: diag of the obs. noise     */
     const int64_t *obs_t;                        /* M sorted unique indices,
                                                     shared by the batch
-                                                    (stochastic_process.py:166-175) */
+                                                    (stochastic_process.py:166-175);
+                                                    vgpa_create_obs_rows: NULL   */
     const double *obs_y;  int64_t obs_y_stride;  /* M x D observation values      */
     const double *m0;     int64_t m0_stride;     /* D                             */
     const double *s0;     int64_t s0_stride;     /* D x D                         */
@@ -89,6 +90,18 @@ typedef struct {
 
 /* VarGP.__init__ (variational.py:15-71): validate, upload, allocate scratch. */
 int vgpa_create(const vgpa_desc *desc, vgpa_handle **out);
+/* Per-problem observation schedules.  Problem p has M[p] observations, at the time indices
+ * obs_t + p * obs_t_stride (sorted, unique, in [0, N)).  Its values are the M[p] x D entries at
+ * desc->obs_y + p * desc->obs_y_stride.  desc->M is the row capacity: M[p] <= desc->M, and each
+ * obs_y row holds desc->M x D entries (obs_y_stride >= desc->M * D, or 0 = one row shared by all).
+ * desc->obs_t must be NULL.  obs_t_stride == 0: one row shared by every problem (the first M[p]
+ * entries are problem p's), else obs_t_stride >= desc->M.  M == NULL: every problem has desc->M
+ * observations.  With both, this is vgpa_create.  Every entry point of the handle uses each
+ * problem's own schedule; vgpa_initialization fails (VGPA_EINVAL, naming the problem) when a
+ * problem has no observation or one at the first or last grid index.  The handle keeps a (B, N)
+ * int32 table of observation ordinals on the device (B * N * 4 bytes). */
+int vgpa_create_obs_rows(const vgpa_desc *desc, const int64_t *obs_t, int64_t obs_t_stride,
+                         const int32_t *M, vgpa_handle **out);
 void vgpa_destroy(vgpa_handle *h);
 /* Text of the last error on this handle (or of the last failed vgpa_create
  * when h is NULL).  Valid until the next call on the handle. */

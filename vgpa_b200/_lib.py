@@ -69,6 +69,8 @@ def _load():
     H = C.c_void_p
     lib.vgpa_create.restype = C.c_int
     lib.vgpa_create.argtypes = [C.POINTER(VgpaDesc), C.POINTER(H)]
+    lib.vgpa_create_obs_rows.restype = C.c_int
+    lib.vgpa_create_obs_rows.argtypes = [C.POINTER(VgpaDesc), C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(H)]
     lib.vgpa_destroy.restype = None
     lib.vgpa_destroy.argtypes = [H]
     lib.vgpa_last_error.restype = C.c_char_p

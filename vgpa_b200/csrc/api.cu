@@ -210,7 +210,9 @@ struct vgpa_handle {
     Batch batch{};
     int chunk = 0;
     long long n_x = 0;   // N * D * (D + 1)
-    DevBuf theta, sigma, R, obs_t, obs_index, obs_y, m0, s0, E0, status;
+    DevBuf theta, sigma, R, obs_t, obs_index, obs_count, obs_y, m0, s0, E0, status;
+    bool obs_rows = false;              // per-problem observation schedules (vgpa_create_obs_rows)
+    int init_empty = -1, init_edge = -1;   // ... the first problem without observations / with one at index 0 or N - 1
     ScratchBufs sc;
     cudaEvent_t ev_done = nullptr;      // end of the last vgpa_eval_device (a call on ANOTHER stream waits for it: one scratch)
     // host-API staging: two slots of one chunk each
@@ -404,10 +406,16 @@ const char* vgpa_version(void) { return "vgpa_b200 0.1 (sm_100a)"; }
 
 const char* vgpa_last_error(const vgpa_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
-int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
+}  // extern "C"
+
+namespace {
+
+// vgpa_create and vgpa_create_obs_rows.  obs_t: the schedules, obs_t_stride elements apart (0 = one row shared by
+// every problem); counts: B observation counts or NULL (desc->M each).  rows == false: vgpa_create's one schedule,
+// desc->obs_t.
+int create_handle(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride, const int32_t* counts, bool rows,
+                  vgpa_handle** out)
 {
-    if (out) *out = nullptr;
-    if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create: NULL argument");
     vgpa_handle* h = new vgpa_handle();
     h->d = *d;
     auto bail = [&](int rc) {
@@ -431,12 +439,33 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
     if (d->M < 0 || d->B < 1) return bail(h->fail(VGPA_EINVAL, "Wrong sizes M=%d B=%d", d->M, d->B));
     if (!(d->dt > 0.0) || !(d->dt_model > 0.0))
         return bail(h->fail(VGPA_EINVAL, "Discrete time step should be strictly positive -> %g", d->dt));
-    if (d->M > 0 && d->obs_t == nullptr) return bail(h->fail(VGPA_EINVAL, "obs_t is NULL"));
-    for (int n = 0; n < d->M; ++n) {
-        if (d->obs_t[n] < 0 || d->obs_t[n] >= d->N || (n > 0 && d->obs_t[n] <= d->obs_t[n - 1]))
-            return bail(h->fail(VGPA_EINVAL, "obs_t must be sorted unique indices in [0, N)"));
-        // gaussian_like.py:137-146 indexes the covariance by the observation ordinal n
-        if (n >= d->N) return bail(h->fail(VGPA_EINVAL, "more observations than time points"));
+    if (!rows) {
+        if (d->M > 0 && d->obs_t == nullptr) return bail(h->fail(VGPA_EINVAL, "obs_t is NULL"));
+        for (int n = 0; n < d->M; ++n) {
+            if (d->obs_t[n] < 0 || d->obs_t[n] >= d->N || (n > 0 && d->obs_t[n] <= d->obs_t[n - 1]))
+                return bail(h->fail(VGPA_EINVAL, "obs_t must be sorted unique indices in [0, N)"));
+            // gaussian_like.py:137-146 indexes the covariance by the observation ordinal n
+            if (n >= d->N) return bail(h->fail(VGPA_EINVAL, "more observations than time points"));
+        }
+    } else {
+        if (d->obs_t != nullptr)
+            return bail(h->fail(VGPA_EINVAL, "desc->obs_t must be NULL: the schedules are the obs_t argument"));
+        if (d->M > 0 && obs_t == nullptr) return bail(h->fail(VGPA_EINVAL, "obs_t is NULL"));
+        if (obs_t_stride < 0 || (obs_t_stride > 0 && obs_t_stride < d->M))
+            return bail(h->fail(VGPA_EINVAL, "obs_t_stride %lld: 0 (one shared row) or at least M = %d", (long long)obs_t_stride,
+                                d->M));
+        for (int p = 0; p < d->B; ++p) {
+            const int Mp = counts ? counts[p] : d->M;
+            if (Mp < 0 || Mp > d->M)
+                return bail(h->fail(VGPA_EINVAL, "M of problem %d is %d, outside [0, desc->M = %d]", p, Mp, d->M));
+            const int64_t* ot = obs_t + p * obs_t_stride;
+            for (int n = 0; n < Mp; ++n)
+                if (ot[n] < 0 || ot[n] >= d->N || (n > 0 && ot[n] <= ot[n - 1]))
+                    return bail(h->fail(VGPA_EINVAL, "obs_t of problem %d must be sorted unique indices in [0, N)", p));
+            // VarGP.initialization's spline (variational.py:86-104) needs knots strictly inside the time window
+            if (h->init_empty < 0 && Mp < 1) h->init_empty = p;
+            if (h->init_edge < 0 && Mp > 0 && (ot[0] == 0 || ot[Mp - 1] == d->N - 1)) h->init_edge = p;
+        }
     }
     {
         const long long cnt = (d->sigma_stride == 0) ? 1 : d->B;
@@ -489,7 +518,7 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
         b.obs_y_stride = 0;
     }
 #undef UP
-    {
+    if (!rows) {
         std::vector<long long> ot(std::max(M, 1), 0);
         std::vector<int> oi(N, -1);
         for (int n = 0; n < M; ++n) {
@@ -502,6 +531,30 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
         if (e != cudaSuccess) return bail(h->cuda_fail(e, "upload(obs_t)"));
         b.obs_t = h->obs_t.as<long long>();
         b.obs_index = h->obs_index.as<int>();
+    } else {
+        // (B, max(M, 1)) index rows, the (B, N) ordinal table the backward sweeps read at every step, B counts
+        const long long Mc = std::max(M, 1);
+        std::vector<long long> ot((size_t)B * Mc, 0);
+        std::vector<int> oi((size_t)B * N, -1), cnt(B);
+        for (int p = 0; p < B; ++p) {
+            cnt[p] = counts ? counts[p] : M;
+            const int64_t* src = obs_t + p * obs_t_stride;
+            for (int n = 0; n < cnt[p]; ++n) {
+                ot[(size_t)p * Mc + n] = src[n];
+                oi[(size_t)p * N + src[n]] = n;
+            }
+        }
+        cudaError_t e = cudaSuccess;
+        upload(e, h->obs_t, ot.data(), ot.size());
+        upload(e, h->obs_index, oi.data(), oi.size());
+        upload(e, h->obs_count, cnt.data(), cnt.size());
+        if (e != cudaSuccess) return bail(h->cuda_fail(e, "upload(obs_t)"));
+        b.obs_t = h->obs_t.as<long long>();
+        b.obs_index = h->obs_index.as<int>();
+        b.obs_count = h->obs_count.as<int>();
+        b.obs_t_stride = Mc;
+        b.obs_index_stride = N;
+        h->obs_rows = true;
     }
     // ---- scratch: trajectories for one chunk of problems ----
     const long long per = 8LL * N * (2LL * D + 2LL * D * D + 1);
@@ -550,6 +603,30 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
     }
     *out = h;
     return VGPA_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
+{
+    if (out) *out = nullptr;
+    if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create: NULL argument");
+    return create_handle(d, nullptr, 0, nullptr, false, out);
+}
+
+int vgpa_create_obs_rows(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride, const int32_t* M,
+                         vgpa_handle** out)
+{
+    if (out) *out = nullptr;
+    if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create_obs_rows: NULL argument");
+    if (obs_t_stride == 0 && M == nullptr && d->obs_t == nullptr) {   // one shared schedule: exactly vgpa_create
+        vgpa_desc one = *d;
+        one.obs_t = obs_t;
+        return create_handle(&one, nullptr, 0, nullptr, false, out);
+    }
+    return create_handle(d, obs_t, obs_t_stride, M, true, out);
 }
 
 void vgpa_destroy(vgpa_handle* h)
@@ -1054,6 +1131,11 @@ static int init_check(vgpa_handle* h, const double* x, int64_t x_stride)
     if (x == nullptr) return h->fail(VGPA_EINVAL, "x is NULL");
     if (x_stride < h->n_x) return h->fail(VGPA_EINVAL, "x_stride %lld < %lld", (long long)x_stride, h->n_x);
     if (h->d.M < 1) return h->fail(VGPA_EINVAL, "initialization needs at least one observation");
+    if (h->init_empty >= 0)
+        return h->fail(VGPA_EINVAL, "initialization needs at least one observation: problem %d has none", h->init_empty);
+    if (h->init_edge >= 0)
+        return h->fail(VGPA_EINVAL, "`x` must be strictly increasing sequence: an observation of problem %d sits at the first "
+                                    "or last grid index", h->init_edge);
     return VGPA_OK;
 }
 

@@ -48,10 +48,27 @@ struct Batch {
     const int* plist;         // or null.  Compacted launches of the Lorenz-96 kernels (vgpa_set_active_list): the
                               // pass covers list positions [p0, p0 + count) and the problem at position k is
                               // plist[k], so that a thinned-out ensemble still fills whole waves
+    // Per-problem observation schedules (vgpa_create_obs_rows).  Problem p observes at obs_t + p * obs_t_stride, its
+    // grid table is obs_index + p * obs_index_stride (a (B, N) table), and it has obs_count[p] observations.  A handle
+    // of vgpa_create has both strides 0 and a null count: one schedule of M observations for the batch.
+    long long obs_t_stride;
+    long long obs_index_stride;
+    const int* obs_count;     // B counts <= M, or null = M each
+    long long pad_;           // keeps the fields added with the schedules at 32 bytes: the kernel parameters that follow
+                              // a Batch keep their 16-byte alignment, and the D = 40 kernels their code (and speed)
 };
 
 // problem served by launch position `pos` (= p0 + local index)
 __device__ __forceinline__ int problem_at(const Batch& b, int pos) { return b.plist != nullptr ? b.plist[pos] : pos; }
+
+// The observation schedule of problem p: sorted time indices, the ordinal of the observation at each grid index (or
+// -1), and the number of observations.
+__device__ __forceinline__ const long long* obs_t_of(const Batch& b, int p) { return b.obs_t + p * b.obs_t_stride; }
+__device__ __forceinline__ const int* obs_index_of(const Batch& b, int p) { return b.obs_index + p * b.obs_index_stride; }
+__device__ __forceinline__ int obs_count_of(const Batch& b, int p) { return b.obs_count != nullptr ? b.obs_count[p] : b.M; }
+// Launchers of the kernels that sit at the edge of the instruction cache (the D = 40 backward sweep) instantiate them
+// twice: ROWS = false reads the one shared schedule exactly as before per-problem schedules existed.
+inline bool obs_rows(const Batch& b) { return b.obs_index_stride != 0; }
 
 // Sum over the CTA in a fixed order (every thread gets it); sh: blockDim.x doubles, blockDim.x a power of two.
 __device__ __forceinline__ double block_sum(double v, double* sh)
@@ -197,7 +214,8 @@ void launch_bwd_dense(int method, int D, int N, double dt, const double* A, cons
                       const double* dEs, const double* jm, const double* js, double* lam,
                       double* psi, cudaStream_t st);
 
-// VarGP.initialization for problems p0 .. p0 + count - 1 (init.cu); scratch: count * D * 2 (M + 2) doubles.
+// VarGP.initialization for problems p0 .. p0 + count - 1 (init.cu); scratch: count * D * 2 (M + 2) doubles, M the
+// handle's row capacity (problem p uses obs_count_of(b, p) + 2 knots of its slot).
 void launch_initialization(const Batch& b, int p0, int count, double t0, double* scratch, double* x,
                            long long x_stride, int* err, cudaStream_t st);
 

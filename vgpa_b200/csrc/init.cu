@@ -10,7 +10,8 @@
 // Knots: time_x = [tw[0], tw[obs_t], tw[-1]], values [y_first, y, y_last] (variational.py:86-104);
 // tw[k] = t0 + k dt_model.
 //   kernel 1: one thread per (problem, dimension) solves for the knot derivatives (Thomas
-//             algorithm; scratch in global memory: 2 (M + 2) doubles per pair)
+//             algorithm; scratch in global memory: 2 (M + 2) doubles per pair, M the handle's row capacity;
+//             each problem has its own M[p] + 2 knots)
 //   kernel 2: one thread per (problem, time index, dimension) evaluates the spline at tw[k] and
 //             tw[k+1], forms b0 and the diagonal entry of A0 (the zeros of A0 come from a memset)
 #include "common.cuh"
@@ -18,17 +19,28 @@
 namespace vgpa {
 namespace {
 
-__device__ __forceinline__ double knot_x(const Batch& b, double t0, int j)
+// The knots of one problem: its n = M + 2 time points and the observations they take their values from
+struct Knots {
+    const long long* ot;   // the problem's M observation indices
+    const double* oy;      // its M x D observation values
+    int M, n;
+};
+__device__ __forceinline__ Knots knots_of(const Batch& b, int p)
 {
-    const int n = b.M + 2;
-    const long long idx = (j == 0) ? 0 : (j == n - 1 ? (long long)(b.N - 1) : b.obs_t[j - 1]);
+    const int M = obs_count_of(b, p);
+    return Knots{obs_t_of(b, p), b.obs_y + p * b.obs_y_stride, M, M + 2};
+}
+__device__ __forceinline__ double knot_x(const Batch& b, const Knots& kn, double t0, int j)
+{
+    const int n = kn.n;
+    const long long idx = (j == 0) ? 0 : (j == n - 1 ? (long long)(b.N - 1) : kn.ot[j - 1]);
     return t0 + (double)idx * b.dt_model;
 }
-__device__ __forceinline__ double knot_y(const Batch& b, const double* oy, int d, int j)
+__device__ __forceinline__ double knot_y(const Batch& b, const Knots& kn, int d, int j)
 {
-    const int n = b.M + 2;
-    const int o = (j == 0) ? 0 : (j == n - 1 ? b.M - 1 : j - 1);
-    return oy[(long long)o * b.D + d];
+    const int n = kn.n;
+    const int o = (j == 0) ? 0 : (j == n - 1 ? kn.M - 1 : j - 1);
+    return kn.oy[(long long)o * b.D + d];
 }
 
 __global__ void __launch_bounds__(128)
@@ -36,17 +48,18 @@ init_slopes_kernel(Batch b, int p0, int count, double t0, double* __restrict__ s
 {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     if (pair >= count * b.D) return;
-    const int lp = pair / b.D, d = pair - lp * b.D, p = p0 + lp, n = b.M + 2;
-    const double* oy = b.obs_y + p * b.obs_y_stride;
-    double* s = scratch + (long long)pair * 2 * n;
+    const int lp = pair / b.D, d = pair - lp * b.D, p = p0 + lp;
+    const Knots kn = knots_of(b, p);
+    const int n = kn.n;
+    double* s = scratch + (long long)pair * 2 * (b.M + 2);   // slots of the handle's capacity
     double* cp = s + n;
     for (int i = 0; i + 1 < n; ++i)
-        if (!(knot_x(b, t0, i + 1) > knot_x(b, t0, i))) {   // scipy: x must be strictly increasing
+        if (!(knot_x(b, kn, t0, i + 1) > knot_x(b, kn, t0, i))) {   // scipy: x must be strictly increasing
             atomicExch(err, 1);
             return;
         }
-    auto X = [&](int j) { return knot_x(b, t0, j); };
-    auto Y = [&](int j) { return knot_y(b, oy, d, j); };
+    auto X = [&](int j) { return knot_x(b, kn, t0, j); };
+    auto Y = [&](int j) { return knot_y(b, kn, d, j); };
     if (n == 2) {
         s[0] = s[1] = (Y(1) - Y(0)) / (X(1) - X(0));
         return;
@@ -82,20 +95,19 @@ init_slopes_kernel(Batch b, int p0, int count, double t0, double* __restrict__ s
     for (int i = n - 2; i >= 0; --i) s[i] -= cp[i] * s[i + 1];
 }
 
-__device__ __forceinline__ double spline_at(const Batch& b, const double* oy, const double* s, int d,
-                                            double t0, int k)
+__device__ __forceinline__ double spline_at(const Batch& b, const Knots& kn, const double* s, int d, double t0, int k)
 {
-    const int n = b.M + 2;
+    const int n = kn.n;
     // interval i: x[i] <= tw[k] < x[i+1], i.e. i = #{ observation indices <= k } (last interval closed)
-    int lo = 0, hi = b.M;
+    int lo = 0, hi = kn.M;
     while (lo < hi) {
         const int mid = (lo + hi) >> 1;
-        if (b.obs_t[mid] <= k) lo = mid + 1; else hi = mid;
+        if (kn.ot[mid] <= k) lo = mid + 1; else hi = mid;
     }
     int i = lo;
     if (i > n - 2) i = n - 2;
-    const double xi = knot_x(b, t0, i), xj = knot_x(b, t0, i + 1);
-    const double yi = knot_y(b, oy, d, i), yj = knot_y(b, oy, d, i + 1);
+    const double xi = knot_x(b, kn, t0, i), xj = knot_x(b, kn, t0, i + 1);
+    const double yi = knot_y(b, kn, d, i), yj = knot_y(b, kn, d, i + 1);
     const double h = xj - xi, slope = (yj - yi) / h;
     const double tt = (s[i] + s[i + 1] - 2 * slope) / h;
     const double c0 = tt / h, c1 = (slope - s[i]) / h - tt;
@@ -108,16 +120,16 @@ init_x0_kernel(Batch b, int p0, int count, double t0, const double* __restrict__
                long long xs)
 {
     const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int D = b.D, N = b.N, n = b.M + 2;
+    const int D = b.D, N = b.N;
     if (gid >= (long long)count * N * D) return;
     const int d = (int)(gid % D);
     const long long r = gid / D;
     const int k = (int)(r % N), lp = (int)(r / N), p = p0 + lp;
-    const double* oy = b.obs_y + p * b.obs_y_stride;
-    const double* s = scratch + ((long long)lp * D + d) * 2 * n;
+    const Knots kn = knots_of(b, p);
+    const double* s = scratch + ((long long)lp * D + d) * 2 * (b.M + 2);
     double* xo = x + (long long)p * xs;
     const double ad = 0.5 * (b.sigma[p * b.sigma_stride + d] / 0.25);      // variational.py:95 / :122-126
-    const double m0 = spline_at(b, oy, s, d, t0, k);
+    const double m0 = spline_at(b, kn, s, d, t0, k);
     if (D == 1) {
         xo[k] = ad;
         xo[N + k] = m0;                                                     // :101
@@ -125,7 +137,7 @@ init_x0_kernel(Batch b, int p0, int count, double t0, const double* __restrict__
     }
     xo[((long long)k * D + d) * D + d] = ad;           // the rest of A0 was zero-filled by the launcher
     double bk = ad * m0;                                                    // :133 at the last index
-    if (k < N - 1) bk += (spline_at(b, oy, s, d, t0, k + 1) - m0) / b.dt_model;  // :121, :127 (self.dt = model.time_step, :57)
+    if (k < N - 1) bk += (spline_at(b, kn, s, d, t0, k + 1) - m0) / b.dt_model;  // :121, :127 (self.dt = model.time_step, :57)
     xo[(long long)N * D * D + (long long)k * D + d] = bk;
 }
 

@@ -236,6 +236,7 @@ l63_bwd_lanes_kernel(Batch b, Scratch s, const double* __restrict__ x, long long
     const double* dEs = s.dEs + (long long)lp * N * DD;
     const double* th = b.theta + p * b.theta_stride;
     const double* oy = b.obs_y + p * b.obs_y_stride;
+    const int* oidx = obs_index_of(b, p);
     const double vS = th[0], vR = th[1], vB = th[2];
     const double isg_i = 1.0 / b.sigma[p * b.sigma_stride + i];
     const double Rv_i = b.R[p * b.R_stride + i];
@@ -314,7 +315,7 @@ l63_bwd_lanes_kernel(Batch b, Scratch s, const double* __restrict__ x, long long
             // jump at index t-1 (gaussian_like.py:188,191 / :235,238); H = I, R diagonal
             double jmv = 0.0, jsv = 0.0;
             {
-                const int no = b.obs_index[t - 1];
+                const int no = oidx[t - 1];
                 if (no >= 0) {
                     jmv = -(oy[(long long)no * D + i] - sm[up * D + i]) / Rv_i;
                     jsv = 0.5 / Rv_i;

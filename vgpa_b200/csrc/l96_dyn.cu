@@ -401,6 +401,7 @@ l96d_bwd_kernel(Batch b, DynBwdArgs a, int p0)
     const bool dense = a.jm_dense != nullptr;
     const bool keep = a.lam_out != nullptr && lp == 0;
     const double* oy = dense ? nullptr : b.obs_y + p * b.obs_y_stride;
+    const int* oidx = dense ? nullptr : obs_index_of(b, p);
     const double dt = b.dt, dtm = b.dt_model;
     const double theta = (b.theta != nullptr) ? b.theta[p * b.theta_stride] : 0.0;
 
@@ -471,7 +472,7 @@ l96d_bwd_kernel(Batch b, DynBwdArgs a, int p0)
             }
             __syncthreads();   // Q complete
             const double wt = ksum_w(METHOD, sidx), cdt = next_coef(METHOD, sidx) * dt;
-            const int n_obs = dense ? -1 : b.obs_index[t - 1];
+            const int n_obs = dense ? -1 : oidx[t - 1];
 #pragma unroll
             for (int r = 0; r < EPT; ++r) {
                 const int e = tid + r * NTH;

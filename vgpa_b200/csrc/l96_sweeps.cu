@@ -415,7 +415,8 @@ __device__ __forceinline__ void mma_rowx(const double (&Xc)[5][2], const double 
     yv = y;
 }
 
-template <int METHOD>
+// ROWS: per-problem observation schedules (obs_rows); ROWS = false is the shared-schedule kernel, unchanged
+template <int METHOD, bool ROWS>
 __global__ void __launch_bounds__(NTH, 3)
 l96_bwd_kernel(Batch b, BwdArgs a, int p0)
 {
@@ -665,7 +666,7 @@ l96_bwd_kernel(Batch b, BwdArgs a, int p0)
             parA[nxt] ^= 1u;
         }
         // ---- final combination + jump at index t-1 -----------------------------------
-        const int n_obs = dense ? -1 : b.obs_index[t - 1];
+        const int n_obs = dense ? -1 : (ROWS ? obs_index_of(b, p)[t - 1] : b.obs_index[t - 1]);
         {
             const int i = irow;
 #pragma unroll
@@ -711,8 +712,13 @@ static void bwd_launch(const Batch& b, const BwdArgs& a, int p0, int count, cuda
 {
     const size_t sh = sizeof(BwdSmem);
     with_method(b.method, [&](auto m) {
-        set_smem(l96_bwd_kernel<m>, sh);
-        l96_bwd_kernel<m><<<count, NTH, sh, st>>>(b, a, p0);
+        if (obs_rows(b)) {
+            set_smem(l96_bwd_kernel<m, true>, sh);
+            l96_bwd_kernel<m, true><<<count, NTH, sh, st>>>(b, a, p0);
+        } else {
+            set_smem(l96_bwd_kernel<m, false>, sh);
+            l96_bwd_kernel<m, false><<<count, NTH, sh, st>>>(b, a, p0);
+        }
     });
 }
 

@@ -731,6 +731,7 @@ small_bwd_kernel(Batch b, Scratch s, SmallBwdArgs a, int p0, int count, Extra ex
     const double* dEs = s.dEs + (long long)lp * N * DD;
     const double* th = dense ? nullptr : b.theta + p * b.theta_stride;
     const double* oy = dense ? nullptr : b.obs_y + p * b.obs_y_stride;
+    const int* oidx = dense ? nullptr : obs_index_of(b, p);
     double isg[D], Rv[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) {
@@ -802,7 +803,7 @@ small_bwd_kernel(Batch b, Scratch s, SmallBwdArgs a, int p0, int count, Extra ex
         if (t == 0) break;
         // jump at index t-1 (gaussian_like.py:188,191 / :235,238); H = I, R diagonal
         double jm[D], js[D];
-        const int n = dense ? -1 : b.obs_index[t - 1];
+        const int n = dense ? -1 : oidx[t - 1];
 #pragma unroll
         for (int i = 0; i < D; ++i) {
             jm[i] = dense ? a.jm_dense[(long long)(t - 1) * D + i] : 0.0;
@@ -857,7 +858,8 @@ __device__ __forceinline__ double free_energy_of(const Batch& b, int p, const do
 {
     constexpr int W = ESDE_THREADS;
     const int tid = threadIdx.x;
-    const int D = b.D, M = b.M, DD = D * D;
+    const int D = b.D, M = obs_count_of(b, p), DD = D * D;
+    const long long* ot = obs_t_of(b, p);
     const double Esde = esde_of(b, p, f, sh);
     double acc;
     // observation energy
@@ -868,7 +870,7 @@ __device__ __forceinline__ double free_energy_of(const Batch& b, int p, const do
     if (D == 1) {  // gaussian_like.py:69-96
         acc = 0.0;
         for (int n = tid; n < (tid < W ? M : 0); n += W) {
-            const long long t = b.obs_t[n];
+            const long long t = ot[n];
             const double y = oy[n], E2 = mt[t] * mt[t] + st[t];
             acc += (y * y) - 2.0 * y * mt[t] + E2;
         }
@@ -878,7 +880,7 @@ __device__ __forceinline__ double free_energy_of(const Batch& b, int p, const do
         acc = 0.0;
         for (int q = tid; q < (tid < W ? M * D : 0); q += W) {
             const int n = q / D, i = q % D;
-            const long long t = b.obs_t[n];
+            const long long t = ot[n];
             const double z = (oy[(long long)n * D + i] - mt[t * D + i]) / sqrt(R[i]);
             acc += z * z + (1.0 / R[i]) * st[(long long)n * DD + (long long)i * D + i];
         }
@@ -1059,6 +1061,7 @@ __device__ __forceinline__ void scan1_bwd_body(const Batch& b, int p, const doub
     const int tid = threadIdx.x, N = b.N;
     const double* th = b.theta + p * b.theta_stride;
     const double* oy = b.obs_y + p * b.obs_y_stride;
+    const int* oidx = obs_index_of(b, p);
     const double isg = 1.0 / b.sigma[p * b.sigma_stride], Rv = b.R[p * b.R_stride];
     const double dt = b.dt, dtm = b.dt_model;
     // step q = 0 .. N-2 takes index t = N-1-q to t-1
@@ -1068,7 +1071,7 @@ __device__ __forceinline__ void scan1_bwd_body(const Batch& b, int p, const doub
 
     // jump of lambda and Psi at index t (gaussian_like.py:188,191), as in small_bwd_kernel
     auto jump = [&](int t, double& jm, double& js) {
-        const int n = b.obs_index[t];
+        const int n = oidx[t];
         jm = 0.0;
         js = 0.0;
         if (n >= 0) {

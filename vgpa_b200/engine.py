@@ -25,6 +25,40 @@ def _rows(a, B, n, name):
     raise ValueError(f"{name}: expected {n} or {B}x{n} values, got {a.size}")
 
 
+def _is_schedule_list(obs_t):
+    """True for per-problem schedules: a list or tuple whose entries are index arrays (not ints)."""
+    return isinstance(obs_t, (list, tuple)) and len(obs_t) > 0 and any(np.ndim(o) > 0 for o in obs_t)
+
+
+def _schedule_rows(obs_t, obs_y, B, D):
+    """Per-problem schedules: B index arrays and B (M_p, D) value arrays ((M_p,) too for D = 1), padded to the
+    largest M_p.  Returns the (B, max(M, 1)) int64 index rows, the (B, M, D) values, the B counts and M."""
+    if len(obs_t) != B:
+        raise ValueError(f"obs_t: expected {B} per-problem index arrays, got {len(obs_t)}")
+    if not isinstance(obs_y, (list, tuple)) or len(obs_y) != B:
+        raise ValueError(f"obs_y: per-problem obs_t needs a matching sequence of {B} (M_p, D) arrays")
+    ts, ys = [], []
+    for p, (t, y) in enumerate(zip(obs_t, obs_y)):
+        t = np.asarray(t)
+        if t.ndim != 1 or (t.size and not np.issubdtype(t.dtype, np.integer)):
+            raise ValueError(f"obs_t of problem {p}: expected a 1-D array of integer indices, got shape {t.shape}")
+        y = np.asarray(y, dtype=np.float64)
+        if D == 1 and y.ndim == 1:
+            y = y.reshape(-1, 1)
+        if y.shape != (t.size, D):
+            raise ValueError(f"obs_y of problem {p}: expected shape ({t.size}, {D}), got {y.shape}")
+        ts.append(t.astype(np.int64))
+        ys.append(y)
+    counts = np.array([t.size for t in ts], dtype=np.int32)
+    M = int(counts.max())
+    rows = np.zeros((B, max(M, 1)), dtype=np.int64)
+    vals = np.zeros((B, M, D))
+    for p, (t, y) in enumerate(zip(ts, ys)):
+        rows[p, :t.size] = t
+        vals[p, :t.size] = y
+    return rows, vals, counts, M
+
+
 class BatchEvaluator:
     """
     :param model:  "DW" | "OU" | "L63" | "L96"   (simulation.py:20)
@@ -32,7 +66,12 @@ class BatchEvaluator:
     :param N: number of time-grid points; dt: sweep step; dt_model: model.time_step
     :param theta, sigma (D diag), R (D diag), obs_y (M,D), m0 (D), s0 (D,D), E0:
            one value set shared by the batch, or B of them stacked on axis 0
-    :param obs_t: (M,) sorted unique observation indices, shared by the batch
+    :param obs_t: (M,) sorted unique observation indices, shared by the batch; or a list of B such index arrays,
+           one schedule per problem (their counts may differ, 0 included), with obs_y a matching list of B
+           (M_p, D) arrays ((M_p,) accepted for D = 1).  A list or tuple is read as per-problem schedules as soon
+           as one entry is not a scalar: a nested list such as [[3, 6]] is one schedule per problem (here B = 1),
+           not a flattened shared schedule, and needs obs_y as a list too.  A flat list or any numpy array keeps
+           the shared meaning.
     :param D: state dimension; None = the model's (L96: 40).  L96 takes any 10 <= D <= 64
     """
 
@@ -48,10 +87,15 @@ class BatchEvaluator:
         self.model, self.method, self.D, self.N, self.B = key, mkey, D, int(N), int(B)
         self.n_x = self.N * D * (D + 1)
         self.device = int(device)
-        obs_t = np.ascontiguousarray(np.asarray(obs_t, dtype=np.int64).ravel())
-        M = obs_t.size
-        nth = 3 if key == "L63" else 1
         keep = {}
+        rows = _is_schedule_list(obs_t)
+        if rows:
+            obs_t, obs_y, counts, M = _schedule_rows(obs_t, obs_y, self.B, D)
+            keep["counts"] = counts
+        else:
+            obs_t = np.ascontiguousarray(np.asarray(obs_t, dtype=np.int64).ravel())
+            M = obs_t.size
+        nth = 3 if key == "L63" else 1
         d = VgpaDesc()
         d.model, d.method, d.D, d.N, d.M, d.B = MODELS[key], METHODS[mkey], D, self.N, M, self.B
         d.device = self.device
@@ -66,10 +110,14 @@ class BatchEvaluator:
             setattr(d, name, dptr(arr))
             setattr(d, name + "_stride", stride)
         keep["obs_t"] = obs_t
-        d.obs_t = obs_t.ctypes.data_as(C.POINTER(C.c_int64))
         d.scratch_bytes = int(scratch_bytes)
         self._h = C.c_void_p()
-        rc = lib.vgpa_create(C.byref(d), C.byref(self._h))
+        if rows:   # every problem its own schedule, padded to M rows
+            rc = lib.vgpa_create_obs_rows(C.byref(d), obs_t.ctypes.data, obs_t.shape[1], counts.ctypes.data,
+                                          C.byref(self._h))
+        else:
+            d.obs_t = obs_t.ctypes.data_as(C.POINTER(C.c_int64))
+            rc = lib.vgpa_create(C.byref(d), C.byref(self._h))
         raise_for(rc, None)
         self._keep = keep
 
