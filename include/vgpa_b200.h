@@ -14,9 +14,12 @@
  *
  * D = 1 (DW, OU) uses the same layout with 1x1 matrices.
  *
- * Scope: diagonal system noise Sigma, diagonal observation noise R, identity
- * observation operator -- everything the sim_params JSON schema can express
- * (vgpa_main.py:38-40, simulation.py:107-176).  L96 takes any 10 <= D <= 64
+ * Scope: diagonal system noise Sigma, diagonal observation noise R, and an
+ * observation operator H that selects components: the identity, or per problem
+ * any non-empty subset of the state components (vgpa_create_observed; the
+ * sim_params JSON's Observations.operator, simulation.py:107-176).  That is
+ * everything the sim_params JSON schema can express (vgpa_main.py:38-40).  A
+ * general H and a non-diagonal R are out of scope.  L96 takes any 10 <= D <= 64
  * (lorenz_96.py:104-140 accepts dim_d >= 10): D = 40, the only size simulation.py:20,134
  * constructs, runs hand-tuned kernels, every other D a run-time-D kernel family.
  *
@@ -102,6 +105,20 @@ int vgpa_create(const vgpa_desc *desc, vgpa_handle **out);
  * int32 table of observation ordinals on the device (B * N * 4 bytes). */
 int vgpa_create_obs_rows(const vgpa_desc *desc, const int64_t *obs_t, int64_t obs_t_stride,
                          const int32_t *M, vgpa_handle **out);
+/* Partially observed problems.  Bit i of observed[p * observed_stride] set: component i of problem p
+ * is observed (D <= 64, so one word holds a mask).  observed_stride == 0: one mask shared by the batch.
+ * observed == NULL: exactly vgpa_create_obs_rows; the first four arguments follow its rules.
+ * Problem p observes the set O_p: H is the rows of the identity at O_p and R is diagonal over O_p, so
+ *   Eobs = 1/2 [ sum_n sum_{i in O} ((y_ni - m_i(t_n))^2 / R_i + S_ii[n] / R_i) + M (D_o log 2pi + sum_{i in O} log R_i) ]
+ * (S indexed by the observation ordinal n, as for H = I), the jumps at t_n are -(y_ni - m_i) / R_i and
+ * 1/2 / R_i for i in O and 0 otherwise, and vgpa_initialization gives an unobserved component the
+ * constant mean path m0[p][i] (b0(t)_i = a_ii m0_i) in place of the spline.  obs_y keeps its M x D rows and
+ * R its D values: the entries of unobserved components are never read (NaN allowed).  Every entry point
+ * of the handle follows the masks.  With every bit below D set, a handle computes what
+ * vgpa_create_obs_rows's does, bit for bit.  VGPA_EINVAL, naming the problem, before any CUDA call: a
+ * mask with no bit set, a bit at or above D, a negative observed_stride. */
+int vgpa_create_observed(const vgpa_desc *desc, const int64_t *obs_t, int64_t obs_t_stride, const int32_t *M,
+                         const uint64_t *observed, int64_t observed_stride, vgpa_handle **out);
 void vgpa_destroy(vgpa_handle *h);
 /* Text of the last error on this handle (or of the last failed vgpa_create
  * when h is NULL).  Valid until the next call on the handle. */
@@ -216,6 +233,15 @@ int vgpa_obs_energy(int device, int D, int N, int M, const int64_t *obs_t, const
                     double *dEobs_dm, double *dEobs_ds, double *dEobs_dr);
 /* dEobs_dr (may be NULL): third output of GaussianLikelihood.gradients -- N values for D = 1
  * (gaussian_like.py:194), N x M x M zeros for D > 1 (the reference never fills it, :226). */
+/* The same likelihood for a component-selecting operator: `observed` holds the observed components (bit i =
+ * component i; vgpa_create_observed gives the formulas).  obs_y is M x D and R has D values; the entries of
+ * unobserved components are not read.  jm (N,D) and js (N,D,D) are the jump tables dEobs_dm, dEobs_ds,
+ * zero except at obs_t and at observed components.  With every
+ * bit below D set, the outputs are those of vgpa_obs_energy, bit for bit.  VGPA_EINVAL for a mask with no
+ * bit set or a bit at or above D. */
+int vgpa_obs_energy_observed(int device, int D, int N, int M, const int64_t *obs_t, const double *obs_y,
+                             const double *R, uint64_t observed, const double *mt, const double *st,
+                             double *Eobs, double *jm, double *js);
 
 /* VarGP.initialization (variational.py:73-139) for every problem of the handle: the starting
  * point x0 = [A0 | b0] from cubic splines (scipy CubicSpline, not-a-knot) through each problem's

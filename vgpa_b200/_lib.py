@@ -71,6 +71,9 @@ def _load():
     lib.vgpa_create.argtypes = [C.POINTER(VgpaDesc), C.POINTER(H)]
     lib.vgpa_create_obs_rows.restype = C.c_int
     lib.vgpa_create_obs_rows.argtypes = [C.POINTER(VgpaDesc), C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(H)]
+    lib.vgpa_create_observed.restype = C.c_int
+    lib.vgpa_create_observed.argtypes = [C.POINTER(VgpaDesc), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                         C.POINTER(H)]
     lib.vgpa_destroy.restype = None
     lib.vgpa_destroy.argtypes = [H]
     lib.vgpa_last_error.restype = C.c_char_p
@@ -103,6 +106,8 @@ def _load():
     lib.vgpa_model_energy.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double] + [_dp] * 13
     lib.vgpa_obs_energy.restype = C.c_int
     lib.vgpa_obs_energy.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, _ip] + [_dp] * 8
+    lib.vgpa_obs_energy_observed.restype = C.c_int
+    lib.vgpa_obs_energy_observed.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, C.c_uint64] + [_dp] * 5
     i64 = C.c_int64
     traj = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double] + [C.c_void_p, i64] * 5
     obs = [C.c_int] * 5 + [C.c_void_p] + [C.c_void_p, i64] * 4

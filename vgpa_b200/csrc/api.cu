@@ -3,6 +3,7 @@
 // sweep fused with the gradient), the batched hyper-parameter gradients, host staging
 // with copy/compute overlap.
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -210,7 +211,7 @@ struct vgpa_handle {
     Batch batch{};
     int chunk = 0;
     long long n_x = 0;   // N * D * (D + 1)
-    DevBuf theta, sigma, R, obs_t, obs_index, obs_count, obs_y, m0, s0, E0, status;
+    DevBuf theta, sigma, R, obs_t, obs_index, obs_count, obs_y, m0, s0, E0, observed, status;
     bool obs_rows = false;              // per-problem observation schedules (vgpa_create_obs_rows)
     int init_empty = -1, init_edge = -1;   // ... the first problem without observations / with one at index 0 or N - 1
     ScratchBufs sc;
@@ -410,11 +411,12 @@ const char* vgpa_last_error(const vgpa_handle* h) { return h ? h->err.c_str() : 
 
 namespace {
 
-// vgpa_create and vgpa_create_obs_rows.  obs_t: the schedules, obs_t_stride elements apart (0 = one row shared by
-// every problem); counts: B observation counts or NULL (desc->M each).  rows == false: vgpa_create's one schedule,
-// desc->obs_t.
+// vgpa_create, vgpa_create_obs_rows and vgpa_create_observed.  obs_t: the schedules, obs_t_stride elements apart (0 =
+// one row shared by every problem); counts: B observation counts or NULL (desc->M each).  rows == false: vgpa_create's
+// one schedule, desc->obs_t.  observed: the masks of the observed components, observed_stride words apart (0 = one
+// mask shared by every problem), or NULL = every component.
 int create_handle(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride, const int32_t* counts, bool rows,
-                  vgpa_handle** out)
+                  const uint64_t* observed, int64_t observed_stride, vgpa_handle** out)
 {
     vgpa_handle* h = new vgpa_handle();
     h->d = *d;
@@ -467,6 +469,16 @@ int create_handle(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride
             if (h->init_edge < 0 && Mp > 0 && (ot[0] == 0 || ot[Mp - 1] == d->N - 1)) h->init_edge = p;
         }
     }
+    if (observed != nullptr) {
+        if (observed_stride < 0)
+            return bail(h->fail(VGPA_EINVAL, "observed_stride %lld: 0 (one shared mask) or positive", (long long)observed_stride));
+        for (int p = 0; p < d->B; ++p) {
+            const uint64_t w = observed[p * observed_stride];
+            if (w == 0) return bail(h->fail(VGPA_EINVAL, "the observation mask of problem %d has no bit set", p));
+            if (d->D < 64 && (w >> d->D) != 0)
+                return bail(h->fail(VGPA_EINVAL, "the observation mask of problem %d has a bit at or above D = %d", p, d->D));
+        }
+    }
     {
         const long long cnt = (d->sigma_stride == 0) ? 1 : d->B;
         for (long long q = 0; d->sigma && q < cnt; ++q)
@@ -500,24 +512,55 @@ int create_handle(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride
         *dev = buf.as<double>();
         return VGPA_OK;
     };
+    // Partially observed problems: the device copies of R and obs_y hold +inf and 0 at every unobserved (problem,
+    // component), so that the sweeps' jumps -(y - m) / R and 0.5 / R are zeros there without a mask, and neither a NaN
+    // nor any other value the caller left in those entries reaches the arithmetic.  B rows, or one when the values
+    // and the masks are both shared.
+    std::vector<double> R_obs, y_obs;
+    const double* R_src = d->R;
+    const double* y_src = d->obs_y;
+    long long R_stride = d->R_stride, y_stride = d->obs_y_stride;
+    auto mask_rows = [&](const double*& src, long long& stride, long long len, double fill, std::vector<double>& v) {
+        if (observed == nullptr || src == nullptr || (stride != 0 && stride < len)) return;   // upload_param reports these
+        const int rows = (stride == 0 && observed_stride == 0) ? 1 : B;
+        v.resize((size_t)rows * len);
+        for (int p = 0; p < rows; ++p) {
+            const uint64_t w = observed[p * observed_stride];
+            for (long long k = 0; k < len; ++k)
+                v[(size_t)p * len + k] = ((w >> (k % D)) & 1) ? src[p * stride + k] : fill;
+        }
+        src = v.data();
+        stride = rows == 1 ? 0 : len;
+    };
+    mask_rows(R_src, R_stride, D, INFINITY, R_obs);
+    if (M > 0) mask_rows(y_src, y_stride, (long long)M * D, 0.0, y_obs);
     int rc;
-#define UP(field, len)                                                                                       \
-    if ((rc = upload_param(h->field, d->field, d->field##_stride, (len), &b.field, &b.field##_stride, #field)) \
-        != VGPA_OK)                                                                                          \
+#define UP_FROM(field, src, stride, len)                                                                      \
+    if ((rc = upload_param(h->field, (src), (stride), (len), &b.field, &b.field##_stride, #field)) != VGPA_OK) \
         return bail(rc);
+#define UP(field, len) UP_FROM(field, d->field, d->field##_stride, len)
     UP(theta, n_theta(d->model));
     UP(sigma, D);
-    UP(R, D);
+    UP_FROM(R, R_src, R_stride, D);
     UP(m0, D);
     UP(s0, (long long)D * D);
     UP(E0, 1);
     if (M > 0) {
-        UP(obs_y, (long long)M * D);
+        UP_FROM(obs_y, y_src, y_stride, (long long)M * D);
     } else {
         b.obs_y = nullptr;
         b.obs_y_stride = 0;
     }
 #undef UP
+#undef UP_FROM
+    if (observed != nullptr) {   // one word per problem on the device (a shared mask expanded)
+        std::vector<unsigned long long> w(B);
+        for (int p = 0; p < B; ++p) w[p] = observed[p * observed_stride];
+        cudaError_t e = cudaSuccess;
+        upload(e, h->observed, w.data(), w.size());
+        if (e != cudaSuccess) return bail(h->cuda_fail(e, "upload(observed)"));
+        b.observed = h->observed.as<unsigned long long>();
+    }
     if (!rows) {
         std::vector<long long> ot(std::max(M, 1), 0);
         std::vector<int> oi(N, -1);
@@ -613,7 +656,20 @@ int vgpa_create(const vgpa_desc* d, vgpa_handle** out)
 {
     if (out) *out = nullptr;
     if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create: NULL argument");
-    return create_handle(d, nullptr, 0, nullptr, false, out);
+    return create_handle(d, nullptr, 0, nullptr, false, nullptr, 0, out);
+}
+
+int vgpa_create_observed(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride, const int32_t* M,
+                         const uint64_t* observed, int64_t observed_stride, vgpa_handle** out)
+{
+    if (out) *out = nullptr;
+    if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create_observed: NULL argument");
+    if (obs_t_stride == 0 && M == nullptr && d->obs_t == nullptr) {   // one shared schedule: that of vgpa_create
+        vgpa_desc one = *d;
+        one.obs_t = obs_t;
+        return create_handle(&one, nullptr, 0, nullptr, false, observed, observed_stride, out);
+    }
+    return create_handle(d, obs_t, obs_t_stride, M, true, observed, observed_stride, out);
 }
 
 int vgpa_create_obs_rows(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t_stride, const int32_t* M,
@@ -621,12 +677,7 @@ int vgpa_create_obs_rows(const vgpa_desc* d, const int64_t* obs_t, int64_t obs_t
 {
     if (out) *out = nullptr;
     if (d == nullptr || out == nullptr) return set_error(VGPA_EINVAL, "vgpa_create_obs_rows: NULL argument");
-    if (obs_t_stride == 0 && M == nullptr && d->obs_t == nullptr) {   // one shared schedule: exactly vgpa_create
-        vgpa_desc one = *d;
-        one.obs_t = obs_t;
-        return create_handle(&one, nullptr, 0, nullptr, false, out);
-    }
-    return create_handle(d, obs_t, obs_t_stride, M, true, out);
+    return vgpa_create_observed(d, obs_t, obs_t_stride, M, nullptr, 0, out);
 }
 
 void vgpa_destroy(vgpa_handle* h)
@@ -1064,8 +1115,13 @@ int vgpa_model_energy(int device, int model, int D, int N, double dt_model, cons
     return VGPA_OK;
 }
 
-int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const double* obs_y, const double* R,
-                    const double* mt, const double* st, double* Eobs, double* jm, double* js, double* dr)
+}  // extern "C"
+
+// vgpa_obs_energy and vgpa_obs_energy_observed: the components whose bit of `observed` is clear are left out of Eobs
+// and keep zero jumps.
+static int obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const double* obs_y, const double* R,
+                      uint64_t observed, const double* mt, const double* st, double* Eobs, double* jm, double* js,
+                      double* dr)
 {
     if ((D != 1 && D != 3 && (D < 10 || D > 64)) || N < 2 || M < 0 || M > N)
         return set_error(VGPA_EINVAL, "Wrong dimensions for the likelihood");
@@ -1074,11 +1130,13 @@ int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const
         if (obs_t[n] < 0 || obs_t[n] >= N) return set_error(VGPA_EINVAL, "observation index out of range");
     if (cudaSetDevice(device) != cudaSuccess) return set_error(VGPA_ECUDA, "cudaSetDevice failed");
     const long long nv = (long long)N * D, nm = (long long)N * D * D;
-    DevBuf dot, doy, dR, dmt, dst, djm, djs, des, dparts, dzero, dF, ddr;
+    DevBuf dot, doy, dR, dmt, dst, djm, djs, des, dparts, dzero, dF, ddr, dobs;
     std::vector<long long> ot(std::max(M, 1), 0);
     for (int n = 0; n < M; ++n) ot[n] = obs_t[n];
+    const unsigned long long word = observed;
     cudaError_t e = cudaSuccess;
     upload(e, dot, ot.data(), ot.size());
+    upload(e, dobs, &word, 1);
     alloc(e, doy, (size_t)std::max(M, 1) * D);
     if (M > 0) to_device(e, doy.p, obs_y, (size_t)M * D);
     upload(e, dR, R, D);
@@ -1097,13 +1155,13 @@ int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const
     bt.model = (D == 1) ? MODEL_OU : (D == 3 ? MODEL_L63 : MODEL_L96);
     bt.D = D; bt.N = N; bt.M = M; bt.B = 1; bt.dt = 1.0; bt.dt_model = 1.0;
     bt.sigma = dR.as<double>(); bt.R = dR.as<double>(); bt.E0 = dzero.as<double>();
-    bt.obs_t = dot.as<long long>(); bt.obs_y = doy.as<double>();
+    bt.obs_t = dot.as<long long>(); bt.obs_y = doy.as<double>(); bt.observed = dobs.as<unsigned long long>();
     Scratch sc{};
     sc.mt = dmt.as<double>(); sc.st = dst.as<double>(); sc.esde_t = des.as<double>();
     Extra ex{};
     ex.parts = dparts.as<double>();
     launch_finalize(bt, sc, dF.as<double>(), 0, 1, ex, nullptr);
-    launch_jump_tables(D, N, M, dot.as<long long>(), doy.as<double>(), dR.as<double>(), dmt.as<double>(),
+    launch_jump_tables(D, N, M, dot.as<long long>(), doy.as<double>(), dR.as<double>(), observed, dmt.as<double>(),
                        djm.as<double>(), djs.as<double>(), nullptr);
     if (dr != nullptr && D == 1) {
         alloc(e, ddr, N);
@@ -1124,6 +1182,23 @@ int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const
     if (e != cudaSuccess) return set_cuda_error(e, "vgpa_obs_energy");
     *Eobs = parts[2];
     return VGPA_OK;
+}
+
+extern "C" {
+
+int vgpa_obs_energy(int device, int D, int N, int M, const int64_t* obs_t, const double* obs_y, const double* R,
+                    const double* mt, const double* st, double* Eobs, double* jm, double* js, double* dr)
+{
+    return obs_energy(device, D, N, M, obs_t, obs_y, R, ~0ull, mt, st, Eobs, jm, js, dr);
+}
+
+int vgpa_obs_energy_observed(int device, int D, int N, int M, const int64_t* obs_t, const double* obs_y, const double* R,
+                             uint64_t observed, const double* mt, const double* st, double* Eobs, double* jm, double* js)
+{
+    if (observed == 0) return set_error(VGPA_EINVAL, "the observation mask has no bit set");
+    if (D >= 1 && D < 64 && (observed >> D) != 0)
+        return set_error(VGPA_EINVAL, "the observation mask has a bit at or above D = %d", D);
+    return obs_energy(device, D, N, M, obs_t, obs_y, R, observed, mt, st, Eobs, jm, js, nullptr);
 }
 
 static int init_check(vgpa_handle* h, const double* x, int64_t x_stride)

@@ -54,9 +54,20 @@ struct Batch {
     long long obs_t_stride;
     long long obs_index_stride;
     const int* obs_count;     // B counts <= M, or null = M each
-    long long pad_;           // keeps the fields added with the schedules at 32 bytes: the kernel parameters that follow
-                              // a Batch keep their 16-byte alignment, and the D = 40 kernels their code (and speed)
+    // Partially observed problems (vgpa_create_observed): B words, bit i of word p set = component i of problem p is
+    // observed; null = every component of every problem.  Only the observation energy (free_energy_of) and the
+    // initialisation read it.  The sweeps' jumps need no mask: the handle's device copy of R holds +inf and its copy
+    // of obs_y holds 0 at every unobserved (problem, component), so the jump -(y - m) / R is a zero and 0.5 / R is 0.
+    // (The pointer keeps the fields added with the schedules at 32 bytes: the kernel parameters that follow a Batch
+    // keep their 16-byte alignment, and the D = 40 kernels their code and speed.)
+    const unsigned long long* observed;
 };
+
+// The observed components of problem p (bit i = component i).
+__device__ __forceinline__ unsigned long long observed_of(const Batch& b, int p)
+{
+    return b.observed != nullptr ? b.observed[p] : ~0ull;
+}
 
 // problem served by launch position `pos` (= p0 + local index)
 __device__ __forceinline__ int problem_at(const Batch& b, int pos) { return b.plist != nullptr ? b.plist[pos] : pos; }
@@ -245,8 +256,9 @@ void launch_obs_dr(int N, int M, const long long* obs_t, const double* obs_y, co
 void launch_trajectories(const TrajArgs& a, cudaStream_t st);
 void launch_collect_obs(const ObsArgs& a, cudaStream_t st);
 
-// Dense jump tables dEobs_dm (N,D), dEobs_ds (N,D,D) (GaussianLikelihood.gradients).
+// Dense jump tables dEobs_dm (N,D), dEobs_ds (N,D,D) (GaussianLikelihood.gradients); entries of the components
+// whose bit of `observed` is clear stay zero.
 void launch_jump_tables(int D, int N, int M, const long long* obs_t, const double* obs_y, const double* R,
-                        const double* mt, double* jm, double* js, cudaStream_t st);
+                        unsigned long long observed, const double* mt, double* jm, double* js, cudaStream_t st);
 
 }  // namespace vgpa

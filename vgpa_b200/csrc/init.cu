@@ -14,6 +14,8 @@
 //             each problem has its own M[p] + 2 knots)
 //   kernel 2: one thread per (problem, time index, dimension) evaluates the spline at tw[k] and
 //             tw[k+1], forms b0 and the diagonal entry of A0 (the zeros of A0 come from a memset)
+// A component a partially observed problem does not observe (vgpa_create_observed) has no spline: its mean path
+// is the constant m0[p][d], so b0(t)_d = a_dd m0_d (DESIGN.md section 5.1).
 #include "common.cuh"
 
 namespace vgpa {
@@ -49,6 +51,7 @@ init_slopes_kernel(Batch b, int p0, int count, double t0, double* __restrict__ s
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     if (pair >= count * b.D) return;
     const int lp = pair / b.D, d = pair - lp * b.D, p = p0 + lp;
+    if (!((observed_of(b, p) >> d) & 1ull)) return;           // unobserved: no spline (init_x0_kernel writes m0)
     const Knots kn = knots_of(b, p);
     const int n = kn.n;
     double* s = scratch + (long long)pair * 2 * (b.M + 2);   // slots of the handle's capacity
@@ -129,7 +132,9 @@ init_x0_kernel(Batch b, int p0, int count, double t0, const double* __restrict__
     const double* s = scratch + ((long long)lp * D + d) * 2 * (b.M + 2);
     double* xo = x + (long long)p * xs;
     const double ad = 0.5 * (b.sigma[p * b.sigma_stride + d] / 0.25);      // variational.py:95 / :122-126
-    const double m0 = spline_at(b, kn, s, d, t0, k);
+    // An unobserved component has no spline: its mean path is the constant m0[p][d], so b0(t)_d = a_dd m0_d.
+    const bool obs = (observed_of(b, p) >> d) & 1ull;
+    const double m0 = obs ? spline_at(b, kn, s, d, t0, k) : b.m0[p * b.m0_stride + d];
     if (D == 1) {
         xo[k] = ad;
         xo[N + k] = m0;                                                     // :101
@@ -137,7 +142,7 @@ init_x0_kernel(Batch b, int p0, int count, double t0, const double* __restrict__
     }
     xo[((long long)k * D + d) * D + d] = ad;           // the rest of A0 was zero-filled by the launcher
     double bk = ad * m0;                                                    // :133 at the last index
-    if (k < N - 1) bk += (spline_at(b, kn, s, d, t0, k + 1) - m0) / b.dt_model;  // :121, :127 (self.dt = model.time_step, :57)
+    if (obs && k < N - 1) bk += (spline_at(b, kn, s, d, t0, k + 1) - m0) / b.dt_model;  // :121, :127 (self.dt = model.time_step, :57)
     xo[(long long)N * D * D + (long long)k * D + d] = bk;
 }
 

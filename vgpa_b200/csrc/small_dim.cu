@@ -877,17 +877,26 @@ __device__ __forceinline__ double free_energy_of(const Batch& b, int p, const do
         const double sm = block_sum(acc, sh);
         Eobs = 0.5 * sm / R[0] + 0.5 * M * (LOG2PI + log(R[0]));
     } else {  // gaussian_like.py:98-153; S diagonal indexed by the observation ORDINAL n
+        // H = the rows of the identity at the observed components O: the sums run over O, the count term has
+        // D_o = |O|.  With O = every component the arithmetic is the identity operator's, bit for bit.
+        const unsigned long long obs = observed_of(b, p);
         acc = 0.0;
         for (int q = tid; q < (tid < W ? M * D : 0); q += W) {
             const int n = q / D, i = q % D;
+            if (!((obs >> i) & 1ull)) continue;
             const long long t = ot[n];
             const double z = (oy[(long long)n * D + i] - mt[t * D + i]) / sqrt(R[i]);
             acc += z * z + (1.0 / R[i]) * st[(long long)n * DD + (long long)i * D + i];
         }
         const double sm = block_sum(acc, sh);
         double ld = 0.0;
-        for (int i = 0; i < D; ++i) ld += log(sqrt(R[i]));
-        Eobs = 0.5 * (sm + M * (D * LOG2PI + 2.0 * ld));
+        int Do = 0;
+        for (int i = 0; i < D; ++i)
+            if ((obs >> i) & 1ull) {
+                ld += log(sqrt(R[i]));
+                ++Do;
+            }
+        Eobs = 0.5 * (sm + M * (Do * LOG2PI + 2.0 * ld));
     }
     const double E0 = b.E0[p * b.E0_stride];
     if (parts != nullptr && tid == 0) {
@@ -1318,24 +1327,27 @@ void launch_bwd_dense(int method, int D, int N, double dt, const double* A, cons
     else        bwd_dispatch<MODEL_L63, 3>(b, s, a, 0, 1, ex, st);
 }
 
-// gaussian_like.py:188,191 (1-D) / :235,238 (n-D, H = I, diagonal R)
+// gaussian_like.py:188,191 (1-D) / :235,238 (n-D, diagonal R): -H^T R^-1 (y - H m) and 1/2 H^T R^-1 H for H the
+// rows of the identity at the components set in `observed`; the other entries keep the launcher's zeros.
 __global__ void jump_tables_kernel(int D, int N, int M, const long long* __restrict__ obs_t,
                                    const double* __restrict__ obs_y, const double* __restrict__ R,
-                                   const double* __restrict__ mt, double* __restrict__ jm, double* __restrict__ js)
+                                   unsigned long long observed, const double* __restrict__ mt, double* __restrict__ jm,
+                                   double* __restrict__ js)
 {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= M * D) return;
     const int n = q / D, i = q % D;
+    if (!((observed >> i) & 1ull)) return;
     const long long t = obs_t[n];
     jm[t * D + i] = -(obs_y[(long long)n * D + i] - mt[t * D + i]) / R[i];
     js[t * D * D + (long long)i * D + i] = 0.5 / R[i];
 }
 void launch_jump_tables(int D, int N, int M, const long long* obs_t, const double* obs_y, const double* R,
-                        const double* mt, double* jm, double* js, cudaStream_t st)
+                        unsigned long long observed, const double* mt, double* jm, double* js, cudaStream_t st)
 {
     cudaMemsetAsync(jm, 0, sizeof(double) * (size_t)N * D, st);
     cudaMemsetAsync(js, 0, sizeof(double) * (size_t)N * D * D, st);
-    if (M > 0) jump_tables_kernel<<<(M * D + 127) / 128, 128, 0, st>>>(D, N, M, obs_t, obs_y, R, mt, jm, js);
+    if (M > 0) jump_tables_kernel<<<(M * D + 127) / 128, 128, 0, st>>>(D, N, M, obs_t, obs_y, R, observed, mt, jm, js);
 }
 
 void launch_finalize(const Batch& b, const Scratch& s, double* F, int p0, int count, const Extra& ex,

@@ -91,7 +91,8 @@ class StochasticProcess(object):
             xi = self.rand_g.standard_normal(dim_m)
             if device is not None and not h_mask:
                 return obs_t, engine.collect_observations(self.xt, obs_t, [float(rn)], xi[None], device)[0], obs_noise
-            obs_y += np.sqrt(obs_noise) * xi
+            # one observed component of an n-D path (h_mask of length 1): obs_y is (M, 1), one draw per observation
+            obs_y += (np.sqrt(obs_noise) * xi).reshape(obs_y.shape)
         else:
             obs_noise = np.diag(rn) if rn.ndim == 1 else rn * np.eye(dim_d)
             sq_rn = np.sqrt(obs_noise)

@@ -59,6 +59,42 @@ def _schedule_rows(obs_t, obs_y, B, D):
     return rows, vals, counts, M
 
 
+def _mask_word(sel, D, what):
+    """One observation mask: a (D,) bool array or a 1-D sequence of distinct component indices -> the bit word."""
+    a = np.asarray(sel)
+    if a.ndim != 1:
+        raise ValueError(f"{what}: expected a ({D},) bool array or a list of component indices, got shape {a.shape}")
+    if a.dtype == np.bool_:
+        if a.size != D:
+            raise ValueError(f"{what}: a bool mask needs {D} entries, got {a.size}")
+        idx = np.flatnonzero(a)
+    else:
+        if a.size and not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"{what}: component indices must be integers, got {a.dtype}")
+        idx = a.astype(np.int64)
+        if np.any((idx < 0) | (idx >= D)):
+            raise ValueError(f"{what}: component index out of range [0, {D}): {idx.tolist()}")
+        if np.unique(idx).size != idx.size:
+            raise ValueError(f"{what}: duplicate component index in {idx.tolist()}")
+    if idx.size == 0:
+        raise ValueError(f"{what}: no component is observed")
+    return int(sum(1 << int(i) for i in idx))
+
+
+def observed_words(observed, B, D):
+    """The observed components as bit words (bit i = component i): one mask shared by the batch -- a (D,) bool
+    array or a 1-D list of component indices -- or one per problem -- a (B, D) bool array or a list of B index
+    lists.  Returns (uint64 array, stride in words: 0 shared, 1 per problem)."""
+    a = observed if isinstance(observed, np.ndarray) else None
+    per = (a is not None and a.ndim == 2) or (
+        a is None and isinstance(observed, (list, tuple)) and len(observed) > 0 and any(np.ndim(o) > 0 for o in observed))
+    if not per:
+        return np.array([_mask_word(observed, D, "observed")], dtype=np.uint64), 0
+    if len(observed) != B:
+        raise ValueError(f"observed: expected {B} per-problem masks, got {len(observed)}")
+    return np.array([_mask_word(o, D, f"observed of problem {p}") for p, o in enumerate(observed)], dtype=np.uint64), 1
+
+
 class BatchEvaluator:
     """
     :param model:  "DW" | "OU" | "L63" | "L96"   (simulation.py:20)
@@ -73,10 +109,15 @@ class BatchEvaluator:
            not a flattened shared schedule, and needs obs_y as a list too.  A flat list or any numpy array keeps
            the shared meaning.
     :param D: state dimension; None = the model's (L96: 40).  L96 takes any 10 <= D <= 64
+    :param observed: the observed state components; None = all.  One set shared by the batch -- a (D,) bool
+           array or a 1-D list of component indices -- or one per problem -- a (B, D) bool array or a list of B
+           index lists.  obs_y and R keep their D columns; those of unobserved components are ignored.  An
+           unobserved component contributes nothing to Eobs and its jumps, and initialization() gives it the
+           constant mean path m0 (vgpa_create_observed).
     """
 
     def __init__(self, model, method, N, dt, theta, sigma, R, obs_t, obs_y, m0, s0, E0,
-                 B=1, dt_model=None, device=0, scratch_bytes=0, D=None):
+                 B=1, dt_model=None, device=0, scratch_bytes=0, D=None, observed=None):
         key = str(model).upper()
         if key not in MODELS:
             raise ValueError(f" Unknown stochastic model -> {key}")
@@ -95,6 +136,8 @@ class BatchEvaluator:
         else:
             obs_t = np.ascontiguousarray(np.asarray(obs_t, dtype=np.int64).ravel())
             M = obs_t.size
+        if observed is not None:
+            keep["observed"], obs_stride = observed_words(observed, self.B, D)
         nth = 3 if key == "L63" else 1
         d = VgpaDesc()
         d.model, d.method, d.D, d.N, d.M, d.B = MODELS[key], METHODS[mkey], D, self.N, M, self.B
@@ -112,7 +155,11 @@ class BatchEvaluator:
         keep["obs_t"] = obs_t
         d.scratch_bytes = int(scratch_bytes)
         self._h = C.c_void_p()
-        if rows:   # every problem its own schedule, padded to M rows
+        if observed is not None:
+            rc = lib.vgpa_create_observed(C.byref(d), obs_t.ctypes.data, obs_t.shape[1] if rows else 0,
+                                          counts.ctypes.data if rows else None, keep["observed"].ctypes.data,
+                                          obs_stride, C.byref(self._h))
+        elif rows:   # every problem its own schedule, padded to M rows
             rc = lib.vgpa_create_obs_rows(C.byref(d), obs_t.ctypes.data, obs_t.shape[1], counts.ctypes.data,
                                           C.byref(self._h))
         else:
@@ -347,8 +394,10 @@ def model_energy(model, theta, sigma_diag, A, b, m, S, dt_model, device=0, hyper
     return out + (dth, dsig.reshape(D, D)) if hyper else out
 
 
-def obs_energy(obs_t, obs_y, R_diag, m, s, device=0, with_dr=False):
-    """GaussianLikelihood.__call__ / .gradients: returns Eobs, dEobs_dm, dEobs_ds (+ dEobs_dr)."""
+def obs_energy(obs_t, obs_y, R_diag, m, s, device=0, with_dr=False, observed=None):
+    """GaussianLikelihood.__call__ / .gradients: returns Eobs, dEobs_dm, dEobs_ds (+ dEobs_dr).  observed: the bit
+    word of the observed components (vgpa_obs_energy_observed; obs_y (M, D) and R (D,) with ignored entries at the
+    others), None = all; dEobs_dr is not available with a mask."""
     m = f64(m)
     single = m.ndim == 1
     N = m.shape[0]
@@ -361,8 +410,14 @@ def obs_energy(obs_t, obs_y, R_diag, m, s, device=0, with_dr=False):
     E = np.zeros(1)
     jm, js = np.empty(N * D), np.empty(N * D * D)
     dr = np.empty(N if single else N * M * M) if with_dr else None
-    rc = lib.vgpa_obs_energy(device, D, N, M, ot.ctypes.data_as(C.POINTER(C.c_int64)), dptr(oy), dptr(R),
-                             dptr(m), dptr(s), dptr(E), dptr(jm), dptr(js), dptr(dr) if with_dr else None)
+    if observed is not None:
+        if with_dr:
+            raise ValueError("obs_energy: dEobs_dr is not computed for a component-selecting operator")
+        rc = lib.vgpa_obs_energy_observed(device, D, N, M, ot.ctypes.data_as(C.POINTER(C.c_int64)), dptr(oy), dptr(R),
+                                          int(observed), dptr(m), dptr(s), dptr(E), dptr(jm), dptr(js))
+    else:
+        rc = lib.vgpa_obs_energy(device, D, N, M, ot.ctypes.data_as(C.POINTER(C.c_int64)), dptr(oy), dptr(R),
+                                 dptr(m), dptr(s), dptr(E), dptr(jm), dptr(js), dptr(dr) if with_dr else None)
     raise_for(rc, None)
     if single:
         out = (float(E[0]), jm, js)

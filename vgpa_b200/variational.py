@@ -133,18 +133,37 @@ class VarGP(object):
         if self._ev_obj is None:
             D = self.dim_d
             m0, s0 = self.output["m0"], self.output["s0"]
+            obs_y, R, observed = self._observations()
             self._ev_obj = BatchEvaluator(
                 model=_model_key(self.model), method=self.fwd_ode.method, N=self.dim_n, dt=self.fwd_ode.dt,
                 theta=np.atleast_1d(np.asarray(self.model.theta, dtype=float)),
                 sigma=_diag(self.model.sigma, "system noise"),
-                R=_diag(self.likelihood.noise, "observation noise"),
+                R=R,
                 obs_t=np.asarray(self.obs_t, dtype=np.int64),
-                obs_y=np.asarray(self.obs_y, dtype=float).reshape(-1, D),
+                obs_y=obs_y.reshape(-1, D),
                 m0=np.atleast_1d(np.asarray(m0, dtype=float)),
                 s0=np.asarray(s0, dtype=float).reshape(D, D),
                 E0=float(np.asarray(self.kl0(m0, s0))),              # constant: variational.py:183-185
-                B=1, dt_model=float(self.dt), device=self._device, D=D)
+                B=1, dt_model=float(self.dt), device=self._device, D=D, observed=observed)
         return self._ev_obj
+
+    def _observations(self):
+        """obs_y (M, D) and the diagonal of R (D,) over the state's components, and the observed components
+        (None = all).  A likelihood whose operator selects components (the JSON's Observations.operator) holds
+        (M, D_o) values and D_o noise values: they go to the selected columns in operator order, and the
+        other columns, which are never read, hold placeholders."""
+        D = self.dim_d
+        y = np.asarray(self.obs_y, dtype=float).reshape(np.asarray(self.obs_t).size, -1)
+        R = _diag(self.likelihood.noise, "observation noise")
+        cols = getattr(self.likelihood, "obs_cols", None)
+        if cols is None or D == 1:
+            return y, R, None
+        if cols.max() >= D:
+            raise ValueError(f" VarGP: the observation operator selects component {int(cols.max())}, the state has {D}")
+        yf, Rf = np.zeros((y.shape[0], D)), np.ones(D)
+        yf[:, cols] = y
+        Rf[cols] = np.broadcast_to(R, cols.shape)
+        return yf, Rf, cols.tolist()
 
     # -- variational.py:73-139 (host-side set-up, not on the per-iteration path) ------
     def initialization(self):
@@ -155,8 +174,14 @@ class VarGP(object):
             a0 = 0.5 * (self.model.sigma / 0.25) * np.ones(self.dim_n)
             b0 = CubicSpline(time_x, obs_z)(time_window)
         else:
-            obs_z = np.vstack((self.obs_y[0], self.obs_y, self.obs_y[-1]))
+            # an unobserved component gets the constant mean path m0 (this project's rule: the reference's
+            # spline combines the D_o observed columns with D-vectors and cannot serve a proper subset)
+            obs_y, _, observed = self._observations()
+            obs_z = np.vstack((obs_y[0], obs_y, obs_y[-1]))
             mt0 = CubicSpline(time_x, obs_z)(time_window)
+            if observed is not None:
+                hidden = np.setdiff1d(np.arange(self.dim_d), observed)
+                mt0[:, hidden] = np.asarray(self.output["m0"], dtype=float).reshape(-1)[hidden]
             a0 = np.zeros((self.dim_n, self.dim_d, self.dim_d))
             b0 = np.zeros((self.dim_n, self.dim_d))
             s0 = 0.25 * np.eye(self.dim_d)
